@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W                    # this implementation
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's own CPU implementation
+    python bench.py ... --dump-outputs DIR                           # also write the last timed step's feature lists
 
 Workload (BASELINE.json configs[1], SURVEY 8(d) "config B"): synthetic textured 1920x1080 frame pairs, 1000 features,
 3 pyramid levels, subsampling 2, 7x7 window, max_residue 10, translational LK, non-sequential KLTTrackFeatures
@@ -310,6 +311,8 @@ def run_b200(args):
     if rank == 0:
         sampler.start()
     dev_ms, dev_wall, launches = timed(step_device, args.steps, args.warmup)
+    if args.dump_outputs:           # the later legs reuse d_x / d_y / d_v: take the timed step's lists now
+        dump_outputs(args.dump_outputs, ctx, d_x, d_y, d_v, B, n, rank, world)
     serial_ms, _, _ = timed(step_device_serial, args.steps, 3)        # the same work as three calls on one stream (no overlap)
     # ---- per-kernel durations, measured live with CUDA events on the launching stream: a separate pass right after the timed
     # region (same clocks and thermal state as `value`; the legs further down run the GPU at its power cap for seconds) ----
@@ -598,6 +601,29 @@ def run_b200(args):
     sys.stdout.flush()
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ctx, d_x, d_y, d_v, B, n, rank, world):
+    """Writes the feature lists the last timed step left in d_x / d_y / d_v -- what a caller of klt_track_pairs_u8 receives --
+    as <out_dir>/{x,y,val}.npy, float64 [pairs, n] (val holds the status codes).  The inputs are seeded, so two builds run
+    with the same arguments can be compared array for array.  Above DUMP_LIMIT_BYTES in all (over every rank) a fixed seeded
+    sample of pairs is written, with its pair indices in pairs.npy.  At N > 1 each rank adds _rank<r> to the names."""
+    x, y, v = np.empty((B, n), np.float64), np.empty((B, n), np.float64), np.empty((B, n), np.int32)
+    ctx.memcpy(x, d_x, B * n * 8); ctx.memcpy(y, d_y, B * n * 8); ctx.memcpy(v, d_v, B * n * 4)
+    ctx.sync()
+    arrays = {"x": x, "y": y, "val": v.astype(np.float64)}
+    max_pairs = DUMP_LIMIT_BYTES // world // ((3 * n + 1) * 8)
+    if B > max_pairs:
+        pick = np.sort(np.random.default_rng(0).choice(B, max_pairs, replace=False))
+        arrays = {k: a[pick] for k, a in arrays.items()}
+        arrays["pairs"] = pick.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "_rank%d" % rank if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
 
 
 def motion_cycle(H, W, seed, period=100):
@@ -1099,7 +1125,13 @@ def main():
     ap.add_argument("--seqs", type=int, default=8, help="config D: lock-stepped sequences per GPU (0 disables the sequence object)")
     ap.add_argument("--seq-frames", type=int, default=300)
     ap.add_argument("--sustain-s", type=float, default=2.5, help="length of the sustained leg in seconds")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the feature lists of the last timed step as DIR/{x,y,val}.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the B200 arm's timed step computed; the reference arm has no such step")
     if args.impl == "reference":
         run_reference(args)
     else:

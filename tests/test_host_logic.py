@@ -435,3 +435,45 @@ def test_bench_select_fast_leg_on_stubs(monkeypatch):
     assert r["ms_per_call"] == 0.5 and r["ms_per_frame"] == 0.125 and r["kernel_ms_per_call"]["eigen_fast"] == 0.1
     fused, unfused = r["eigen_pass"]["bytes_per_frame_fused"], r["eigen_pass"]["bytes_per_frame_unfused_accounting"]
     assert fused >= 4.0 * 64 * 48 and (fused - 4.0 * 64 * 48) % 4 == 0 and unfused - fused == 13.0 * 64 * 48
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: the timed step's x / y / val lists as float64 .npy files, the same seeded sample of pairs on every
+    run once the lists exceed the size limit, and per-rank names at N > 1.  The device arrays are stood in by host arrays."""
+    import os
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+
+    class Ctx(object):
+        def memcpy(self, dst, src, nbytes):
+            assert dst.nbytes == nbytes == src.nbytes
+            dst[...] = src
+
+        def sync(self):
+            pass
+
+    B, n = 12, 5
+    rng = np.random.default_rng(1)
+    x, y = rng.uniform(0, 100, (B, n)), rng.uniform(0, 100, (B, n))
+    v = rng.integers(-5, 1, (B, n)).astype(np.int32)
+    bench.dump_outputs(str(tmp_path / "all"), Ctx(), x, y, v, B, n, 0, 1)
+    got = {k: np.load(str(tmp_path / "all" / (k + ".npy"))) for k in ("x", "y", "val")}
+    assert sorted(os.listdir(str(tmp_path / "all"))) == ["val.npy", "x.npy", "y.npy"]
+    assert all(a.dtype == np.float64 and a.shape == (B, n) for a in got.values())
+    assert np.array_equal(got["x"], x) and np.array_equal(got["y"], y) and np.array_equal(got["val"], v)
+
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 5 * (3 * n + 1) * 8)       # room for 5 pairs
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), Ctx(), x, y, v, B, n, 0, 1)
+    pairs = np.load(str(tmp_path / "s1" / "pairs.npy"))
+    assert np.array_equal(pairs, np.load(str(tmp_path / "s2" / "pairs.npy")))
+    assert len(pairs) == 5 and np.all(np.diff(pairs) > 0)
+    pick = pairs.astype(np.int64)
+    assert np.array_equal(np.load(str(tmp_path / "s1" / "x.npy")), x[pick])
+    assert np.array_equal(np.load(str(tmp_path / "s1" / "val.npy")), v[pick])
+    assert sum(os.path.getsize(str(tmp_path / "s1" / f)) - 128 for f in os.listdir(str(tmp_path / "s1"))) <= bench.DUMP_LIMIT_BYTES
+
+    bench.dump_outputs(str(tmp_path / "r"), Ctx(), x, y, v, B, n, 1, 2)
+    assert sorted(os.listdir(str(tmp_path / "r"))) == ["pairs_rank1.npy", "val_rank1.npy", "x_rank1.npy", "y_rank1.npy"]

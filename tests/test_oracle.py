@@ -265,29 +265,21 @@ def test_live_reference_fractional_min_eigenvalue(oracle, reference):
 
 
 @pytest.mark.parametrize("cfg", ["B", "C"])
-def test_live_reference_full_size(oracle, reference, cfg):
+def test_live_reference_full_size(oracle, golden, golden_fullsize, cfg):
     """The oracle against the unmodified reference at BASELINE's own sizes -- config B (1080p, 1000 features, 3 levels) selection
     + tracking and config C (4K, 10 000 features, 4 levels) selection: the float32 summed-area-table rounding grows with the
-    image size (SURVEY 7.3), so this is the case that pins the selection ORDER.  Bit-identical (==)."""
-    from PIL import Image
+    image size (SURVEY 7.3), so this is the case that pins the selection ORDER.  Bit-identical (==).  The reference's lists
+    for these inputs are stored in tests/golden/reference_golden_fullsize.npz (tests/golden/make_golden_fullsize.py)."""
     from pyfeaturetrack_b200 import synth
-    klt, sgf, tf = reference["klt"], reference["selectGoodFeatures"], reference["trackFeatures"]
     H, W, n, L = (1080, 1920, 1000, 3) if cfg == "B" else (2160, 3840, 10000, 4)
     imgs = synth.frame_pair(H, W, seed=0)
-    kw = dict(nPyramidLevels=L, subsampling=2, max_residue=10.0)
-    tc = klt.KLT_TrackingContext()
-    for k, v in kw.items():
-        setattr(tc, k, v)
-    tc.KLTUpdateTCBorder()
-    p = P(oracle, **kw)
-    assert p.borderx == tc.borderx
-    ref_fl = sgf.KLTSelectGoodFeatures(tc, Image.fromarray(imgs[0]), n)
+    p = P(oracle, nPyramidLevels=L, subsampling=2, max_residue=10.0)
+    assert [p.borderx] == [b for w, lv, ss, b in golden["borders"] if (w, lv, ss) == (7, L, 2)]
     sel = oracle.select_good_features(p, imgs[0], n)
-    assert_features_equal(sel, ([float(f.x) for f in ref_fl], [float(f.y) for f in ref_fl], [f.val for f in ref_fl]))
-    if cfg == "B":        # (tracking at 4K is covered by the GPU suite against the oracle; the reference needs 7 s per 4K pair)
-        tf.KLTTrackFeatures(tc, Image.fromarray(imgs[0]), Image.fromarray(imgs[1]), ref_fl)
+    assert_features_equal(sel, fl(golden_fullsize, "%s_sel%d" % (cfg, n)))
+    if cfg == "B":        # (tracking at 4K is covered by the GPU suite against the same stored lists)
         trk = oracle.track_features(p, imgs[0], imgs[1], *sel)[:3]
-        assert_features_equal(trk, ([float(f.x) for f in ref_fl], [float(f.y) for f in ref_fl], [f.val for f in ref_fl]))
+        assert_features_equal(trk, fl(golden_fullsize, "B_trk1000"))
         assert (trk[2] == 0).sum() > 900
 
 
