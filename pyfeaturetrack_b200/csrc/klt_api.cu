@@ -134,9 +134,7 @@ int klt_ctx_create(int device, void *stream, klt_ctx **out) {
     cudaEventCreate(&ctx->ev1);
     cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking);
     cudaStreamCreateWithFlags(&ctx->aux_stream, cudaStreamNonBlocking);
-    for (int i = 0; i < 10; i++) cudaEventCreateWithFlags(&ctx->ov_ev[i], cudaEventDisableTiming);
-    ctx->overlap_subs = 1;      // measured on B200 (64 x 1080p pairs): 0.874 ms serial, 0.904 / 0.970 / 1.090 ms with 2 / 4 / 8 overlapped sub-batches
-    if (const char *e4 = getenv("KLT_B200_OVERLAP_SUBS")) { const int v = atoi(e4); if (v >= 1 && v <= 8) ctx->overlap_subs = v; }
+    for (int i = 0; i < 2; i++) cudaEventCreateWithFlags(&ctx->ov_ev[i], cudaEventDisableTiming);
     ctx->iters_dev = nullptr;
     for (int i = 0; i < 16; i++) cudaEventCreateWithFlags(&ctx->chunk_ev[i], cudaEventDisableTiming);
     for (int i = 0; i < 2; i++) cudaEventCreateWithFlags(&ctx->half_free[i], cudaEventDisableTiming);
@@ -146,8 +144,6 @@ int klt_ctx_create(int device, void *stream, klt_ctx **out) {
     for (int i = 0; i < 16; i++) cudaEventCreateWithFlags(&ctx->marks[i], cudaEventDisableTiming);
     if (cudaMalloc(&ctx->async_flag_dev, 256) == cudaSuccess) { cudaMemset(ctx->async_flag_dev, 0, 256); ctx->iters_dev = (unsigned long long *)(ctx->async_flag_dev + 16); }
     ctx->num_sms = prop.multiProcessorCount;
-    ctx->fast_quad_nc = 4;
-    if (const char *e3 = getenv("KLT_B200_FAST_NC")) { if (atoi(e3) == 2) ctx->fast_quad_nc = 2; }
     ctx->select_chunk = 4096;
     if (const char *e2 = getenv("KLT_B200_SELECT_CHUNK")) {
         const int v = atoi(e2);
@@ -166,7 +162,7 @@ int klt_ctx_destroy(klt_ctx *ctx) {
     if (ctx->frames_dev) cudaFree(ctx->frames_dev);
     cudaStreamDestroy(ctx->copy_stream);
     cudaStreamDestroy(ctx->aux_stream);
-    for (int i = 0; i < 10; i++) cudaEventDestroy(ctx->ov_ev[i]);
+    for (int i = 0; i < 2; i++) cudaEventDestroy(ctx->ov_ev[i]);
     for (int i = 0; i < 16; i++) cudaEventDestroy(ctx->chunk_ev[i]);
     for (int i = 0; i < 2; i++) cudaEventDestroy(ctx->half_free[i]);
     if (ctx->async_flag_dev) cudaFree(ctx->async_flag_dev);
@@ -413,15 +409,12 @@ int klt_build_u8_device(klt_ctx *ctx, klt_pyr *p, const uint8_t *dframes, size_t
     if (windowed) {
         // u8 -> smoothed image + level 1 in one pass
         // a caller that forks after level 0 (klt_sequence's eigenvalue pass) forks after the fused kernel instead: measured
-        // 0.273 against 0.276 ms per step of 8 sequences, one launch fewer ($KLT_B200_SEQ_FUSED01=0: the two-kernel build)
-        static const bool fork_after_fused = [] { const char *e = getenv("KLT_B200_SEQ_FUSED01"); return !(e && e[0] == '0'); }();
-        if (!ctx->level0_event || fork_after_fused) {
-            rc = klt_stream_level01(ctx, dframes, pitch, frame_stride, p, taps, first, count);
-            if (rc < 0) return rc;
-            if (rc == 1) {
-                if (ctx->level0_event) KLT_CUDA(ctx, cudaEventRecord(ctx->level0_event, ctx->stream));
-                return build_rest(ctx, p, taps, precision, false, first, count, true, 2);
-            }
+        // 0.273 against 0.276 ms per step of 8 sequences with the two-kernel build, one launch fewer
+        rc = klt_stream_level01(ctx, dframes, pitch, frame_stride, p, taps, first, count);
+        if (rc < 0) return rc;
+        if (rc == 1) {
+            if (ctx->level0_event) KLT_CUDA(ctx, cudaEventRecord(ctx->level0_event, ctx->stream));
+            return build_rest(ctx, p, taps, precision, false, first, count, true, 2);
         }
         // u8 -> smoothed image only
         rc = klt_stream_smooth0(ctx, dframes, pitch, frame_stride, p, taps, first, count);
@@ -845,48 +838,10 @@ static int track_pairs_impl(klt_ctx *ctx, const klt_params *params, const klt_ta
     int rc;
     const bool host1 = !klt_is_device_ptr(frames1), host2 = !klt_is_device_ptr(frames2);
     if (!host1 && !host2) {
-        // Device-resident frames AND feature lists: the batch is cut into sub-batches; the tracking kernel of sub-batch i
-        // (instruction-issue bound) runs on a second stream while the pyramid builds of sub-batch i + 1 (HBM bound) run on
-        // the context's stream.  The call only enqueues; a window that leaves the image raises the sticky flag (klt_sync).
-        const int B = pyr1->batch;
-        int nsub = ctx->overlap_subs;
-        if (nsub > B / 2) nsub = B / 2;
-        if (nsub > 8) nsub = 8;
-        const bool dev_lists = x && y && val && klt_is_device_ptr(x) && klt_is_device_ptr(y) && klt_is_device_ptr(val);
-        if (nsub >= 2 && dev_lists && !ctx->profiling && !params->lighting_insensitive && ctx->iters_dev && n_per_image > 0 &&
-            pyr1->batch == pyr2->batch && pyr1->w == pyr2->w && pyr1->h == pyr2->h && pitch >= (size_t)pyr1->w) {
-            if ((rc = check_track_args(ctx, params, pyr1, pyr2))) return rc;
-            KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-            bool windowed;
-            klt_begin_build(pyr1, taps, precision, &windowed);
-            const int arith = klt_begin_build(pyr2, taps, precision, &windowed);
-            if (!windowed || klt_windowed_supported(params, pyr1, pyr2)) {
-                cudaStream_t main = ctx->stream;
-                KLT_CUDA(ctx, cudaEventRecord(ctx->ov_ev[0], main));
-                KLT_CUDA(ctx, cudaStreamWaitEvent(ctx->aux_stream, ctx->ov_ev[0], 0));      // the lists may still be written by earlier work
-                const int per = (B + nsub - 1) / nsub;
-                int k = 0;
-                for (int first = 0; first < B; first += per, k++) {
-                    const int count = first + per <= B ? per : B - first;
-                    const size_t off = (size_t)first * frame_stride;
-                    if ((rc = klt_build_u8_device(ctx, pyr1, frames1 + off, pitch, frame_stride, taps, arith, first, count, windowed))) return rc;
-                    if ((rc = klt_build_u8_device(ctx, pyr2, frames2 + off, pitch, frame_stride, taps, arith, first, count, windowed))) return rc;
-                    KLT_CUDA(ctx, cudaEventRecord(ctx->ov_ev[1 + k], main));
-                    KLT_CUDA(ctx, cudaStreamWaitEvent(ctx->aux_stream, ctx->ov_ev[1 + k], 0));
-                    ctx->stream = ctx->aux_stream;                                            // launch helpers use ctx->stream
-                    rc = klt_launch_track(ctx, params, pyr1, pyr2, n_per_image, x, y, val, ctx->iters_dev, ctx->async_flag_dev, first, count);
-                    ctx->stream = main;
-                    if (rc) return rc;
-                }
-                KLT_CUDA(ctx, cudaEventRecord(ctx->ov_ev[9], ctx->aux_stream));
-                KLT_CUDA(ctx, cudaStreamWaitEvent(main, ctx->ov_ev[9], 0));                   // later work on the context sees the results
-                return KLT_OK;
-            }
-        }
-        static const bool dual = !(getenv("KLT_B200_DUAL_BUILD") && atoi(getenv("KLT_B200_DUAL_BUILD")) == 0);
-        if (dual && !ctx->profiling && pyr1 != pyr2) {
+        if (!ctx->profiling && pyr1 != pyr2) {
             // the two (independent) pyramid builds on two streams: the CTAs of one fill the SM slots the other's last wave
-            // leaves idle (0.774 -> 0.733 ms per 64 pairs at 1080p); $KLT_B200_DUAL_BUILD=0 serialises them again
+            // leaves idle (0.774 -> 0.733 ms per 64 pairs at 1080p).  Profiling brackets every launch with events on the
+            // context's stream, and one pyramid cannot be built twice at once, so those two cases build serially below.
             cudaStream_t main = ctx->stream;
             KLT_CUDA(ctx, cudaEventRecord(ctx->ov_ev[0], main));
             KLT_CUDA(ctx, cudaStreamWaitEvent(ctx->aux_stream, ctx->ov_ev[0], 0));
@@ -895,8 +850,8 @@ static int track_pairs_impl(klt_ctx *ctx, const klt_params *params, const klt_ta
             rc = klt_pyr_build_u8(ctx, pyr2, frames2, pitch, frame_stride, taps, precision);
             ctx->stream = main;
             if (rc) return rc;
-            KLT_CUDA(ctx, cudaEventRecord(ctx->ov_ev[9], ctx->aux_stream));
-            KLT_CUDA(ctx, cudaStreamWaitEvent(main, ctx->ov_ev[9], 0));
+            KLT_CUDA(ctx, cudaEventRecord(ctx->ov_ev[1], ctx->aux_stream));
+            KLT_CUDA(ctx, cudaStreamWaitEvent(main, ctx->ov_ev[1], 0));
             return track_impl(ctx, params, pyr1, pyr2, n_per_image, x, y, val, nullptr, nullptr, async);
         }
         if ((rc = klt_pyr_build_u8(ctx, pyr1, frames1, pitch, frame_stride, taps, precision))) return rc;

@@ -76,10 +76,9 @@ struct klt_ctx {
     cudaEvent_t ev0, ev1;
     // upload pipeline of klt_track_pairs_u8: copy stream, per-chunk events, device staging for the frames
     cudaStream_t copy_stream;
-    cudaStream_t aux_stream;    // second compute stream: tracking of sub-batch i overlaps the pyramid builds of sub-batch i + 1
-    cudaEvent_t ov_ev[10];      // [0] entry, [1..8] "sub-batch built", [9] "all tracked"
+    cudaStream_t aux_stream;    // second compute stream: the second pyramid build of a device-resident klt_track_pairs_u8
+    cudaEvent_t ov_ev[2];       // [0] entry, [1] "second pyramid built"
     cudaEvent_t level0_event;   // if set, klt_build_u8_device records it right after the level-0 kernel (klt_sequence forks its eigenvalue pass there)
-    int overlap_subs;           // sub-batches of the overlapped device path (1 = off, the default: it measured slower; $KLT_B200_OVERLAP_SUBS)
     unsigned long long *iters_dev;   // device counter for calls that do not read it back
     cudaEvent_t chunk_ev[16];
     cudaEvent_t half_free[2];   // recorded on the compute stream once the builds have consumed that staging half
@@ -92,7 +91,6 @@ struct klt_ctx {
     void *ws;
     size_t ws_bytes;
     int num_sms;
-    int fast_quad_nc;           // columns per lane of the fused eigen pass (4; $KLT_B200_FAST_NC=2 for the narrow variant)
     int select_chunk;           // chunk capacity of select_walk_kernel (4096; $KLT_B200_SELECT_CHUNK shrinks it for tests)
 };
 

@@ -96,25 +96,24 @@ eigen_fast_kernel(const float *__restrict__ img0, size_t img_stride, size_t pitc
 }
 
 // ---- windows up to 7x7: the same pass with no shared memory and no barriers -------------------------------------------
-// A WARP owns 32 * NC adjacent columns and marches down its row segment; a lane owns NC adjacent columns (one 64/128-bit load
+// A WARP owns 32 * NC adjacent columns and marches down its row segment; a lane owns NC = 4 adjacent columns (one 128-bit load
 // per row).  Horizontal neighbours -- three image columns for the 7-tap gradient filters, HH columns of window sums -- come
 // from the adjacent lanes by shuffle; the outermost HL = ceil(6 / NC) lanes on either side are halo lanes.  Everything else is
 // arithmetic on NC independent columns; the vertical window sums run as add-new / subtract-old on a warp-private ring.
 #define FQ_L2PF 16           // rows ahead of the L2 prefetch (the register queue covers an L2 hit, this covers DRAM)
+#define FQ_NC 4              // columns per lane
 // MUFU.SQRT: within 1 ulp of sqrtf without its Newton step and special-case branch (this mode is judged by set overlap)
 __device__ __forceinline__ float sqrt_approx(float x) { float r; asm("sqrt.approx.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
-template <int NC> struct QuadVec;
-template <> struct QuadVec<4> { typedef float4 type; };
-template <> struct QuadVec<2> { typedef float2 type; };
 
-template <int HH, int NC, bool STEP1>
+template <int HH, bool STEP1>
 __global__ void __launch_bounds__(FS_THREADS)
 eigen_fast_quad_kernel(const float *__restrict__ img0, size_t img_stride, size_t pitch, const __grid_constant__ SelDev S,
                        const __grid_constant__ FastTaps T, int rows_per_seg, int n_strips, int vec_ok) {
+    constexpr int NC = FQ_NC;
     constexpr int HL = (FS_R + HH + NC - 1) / NC;                   // halo lanes per side
     constexpr int USE = (32 - 2 * HL) * NC;                         // output columns per warp
     constexpr int NB = (FS_R + NC - 1) / NC, NBH = (HH + NC - 1) / NC;   // neighbour lanes that hold the 3 / HH adjacent columns
-    typedef typename QuadVec<NC>::type vec_t;
+    typedef float4 vec_t;
     const int t = threadIdx.x, lane = t & 31, warp = t >> 5, b = blockIdx.z;
     const int W = S.W, H = S.H;
     const int strip = blockIdx.x * (FS_THREADS / 32) + warp;
@@ -214,7 +213,7 @@ eigen_fast_quad_kernel(const float *__restrict__ img0, size_t img_stride, size_t
 #pragma unroll
         for (int c = 0; c < NC; c++) cur[c] = nxt[c];
         load_row(min(y + 1, y_end), nxt);
-        if (y + FQ_L2PF <= y_end && (lane & (NC == 4 ? 7 : 15)) == 0)       // one touch per 128-byte line
+        if (y + FQ_L2PF <= y_end && (lane & 7) == 0)       // one touch per 128-byte line
             asm volatile("prefetch.global.L2 [%0];" ::"l"(img + (size_t)refl(y + FQ_L2PF) * pitch + cr[0]));
         float vxx[NC], vxy[NC], vyy[NC];
         __align__(16) float nxx[NC], nxy[NC], nyy[NC];
@@ -267,8 +266,9 @@ eigen_fast_quad_kernel(const float *__restrict__ img0, size_t img_stride, size_t
     }
 }
 
-template <int HH, int NC>
+template <int HH>
 static int launch_fast_quad(klt_ctx *ctx, const SelDev *S, int B, const float *img0, size_t img_stride, size_t pitch, const FastTaps &T) {
+    constexpr int NC = FQ_NC;
     constexpr int HL = (FS_R + HH + NC - 1) / NC, USE = (32 - 2 * HL) * NC;
     const int ncols = S->W - S->bx - (S->bx & ~(NC - 1)), nrows = S->H - 2 * S->by;
     if (S->W - 2 * S->bx <= 0 || nrows <= 0) return 1;
@@ -285,9 +285,9 @@ static int launch_fast_quad(klt_ctx *ctx, const SelDev *S, int B, const float *i
     const int vec_ok = (pitch % 4) == 0 && (img_stride % 4) == 0 && (reinterpret_cast<uintptr_t>(img0) & 15) == 0;
     const size_t smem = (size_t)(FS_THREADS / 32) * (2 * HH + 1) * 3 * 32 * NC * sizeof(float);      // <= 43 KB
     if (S->step == 1)
-        KLT_LAUNCH(ctx, "eigen_fast", bytes, (eigen_fast_quad_kernel<HH, NC, true><<<grid, FS_THREADS, smem, ctx->stream>>>(img0, img_stride, pitch, *S, T, rows, n_strips, vec_ok)));
+        KLT_LAUNCH(ctx, "eigen_fast", bytes, (eigen_fast_quad_kernel<HH, true><<<grid, FS_THREADS, smem, ctx->stream>>>(img0, img_stride, pitch, *S, T, rows, n_strips, vec_ok)));
     else
-        KLT_LAUNCH(ctx, "eigen_fast", bytes, (eigen_fast_quad_kernel<HH, NC, false><<<grid, FS_THREADS, smem, ctx->stream>>>(img0, img_stride, pitch, *S, T, rows, n_strips, vec_ok)));
+        KLT_LAUNCH(ctx, "eigen_fast", bytes, (eigen_fast_quad_kernel<HH, false><<<grid, FS_THREADS, smem, ctx->stream>>>(img0, img_stride, pitch, *S, T, rows, n_strips, vec_ok)));
     return 1;
 }
 
@@ -327,9 +327,9 @@ int klt_sel_launch_eigen_fast(klt_ctx *ctx, const SelDev *S, int B, const float 
         }
     }
     switch (S->hh) {
-        case 1: return ctx->fast_quad_nc == 2 ? launch_fast_quad<1, 2>(ctx, S, B, img0, img_stride, pitch, T) : launch_fast_quad<1, 4>(ctx, S, B, img0, img_stride, pitch, T);
-        case 2: return ctx->fast_quad_nc == 2 ? launch_fast_quad<2, 2>(ctx, S, B, img0, img_stride, pitch, T) : launch_fast_quad<2, 4>(ctx, S, B, img0, img_stride, pitch, T);
-        case 3: return ctx->fast_quad_nc == 2 ? launch_fast_quad<3, 2>(ctx, S, B, img0, img_stride, pitch, T) : launch_fast_quad<3, 4>(ctx, S, B, img0, img_stride, pitch, T);
+        case 1: return launch_fast_quad<1>(ctx, S, B, img0, img_stride, pitch, T);
+        case 2: return launch_fast_quad<2>(ctx, S, B, img0, img_stride, pitch, T);
+        case 3: return launch_fast_quad<3>(ctx, S, B, img0, img_stride, pitch, T);
         case 4: return launch_fast<4>(ctx, S, B, img0, img_stride, pitch, T);
         case 5: return launch_fast<5>(ctx, S, B, img0, img_stride, pitch, T);
         case 6: return launch_fast<6>(ctx, S, B, img0, img_stride, pitch, T);

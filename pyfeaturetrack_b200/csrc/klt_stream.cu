@@ -55,10 +55,6 @@ __device__ __forceinline__ void prefetch_l2(const void *p) { asm volatile("prefe
 
 // one I2F.U8 with a byte selector (conversion pipe, a quarter of the FMA rate -- plenty for 4..8 pixels per lane-row)
 __device__ __forceinline__ float u8_byte_to_f32(unsigned int word, int byte) { return (float)((word >> (8 * byte)) & 0xffu); }
-__device__ __forceinline__ float u8_to_f32(unsigned int word, int byte) {
-    // 0x4B000000 | b is the float 8388608 + b; exact for b in 0..255, and runs on the ALU/FMA pipes (no I2F)
-    return __uint_as_float(__byte_perm(word, 0x4B000000u, 0x7650u | (unsigned int)byte)) - 8388608.0f;
-}
 
 // vertical accumulate-and-shift: returns the completed output row value; acc[m] <- acc[m+1] + c[2R-1-m]*v
 template <int R>
@@ -214,104 +210,23 @@ stream_level0_kernel(const unsigned char *__restrict__ frames, size_t pitch, siz
 }
 
 // ---- level 0 of an image-only pyramid: u8 frame -> smoothed image (KLT_PRECISION_FAST_WINDOWED) -----------------------
-// Same strip/lane geometry as stream_level0_kernel without the gradient stage: 1 B read + 4 B written per pixel,
-// 2*(2*RS+1) FMAs.  With so little arithmetic per byte the kernel is bound by instruction issue, so the row loop is kept
-// minimal: each lane loads and converts only its own quad (the RS neighbour columns come from the adjacent lanes by
-// shuffle), and segments that do not touch the top/bottom border walk a running row pointer (no reflection arithmetic).
-// one input row of the smooth-only kernel; STORE = the vertical filter has seen 2*RS rows (output row t - RS is complete)
-template <int RS, bool INTERIOR, bool STORE>
-__device__ __forceinline__ void smooth0_row(const unsigned char *__restrict__ b0, const unsigned char *&pr, unsigned int &w0,
-                                            unsigned int sel0, unsigned int upitch, int H, int t, int t1, bool writer,
-                                            float *&p_img, int out_pitch, float (&sa)[4][2 * RS], const StreamTaps &T) {
-    const unsigned int q0 = __byte_perm(w0, 0u, sel0);
-    float u[4 + 2 * RS];
-    // I2F.U8 with a byte selector: one instruction per pixel on the conversion pipe, which this kernel leaves idle
-    // (the level-0 kernel with its 38 FMA/px keeps the two-instruction ALU form of u8_to_f32)
-#pragma unroll
-    for (int i = 0; i < 4; i++) u[RS + i] = u8_byte_to_f32(q0, i);
-    if (INTERIOR) {
-        pr += upitch;                                              // one row past the segment is still inside the image
-        w0 = __ldg(reinterpret_cast<const unsigned int *>(pr));
-        prefetch_l2(pr + (PREFETCH_ROWS - 1) * upitch);
-    } else {
-        w0 = __ldg(reinterpret_cast<const unsigned int *>(b0 + (unsigned int)reflect1(min(t + 1, t1 - 1), H) * upitch));
-        const int tp = t + PREFETCH_ROWS;
-        if (tp < t1) prefetch_l2(b0 + (unsigned int)reflect1(tp, H) * upitch);
-    }
-#pragma unroll
-    for (int k = 0; k < RS; k++) {
-        u[k] = __shfl_up_sync(FULLMASK, u[4 + k], 1);               // columns c-RS .. c-1: the left lane's last RS
-        u[RS + 4 + k] = __shfl_down_sync(FULLMASK, u[RS + k], 1);   // columns c+4 .. c+3+RS: the right lane's first RS
-    }
-    float s[4];
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-        float h = T.s[0] * u[i];
-#pragma unroll
-        for (int j = 1; j < 2 * RS + 1; j++) h = fmaf(T.s[j], u[i + j], h);
-        s[i] = vacc<RS>(sa[i], T.s, h);
-    }
-    if (STORE) {
-        if (writer) *reinterpret_cast<float4 *>(p_img) = make_float4(s[0], s[1], s[2], s[3]);
-        p_img += out_pitch;
-    }
-}
-
-template <int RS, bool INTERIOR>
-__device__ __forceinline__ void smooth0_rows(const unsigned char *__restrict__ b0, unsigned int sel0, unsigned int upitch, int H,
-                                             int ys, int t0, int t1, bool writer, float *p_img, int out_pitch,
-                                             const StreamTaps &T) {
-    float sa[4][2 * RS];
-#pragma unroll
-    for (int i = 0; i < 4; i++)
-#pragma unroll
-        for (int m = 0; m < 2 * RS; m++) sa[i][m] = 0.f;
-    const unsigned char *pr = b0 + (INTERIOR ? (size_t)t0 * upitch : (size_t)reflect1(t0, H) * upitch);
-    unsigned int w0 = __ldg(reinterpret_cast<const unsigned int *>(pr));
-    int t = t0;
-    for (; t < t0 + 2 * RS; t++)                       // warm-up rows: nothing to store yet (t - RS < ys)
-        smooth0_row<RS, INTERIOR, false>(b0, pr, w0, sel0, upitch, H, t, t1, writer, p_img, out_pitch, sa, T);
-#pragma unroll 2
-    for (; t < t1; t++)
-        smooth0_row<RS, INTERIOR, true>(b0, pr, w0, sel0, upitch, H, t, t1, writer, p_img, out_pitch, sa, T);
-}
-
-template <int RS>
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32, 8)
-stream_smooth0_kernel(const unsigned char *__restrict__ frames, size_t pitch, size_t frame_stride, float *__restrict__ img,
-                      int out_pitch, size_t out_stride, int W, int H, int rows_per_seg, int n_strips,
-                      const __grid_constant__ StreamTaps T) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int strip = blockIdx.x * WARPS_PER_CTA + warp;
-    if (strip >= n_strips) return;
-    const int ys = blockIdx.y * rows_per_seg, ye = min(H, ys + rows_per_seg);
-    const int c = strip * 120 + 4 * (lane - 1);
-    const unsigned char *src = frames + (size_t)blockIdx.z * frame_stride;
-    bool rv0;
-    const int m0 = mirror_quad(c, W, rv0);
-    const unsigned char *b0 = src + m0;
-    const unsigned int sel0 = rv0 ? 0x0123u : 0x3210u;
-    const bool writer = lane >= 1 && lane <= 30 && c < W;
-    float *p_img = img + (size_t)blockIdx.z * out_stride + (size_t)c + (size_t)ys * out_pitch;
-    const int t0 = ys - RS, t1 = ye + RS;
-    // interior: every row the loop loads or prefetches, [t0, t1 + PREFETCH_ROWS), lies inside the frame
-    if (t0 >= 0 && t1 + PREFETCH_ROWS <= H) smooth0_rows<RS, true>(b0, sel0, (unsigned int)pitch, H, ys, t0, t1, writer, p_img, out_pitch, T);
-    else smooth0_rows<RS, false>(b0, sel0, (unsigned int)pitch, H, ys, t0, t1, writer, p_img, out_pitch, T);
-}
-
-// ---- the same kernel, two strips per warp, packed arithmetic (round 2, second generation) -----------------------------
-// ncu showed stream_smooth0_kernel at 68 % of its issue slots with the FMA pipe at 37 % and DRAM at 62 % (65 instructions
-// per lane-row, 40 of them FFMA/FMUL), which read like an issue-bound kernel.  It is not: this version issues 30 % fewer
-// instructions and takes the same 123 us per 64 x 1080p, because a trivial kernel with the same 1 : 4 read/write mix and size
-// stops at 119 us (tools/mix_probe.cu, DESIGN "How close are the streaming kernels ...").  It stays as the default level-0-only
-// kernel (fewer instructions, less power) and as the first user of the packed idiom the fused kernel below depends on.
+// The strip/lane geometry of stream_level0_kernel without the gradient stage: 1 B read + 4 B written per pixel,
+// 2*(2*RS+1) FMAs.  With so little arithmetic per byte the row loop is kept minimal: each lane loads and converts only its own
+// quad (the RS neighbour columns come from the adjacent lanes by shuffle), and segments that do not touch the top/bottom
+// border walk a running row offset (no reflection arithmetic).
 // sm_100 has packed fp32 arithmetic (PTX fma.rn.f32x2, SASS
 // FFMA2: two FMAs per issue slot, a scalar multiplier may come from the uniform register file), so here one warp marches
 // down TWO adjacent strips A and B = A + 120 columns and every filter value lives in a 64-bit register pair (A, B):
 // the horizontal taps and the pending vertical sums are FFMA2s on such pairs, the conversions and shuffles write the two
 // halves of a pair directly (no packing moves), and the LAST vertical FMA of a row runs as two scalar FFMAs whose
 // destinations are the four consecutive registers each 128-bit store needs (no unpacking moves either): 44 floating
-// point instructions per 8 pixels instead of 80, 46 instead of 65 instructions per 4 pixels overall.
+// point instructions per 8 pixels instead of 80, 46 instead of 65 instructions per 4 pixels overall.  An image of one strip
+// (W <= 120) leaves strip B wholly outside: its loads are clamped into the image and its stores are off.
+// The instruction count is not what bounds this kernel: a scalar one-strip-per-warp version (30 % more instructions) and a
+// version with whole-row CTAs that stored through bulk copies took the same 123-124 us per 64 x 1080p on a B200, because a
+// trivial kernel with the same 1 : 4 read/write mix and size stops at 119 us (tools/mix_probe.cu, DESIGN "How close are the
+// streaming kernels ...").  This one stays for its fewer instructions (less power), and it is the first user of the packed
+// idiom the fused kernel below depends on.
 typedef unsigned long long f32x2;
 __device__ __forceinline__ f32x2 pack2(float a, float b) { f32x2 d; asm("mov.b64 %0, {%1, %2};" : "=l"(d) : "f"(a), "f"(b)); return d; }
 __device__ __forceinline__ float lo2(f32x2 v) { [[maybe_unused]] float a, b; asm("mov.b64 {%0, %1}, %2;" : "=f"(a), "=f"(b) : "l"(v)); return a; }
@@ -437,114 +352,6 @@ stream_smooth0x2_kernel(const unsigned char *__restrict__ frames, size_t pitch, 
         smooth0x2_rows<RS, false>(bA, bB, selA, selB, upitch, pf_delta, H, t0, t1, writerA, writerB, pA, pB, out_pitch, T);
 }
 
-// ---- third generation: one CTA owns whole rows and stores them with bulk copies -------------------------------------------
-// Cutting 30 % of the instructions changed nothing (123 us per 64 x 1080p before and after), so the next suspect was how
-// the stores reach DRAM: each warp of the kernels above writes a 480-byte piece per row and then jumps a whole image
-// row ahead, so the GPU emits ~4000 interleaved piece streams.  (Measured: 124 us again -- the shape of the store stream is
-// not the limit either; the read/write mix is.  Kept as an experiment, $KLT_B200_SMOOTH0=3, and as the default for wide images
-// the fused kernel does not cover.)  Here a CTA of 8 warps covers 1920 columns (a whole 1080p row),
-// the warps deposit their quads in a shared-memory ring, and after every ROWS_PER_GROUP rows one thread hands the group
-// to the bulk-copy engine (cp.async.bulk.global.shared::cta, SASS UBLKCP): the store stream of a CTA is then linear in
-// memory, KB at a time.  Three groups rotate: the group being filled, the one being copied, and one of slack, so a
-// single CTA barrier per group suffices (thread 0 waits for the copy before last to have left shared memory before it
-// arrives at the barrier that releases that slot).
-#define ROWCTA_WARPS 8
-#define ROWS_PER_GROUP 4
-#define ROWCTA_GROUPS 3
-#define ROWCTA_COLS (ROWCTA_WARPS * 240)
-
-__device__ __forceinline__ void bulk_store_row_group(float *gdst, const float *ssrc, unsigned int bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst),
-                 "r"((unsigned int)__cvta_generic_to_shared(ssrc)), "r"(bytes)
-                 : "memory");
-}
-
-template <int RS, bool INTERIOR>
-__device__ __forceinline__ void smooth0r_rows(const unsigned char *__restrict__ bA, const unsigned char *__restrict__ bB,
-                                              unsigned int selA, unsigned int selB, unsigned int upitch, unsigned int pf_delta,
-                                              int H, int t0, int t1, bool writerA, bool writerB, float *smem,
-                                              int colA, int cta_cols, float *gout, int out_pitch, const StreamTaps &T) {
-    f32x2 sa[4][2 * RS];
-#pragma unroll
-    for (int i = 0; i < 4; i++)
-#pragma unroll
-        for (int m = 0; m < 2 * RS; m++) sa[i][m] = 0ull;
-    unsigned int offs = (unsigned int)(INTERIOR ? t0 : reflect1(t0, H)) * upitch;
-    unsigned int wA = __ldg(reinterpret_cast<const unsigned int *>(bA + offs));
-    unsigned int wB = __ldg(reinterpret_cast<const unsigned int *>(bB + offs));
-    int t = t0;
-    float *pA = smem + colA, *pB = pA + 120;
-    for (; t < t0 + 2 * RS; t++)                       // warm-up rows: nothing to store yet
-        smooth0x2_row<RS, INTERIOR, false>(bA, bB, offs, wA, wB, selA, selB, upitch, pf_delta, H, t, t1, writerA, writerB, pA, pB,
-                                           cta_cols, sa, T);
-    const bool contiguous = out_pitch == cta_cols;     // the CTA's rows follow each other in memory: one copy per group
-    int g = 0;
-    while (t < t1) {
-        const int nrows = min(ROWS_PER_GROUP, t1 - t);
-        float *slot = smem + (size_t)(g % ROWCTA_GROUPS) * ROWS_PER_GROUP * cta_cols;
-        pA = slot + colA;
-        pB = pA + 120;
-        if (nrows == ROWS_PER_GROUP) {
-#pragma unroll
-            for (int k = 0; k < ROWS_PER_GROUP; k++)
-                smooth0x2_row<RS, INTERIOR, true>(bA, bB, offs, wA, wB, selA, selB, upitch, pf_delta, H, t + k, t1, writerA, writerB,
-                                                  pA, pB, cta_cols, sa, T);
-        } else {
-            for (int k = 0; k < nrows; k++)
-                smooth0x2_row<RS, INTERIOR, true>(bA, bB, offs, wA, wB, selA, selB, upitch, pf_delta, H, t + k, t1, writerA, writerB,
-                                                  pA, pB, cta_cols, sa, T);
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy writes -> visible to the copy engine
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            if (contiguous) bulk_store_row_group(gout, slot, (unsigned int)(nrows * cta_cols * 4));
-            else
-                for (int k = 0; k < nrows; k++)
-                    bulk_store_row_group(gout + (size_t)k * out_pitch, slot + (size_t)k * cta_cols, (unsigned int)(cta_cols * 4));
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");   // the group before this one has left its slot
-        }
-        gout += (size_t)nrows * out_pitch;
-        t += nrows;
-        g++;
-    }
-    if (threadIdx.x == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-}
-
-template <int RS>
-__global__ void __launch_bounds__(ROWCTA_WARPS * 32, 2)
-stream_smooth0r_kernel(const unsigned char *__restrict__ frames, size_t pitch, size_t frame_stride, float *__restrict__ img,
-                       int out_pitch, size_t out_stride, int W, int H, int rows_per_seg, int n_pairs,
-                       const __grid_constant__ StreamTaps T) {
-    extern __shared__ __align__(128) float rowcta_smem[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    // strips 2 * pair (A) and 2 * pair + 1 (B); warps past the last pair of a narrow image run along on clamped addresses
-    // with their writers off (every warp must reach the CTA barriers)
-    const int pair = blockIdx.x * ROWCTA_WARPS + warp;
-    const int ys = blockIdx.y * rows_per_seg, ye = min(H, ys + rows_per_seg);
-    const int base = blockIdx.x * ROWCTA_COLS;                    // first column of this CTA's rows
-    const int cta_cols = min(W - base, ROWCTA_COLS);
-    const int cA = pair * 240 + 4 * (lane - 1), cB = cA + 120;
-    const unsigned char *src = frames + (size_t)blockIdx.z * frame_stride;
-    bool rvA, rvB;
-    const int mA = mirror_quad(cA, W, rvA), mB = mirror_quad(cB, W, rvB);
-    const unsigned char *bA = src + mA, *bB = src + mB;
-    const unsigned int selA = rvA ? 0x0123u : 0x3210u, selB = rvB ? 0x0123u : 0x3210u;
-    const bool inner = lane >= 1 && lane <= 30;
-    const bool writerA = inner && cA < W, writerB = inner && cB < W;
-    float *gout = img + (size_t)blockIdx.z * out_stride + (size_t)ys * out_pitch + base;
-    const int t0 = ys - RS, t1 = ye + RS;
-    const unsigned int upitch = (unsigned int)pitch;
-    const int pc = min(max(pair * 240 - 4 + 8 * lane, 0), W - 4);
-    const unsigned int pf_delta = (PREFETCH_ROWS - 1) * upitch + (unsigned int)(pc - mA);
-    if (t0 >= 0 && t1 + PREFETCH_ROWS <= H)
-        smooth0r_rows<RS, true>(bA, bB, selA, selB, upitch, pf_delta, H, t0, t1, writerA, writerB, rowcta_smem, cA - base,
-                                cta_cols, gout, out_pitch, T);
-    else
-        smooth0r_rows<RS, false>(bA, bB, selA, selB, upitch, pf_delta, H, t0, t1, writerA, writerB, rowcta_smem, cA - base,
-                                 cta_cols, gout, out_pitch, T);
-}
-
 // ---- gradients only: float image -> gradx, grady (levels >= 1) ---------------------------------------------------
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32, 4)
 stream_grad_kernel(const float *__restrict__ in, int in_pitch, size_t in_stride, float *__restrict__ gxo,
@@ -591,108 +398,9 @@ stream_grad_kernel(const float *__restrict__ in, int in_pitch, size_t in_stride,
 // ---- pyramid step for subsampling 2: out[Y][X] = smooth11(in)[2Y+1][2X+1] -----------------------------------------
 // Lane l owns output columns X..X+3, X = 120*strip + 4*(l-1), i.e. input columns ci = 2X .. ci+7; it needs ci-4 .. ci+12.
 // Lanes 0 and 31 only feed their neighbours.  Vertical: input rows arrive in (even, odd) pairs; output Y completes with
-// even row 2Y+6.  Five partial outputs are pending per column; 11 FMAs per column per output row, no moves.
-struct RowPair { float4 ea, eb, oa, ob; };   // even row: quads at ci, ci+4; odd row: the same
-
-__device__ __forceinline__ void down2_hrow(const StreamTaps &T, float4 a, float4 b, bool warp_rev, bool rva, bool rvb,
-                                           float (&h)[4]) {
-    if (warp_rev) {                                  // warp-uniform: only warps touching an image edge reverse quads
-        if (rva) a = make_float4(a.w, a.z, a.y, a.x);
-        if (rvb) b = make_float4(b.w, b.z, b.y, b.x);
-    }
-    float e[17];                                     // input columns ci-4 .. ci+12
-    e[4] = a.x; e[5] = a.y; e[6] = a.z; e[7] = a.w; e[8] = b.x; e[9] = b.y; e[10] = b.z; e[11] = b.w;
-    e[0] = __shfl_up_sync(FULLMASK, b.x, 1); e[1] = __shfl_up_sync(FULLMASK, b.y, 1);
-    e[2] = __shfl_up_sync(FULLMASK, b.z, 1); e[3] = __shfl_up_sync(FULLMASK, b.w, 1);
-    e[12] = __shfl_down_sync(FULLMASK, a.x, 1); e[13] = __shfl_down_sync(FULLMASK, a.y, 1);
-    e[14] = __shfl_down_sync(FULLMASK, a.z, 1); e[15] = __shfl_down_sync(FULLMASK, a.w, 1);
-    e[16] = __shfl_down_sync(FULLMASK, b.x, 1);
-#pragma unroll
-    for (int i = 0; i < 4; i++) {                    // output column X+i is centred on input column ci + 2i + 1
-        float acc = T.p[0] * e[2 * i];
-#pragma unroll
-        for (int j = 1; j < 11; j++) acc = fmaf(T.p[j], e[2 * i + j], acc);
-        h[i] = acc;
-    }
-}
-
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32, 4)
-stream_down2_kernel(const float *__restrict__ in, int in_pitch, size_t in_stride, int W, int H, float *__restrict__ out,
-                    int out_pitch, size_t out_stride, int OW, int OH, int rows_per_seg, int n_strips,
-                    const __grid_constant__ StreamTaps T) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int strip = blockIdx.x * WARPS_PER_CTA + warp;
-    if (strip >= n_strips) return;
-    const int ys = blockIdx.y * rows_per_seg, ye = min(OH, ys + rows_per_seg);
-    const int X = strip * 120 + 4 * (lane - 1);
-    const int ci = 2 * X;
-    const float *src = in + (size_t)blockIdx.z * in_stride;
-    bool rva, rvb;
-    const int ma = mirror_quad(ci, W, rva), mb = mirror_quad(ci + 4, W, rvb);
-    const bool writer = lane >= 1 && lane <= 30 && X < OW;
-    float *p_out = out + (size_t)blockIdx.z * out_stride + (size_t)ys * out_pitch + X;
-
-    float P[4][5];
-#pragma unroll
-    for (int i = 0; i < 4; i++)
-#pragma unroll
-        for (int m = 0; m < 5; m++) P[i][m] = 0.f;
-
-    auto load_pair = [&](int j, RowPair &rp) {
-        const float *re = src + (size_t)reflect1(2 * j, H) * in_pitch, *ro = src + (size_t)reflect1(2 * j + 1, H) * in_pitch;
-        rp.ea = __ldg(reinterpret_cast<const float4 *>(re + ma)); rp.eb = __ldg(reinterpret_cast<const float4 *>(re + mb));
-        rp.oa = __ldg(reinterpret_cast<const float4 *>(ro + ma)); rp.ob = __ldg(reinterpret_cast<const float4 *>(ro + mb));
-    };
-    // c[j] multiplies in[2Y+1 + j - 5]; input row r contributes to output Y with j = r - 2Y + 4
-    const int j0 = ys - 2, j1 = ye + 3;                  // pair j: rows 2j, 2j+1; even row 2j completes output Y = j - 3
-    const bool warp_rev = __any_sync(FULLMASK, rva || rvb);
-    auto step = [&](const RowPair &cur, int j) {
-        float he[4], ho[4];
-        down2_hrow(T, cur.ea, cur.eb, warp_rev, rva, rvb, he);
-        down2_hrow(T, cur.oa, cur.ob, warp_rev, rva, rvb, ho);
-        float o[4];
-#pragma unroll
-        for (int i = 0; i < 4; i++) {
-            // even row 2j: outputs Y=j-3..j+2 take taps 10, 8, 6, 4, 2, 0; odd row 2j+1: Y=j-2..j+2 take 9, 7, 5, 3, 1
-            o[i] = fmaf(T.p[10], he[i], P[i][0]);
-            const float a0 = fmaf(T.p[8], he[i], P[i][1]);
-            const float a1 = fmaf(T.p[6], he[i], P[i][2]);
-            const float a2 = fmaf(T.p[4], he[i], P[i][3]);
-            const float a3 = fmaf(T.p[2], he[i], P[i][4]);
-            const float a4 = T.p[0] * he[i];
-            P[i][0] = fmaf(T.p[9], ho[i], a0);
-            P[i][1] = fmaf(T.p[7], ho[i], a1);
-            P[i][2] = fmaf(T.p[5], ho[i], a2);
-            P[i][3] = fmaf(T.p[3], ho[i], a3);
-            P[i][4] = fmaf(T.p[1], ho[i], a4);
-        }
-        if (j - 3 >= ys) {                               // Y = j - 3 < ye by construction
-            if (writer) *reinterpret_cast<float4 *>(p_out) = make_float4(o[0], o[1], o[2], o[3]);
-            p_out += out_pitch;
-        }
-        if (j + 3 < j1) {
-            prefetch_l2(src + (size_t)reflect1(2 * j + 6, H) * in_pitch + ma);
-            prefetch_l2(src + (size_t)reflect1(2 * j + 7, H) * in_pitch + ma);
-        }
-    };
-    // two row-pair buffers, loop unrolled by two: each buffer is reloaded right after it has been consumed, one full
-    // step before its next use, without register-to-register copies
-    RowPair A, B;
-    load_pair(j0, A);
-    load_pair(min(j0 + 1, j1 - 1), B);
-    for (int j = j0; j < j1; j += 2) {
-        step(A, j);
-        load_pair(min(j + 2, j1 - 1), A);
-        if (j + 1 < j1) {
-            step(B, j + 1);
-            load_pair(min(j + 3, j1 - 1), B);
-        }
-    }
-}
-
-// ---- the same step on packed arithmetic (round 2, second generation) ------------------------------------------------------
-// stream_down2_kernel issues ~225 instructions per lane and row pair (4 output pixels), 132 of them FFMA/FMUL, at 60-65 % of
-// the issue slots with DRAM at 63-72 % (ncu): co-limited.  This version keeps the geometry and cuts the issue slots:
+// even row 2Y+6; five partial outputs are pending per column.  A scalar form of this step issues ~225 instructions per lane
+// and row pair (4 output pixels), 132 of them FFMA/FMUL, and measured co-limited by issue (60-65 % of the slots) and DRAM
+// (63-72 %), so the arithmetic is packed:
 //   * horizontal: the 128-bit loads deliver even-aligned column pairs (e[2k], e[2k+1]) in adjacent registers, so taps
 //     (p[2m], p[2m+1]) are applied to such pairs with one FFMA2 (per-half multipliers), the two halves are added at the end
 //     and the eleventh tap is a scalar FMA: 7 instead of 11 instructions per output and input row;
@@ -700,8 +408,10 @@ stream_down2_kernel(const float *__restrict__ in, int in_pitch, size_t in_stride
 //     (11 instead of 22 per row pair and column pair); the completed pairs are the four consecutive registers of the store;
 //   * segments whose rows (including the look-ahead loads and prefetches) lie inside the image walk running pointers
 //     instead of reflecting and multiplying row indices.
-// 78 floating-point instructions per row pair instead of 132.  The sums are associated differently from the scalar kernel
+// 78 floating-point instructions per row pair instead of 132.  The sums are associated differently from a plain 11-tap sum
 // (even and odd taps separately), so the two agree to rounding (~1e-7 relative), not bit for bit.
+struct RowPair { float4 ea, eb, oa, ob; };   // even row: quads at ci, ci+4; odd row: the same
+
 __device__ __forceinline__ f32x2 fma2v(f32x2 c, f32x2 v, f32x2 acc) {
     f32x2 d;
     asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(c), "l"(v), "l"(acc));
@@ -980,37 +690,30 @@ __device__ __forceinline__ void l01_rows(const unsigned char *__restrict__ b0, u
     }
 }
 
-// two register budgets of the same kernel: 128 registers = 8 CTAs of 2 warps per SM (the default: 166 us per 64 x 1080p),
-// 112 = 9 CTAs with a few spills (170 us: more warps do not help, the kernel is near its traffic mix's ceiling);
-// $KLT_B200_L01_REGS=112 picks the second (A/B runs)
-#define KLT_DEFINE_LEVEL01(NAME, MAXREG) \
-__global__ void __maxnreg__(MAXREG) \
-NAME(const unsigned char *__restrict__ frames, size_t pitch, size_t frame_stride, float *__restrict__ img0, \
-                      int pitch0, float *__restrict__ img1, int pitch1, size_t out_stride, int W, int H, int OW, int OH, \
-                      int rows_per_seg, int n_strips, int pf_rows, const __grid_constant__ StreamTaps T) { \
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5; \
-    const int strip = blockIdx.x * L01_WARPS + warp; \
-    if (strip >= n_strips) return; \
-    const int ys = blockIdx.y * rows_per_seg, ye = min(OH, ys + rows_per_seg); \
-    const int c0 = strip * 240 + 8 * (lane - 1), X = strip * 120 + 4 * (lane - 1); \
-    bool rev; \
-    const int m0 = mirror_oct(c0, W, rev); \
-    const unsigned char *b0 = frames + (size_t)blockIdx.z * frame_stride + m0; \
-    const unsigned int selx = rev ? 0x4567u : 0x3210u, sely = rev ? 0x0123u : 0x7654u; \
-    const bool inner = lane >= 1 && lane <= 30; \
-    const bool writer0 = inner && c0 < W, writer1 = inner && X < OW; \
-    const int r_end = ye == OH ? H : 2 * ye; \
- \
- \
-    float *p0 = img0 + (size_t)blockIdx.z * out_stride + c0 + ((ptrdiff_t)2 * (ys - 2)) * pitch0; \
-    float *p1 = img1 + (size_t)blockIdx.z * out_stride + (size_t)ys * pitch1 + X; \
- \
-    const int t0 = 2 * (ys - 2) - 2, t_end = 2 * (ye + 2) + 3 + 2 + 2 + pf_rows; \
-    if (t0 >= 0 && t_end < H) l01_rows<true>(b0, selx, sely, (unsigned int)pitch, H, ys, ye, r_end, writer0, writer1, p0, pitch0, p1, pitch1, pf_rows, T); \
-    else l01_rows<false>(b0, selx, sely, (unsigned int)pitch, H, ys, ye, r_end, writer0, writer1, p0, pitch0, p1, pitch1, pf_rows, T); \
+// 128 registers = 8 CTAs of 2 warps per SM: 166 us per 64 x 1080p on a B200.  A 112-register budget (9 CTAs, a few spills)
+// measured 170 us: more warps do not help, the kernel is near its traffic mix's ceiling.
+__global__ void __maxnreg__(128)
+stream_level01_kernel(const unsigned char *__restrict__ frames, size_t pitch, size_t frame_stride, float *__restrict__ img0,
+                      int pitch0, float *__restrict__ img1, int pitch1, size_t out_stride, int W, int H, int OW, int OH,
+                      int rows_per_seg, int n_strips, int pf_rows, const __grid_constant__ StreamTaps T) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int strip = blockIdx.x * L01_WARPS + warp;
+    if (strip >= n_strips) return;
+    const int ys = blockIdx.y * rows_per_seg, ye = min(OH, ys + rows_per_seg);
+    const int c0 = strip * 240 + 8 * (lane - 1), X = strip * 120 + 4 * (lane - 1);
+    bool rev;
+    const int m0 = mirror_oct(c0, W, rev);
+    const unsigned char *b0 = frames + (size_t)blockIdx.z * frame_stride + m0;
+    const unsigned int selx = rev ? 0x4567u : 0x3210u, sely = rev ? 0x0123u : 0x7654u;
+    const bool inner = lane >= 1 && lane <= 30;
+    const bool writer0 = inner && c0 < W, writer1 = inner && X < OW;
+    const int r_end = ye == OH ? H : 2 * ye;
+    float *p0 = img0 + (size_t)blockIdx.z * out_stride + c0 + ((ptrdiff_t)2 * (ys - 2)) * pitch0;
+    float *p1 = img1 + (size_t)blockIdx.z * out_stride + (size_t)ys * pitch1 + X;
+    const int t0 = 2 * (ys - 2) - 2, t_end = 2 * (ye + 2) + 3 + 2 + 2 + pf_rows;
+    if (t0 >= 0 && t_end < H) l01_rows<true>(b0, selx, sely, (unsigned int)pitch, H, ys, ye, r_end, writer0, writer1, p0, pitch0, p1, pitch1, pf_rows, T);
+    else l01_rows<false>(b0, selx, sely, (unsigned int)pitch, H, ys, ye, r_end, writer0, writer1, p0, pitch0, p1, pitch1, pf_rows, T);
 }
-KLT_DEFINE_LEVEL01(stream_level01_kernel, 128)
-KLT_DEFINE_LEVEL01(stream_level01_r112_kernel, 112)
 
 // ---- pyramid step for subsampling SS with a (2R+1)-tap gauss, generic form of the kernel above ------------------------
 // (used for SS = 4, R = 10: the reference's DEFAULT pyramid, sigma = 0.9 * 4 -> 21 taps).
@@ -1205,104 +908,35 @@ int klt_stream_smooth0(klt_ctx *ctx, const uint8_t *frames, size_t pitch, size_t
     const int n_strips = (W + 119) / 120;
     const double bytes = 5.0 * W * H * count;         // 1 B read + 4 B written per pixel
     float *img = p->level(0, first, 0);
-    // generations: 3 = whole-row CTAs with bulk stores, 2 = two strips per warp on packed arithmetic, 1 = one strip per warp;
-    // $KLT_B200_SMOOTH0 = 1 / 2 / 3 forces one (A/B runs)
-    static const int forced_gen = [] { const char *e = getenv("KLT_B200_SMOOTH0"); return e && e[0] >= '1' && e[0] <= '3' ? e[0] - '0' : 0; }();
-    const int gen = forced_gen ? (forced_gen == 3 && RS > 2 ? 2 : forced_gen) : (W >= 960 && RS <= 2 ? 3 : 2);
-    const bool one_strip = gen == 1;
-    if (gen == 3 && n_strips >= 2) {
-        const int n_pairs = (n_strips + 1) / 2;
-        const int row_ctas = (n_pairs + ROWCTA_WARPS - 1) / ROWCTA_WARPS;
-        const int cols = W < ROWCTA_COLS ? W : ROWCTA_COLS;
-        const size_t smem = (size_t)ROWCTA_GROUPS * ROWS_PER_GROUP * cols * sizeof(float);
-        const void *fn = RS == 1 ? (const void *)stream_smooth0r_kernel<1> : RS == 2 ? (const void *)stream_smooth0r_kernel<2>
-                       : RS == 3 ? (const void *)stream_smooth0r_kernel<3> : (const void *)stream_smooth0r_kernel<4>;
-        static bool attr_set[5] = {false, false, false, false, false};
-        if (!attr_set[RS]) {
-            KLT_CUDA(ctx, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, ROWCTA_GROUPS * ROWS_PER_GROUP * ROWCTA_COLS * (int)sizeof(float)));
-            attr_set[RS] = true;
-        }
-        int per_sm = 2;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, ROWCTA_WARPS * 32, smem) != cudaSuccess || per_sm < 1) {
-            cudaGetLastError();
-            per_sm = 1;
-        }
-        long nseg = (long)ctx->num_sms * per_sm / ((long)row_ctas * count);
-        if (nseg < 1) nseg = 1;
-        long rows3 = (H + nseg - 1) / nseg;
-        if (rows3 < 32) rows3 = 32;
-        static const int forced_rows = [] { const char *e = getenv("KLT_B200_S0_ROWS"); return e ? atoi(e) : 0; }();   // experiments
-        if (forced_rows > 0) rows3 = forced_rows;
-        if (rows3 > H) rows3 = H;
-        dim3 grid3(row_ctas, (H + (int)rows3 - 1) / (int)rows3, count), block3(ROWCTA_WARPS * 32);
-#define LAUNCH_S0R(R)                                                                                                  \
-    KLT_LAUNCH(ctx, "stream_smooth0", bytes,                                                                           \
-               (stream_smooth0r_kernel<R><<<grid3, block3, smem, ctx->stream>>>(frames, pitch, frame_stride, img,       \
-                                                                                p->lv[0].pitch, p->plane_floats, W, H, \
-                                                                                (int)rows3, n_pairs, T)))
-        switch (RS) {
-            case 1: LAUNCH_S0R(1); break;
-            case 2: LAUNCH_S0R(2); break;
-            case 3: LAUNCH_S0R(3); break;
-            default: LAUNCH_S0R(4); break;
-        }
-#undef LAUNCH_S0R
-        return 1;
-    }
-    if (!one_strip && n_strips >= 2) {
-        const int n_pairs = (n_strips + 1) / 2;
-        const int pair_ctas = (n_pairs + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
-        int rows2 = 0;
-        switch (RS) {
-            case 1: rows2 = pick_rows_per_seg(ctx, stream_smooth0x2_kernel<1>, H, pair_ctas, count, 32); break;
-            case 2: rows2 = pick_rows_per_seg(ctx, stream_smooth0x2_kernel<2>, H, pair_ctas, count, 32); break;
-            case 3: rows2 = pick_rows_per_seg(ctx, stream_smooth0x2_kernel<3>, H, pair_ctas, count, 32); break;
-            default: rows2 = pick_rows_per_seg(ctx, stream_smooth0x2_kernel<4>, H, pair_ctas, count, 32); break;
-        }
-        dim3 grid2(pair_ctas, (H + rows2 - 1) / rows2, count), block2(WARPS_PER_CTA * 32);
-#define LAUNCH_S0X2(R)                                                                                                 \
-    KLT_LAUNCH(ctx, "stream_smooth0", bytes,                                                                           \
-               (stream_smooth0x2_kernel<R><<<grid2, block2, 0, ctx->stream>>>(frames, pitch, frame_stride, img,         \
-                                                                              p->lv[0].pitch, p->plane_floats, W, H,   \
-                                                                              rows2, n_pairs, T)))
-        switch (RS) {
-            case 1: LAUNCH_S0X2(1); break;
-            case 2: LAUNCH_S0X2(2); break;
-            case 3: LAUNCH_S0X2(3); break;
-            default: LAUNCH_S0X2(4); break;
-        }
-#undef LAUNCH_S0X2
-        return 1;
-    }
-    const int strip_ctas = (n_strips + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
+    const int n_pairs = (n_strips + 1) / 2;
+    const int pair_ctas = (n_pairs + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
     int rows = 0;
     switch (RS) {
-        case 1: rows = pick_rows_per_seg(ctx, stream_smooth0_kernel<1>, H, strip_ctas, count, 32); break;
-        case 2: rows = pick_rows_per_seg(ctx, stream_smooth0_kernel<2>, H, strip_ctas, count, 32); break;
-        case 3: rows = pick_rows_per_seg(ctx, stream_smooth0_kernel<3>, H, strip_ctas, count, 32); break;
-        default: rows = pick_rows_per_seg(ctx, stream_smooth0_kernel<4>, H, strip_ctas, count, 32); break;
+        case 1: rows = pick_rows_per_seg(ctx, stream_smooth0x2_kernel<1>, H, pair_ctas, count, 32); break;
+        case 2: rows = pick_rows_per_seg(ctx, stream_smooth0x2_kernel<2>, H, pair_ctas, count, 32); break;
+        case 3: rows = pick_rows_per_seg(ctx, stream_smooth0x2_kernel<3>, H, pair_ctas, count, 32); break;
+        default: rows = pick_rows_per_seg(ctx, stream_smooth0x2_kernel<4>, H, pair_ctas, count, 32); break;
     }
-    dim3 grid(strip_ctas, (H + rows - 1) / rows, count), block(WARPS_PER_CTA * 32);
-#define LAUNCH_S0(R)                                                                                                   \
+    dim3 grid(pair_ctas, (H + rows - 1) / rows, count), block(WARPS_PER_CTA * 32);
+#define LAUNCH_S0X2(R)                                                                                                 \
     KLT_LAUNCH(ctx, "stream_smooth0", bytes,                                                                           \
-               (stream_smooth0_kernel<R><<<grid, block, 0, ctx->stream>>>(frames, pitch, frame_stride, img, p->lv[0].pitch, \
-                                                                          p->plane_floats, W, H, rows, n_strips, T)))
+               (stream_smooth0x2_kernel<R><<<grid, block, 0, ctx->stream>>>(frames, pitch, frame_stride, img,           \
+                                                                            p->lv[0].pitch, p->plane_floats, W, H,     \
+                                                                            rows, n_pairs, T)))
     switch (RS) {
-        case 1: LAUNCH_S0(1); break;
-        case 2: LAUNCH_S0(2); break;
-        case 3: LAUNCH_S0(3); break;
-        case 4: LAUNCH_S0(4); break;
-        default: return 0;
+        case 1: LAUNCH_S0X2(1); break;
+        case 2: LAUNCH_S0X2(2); break;
+        case 3: LAUNCH_S0X2(3); break;
+        default: LAUNCH_S0X2(4); break;
     }
-#undef LAUNCH_S0
+#undef LAUNCH_S0X2
     return 1;
 }
 
 // levels 0 and 1 of an image-only pyramid in one launch; returns 0 when the configuration is not covered
 int klt_stream_level01(klt_ctx *ctx, const uint8_t *frames, size_t pitch, size_t frame_stride, klt_pyr *p,
                        const klt_taps *taps, int first, int count) {
-    static const bool disabled = [] { const char *e = getenv("KLT_B200_FUSED01"); return e && e[0] == '0'; }();
-    if (disabled || p->n_levels < 2 || p->ss != 2) return 0;
+    if (p->n_levels < 2 || p->ss != 2) return 0;
     StreamTaps T;
     if (taps->smooth.n != 5 || !is_symmetric(&taps->smooth) || !fill_taps(&taps->smooth, T.s, 5)) return 0;
     if (taps->pyramid.n > 11 || !fill_taps(&taps->pyramid, T.p, 11)) return 0;
@@ -1317,11 +951,9 @@ int klt_stream_level01(klt_ctx *ctx, const uint8_t *frames, size_t pitch, size_t
     if ((reinterpret_cast<uintptr_t>(img0) & 31) || (a.pitch & 7) || (p->plane_floats & 7) || !aligned16(img1)) return 0;
     const int n_strips = (W + 239) / 240;
     const int strip_ctas = (n_strips + L01_WARPS - 1) / L01_WARPS;
-    static const int pf_rows = [] { const char *e = getenv("KLT_B200_L01_PF"); const int v = e ? atoi(e) : 0; return v > 0 && v <= 64 ? v : 4; }();
-    static const bool r112 = [] { const char *e = getenv("KLT_B200_L01_REGS"); return e && atoi(e) == 112; }();
-    auto kernel = r112 ? stream_level01_r112_kernel : stream_level01_kernel;
+    const int pf_rows = 4;                             // L2 prefetch distance in frame rows
     int per_sm = 8;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, L01_WARPS * 32, 0) != cudaSuccess || per_sm < 1) {
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, stream_level01_kernel, L01_WARPS * 32, 0) != cudaSuccess || per_sm < 1) {
         cudaGetLastError();
         per_sm = 8;
     }
@@ -1333,7 +965,7 @@ int klt_stream_level01(klt_ctx *ctx, const uint8_t *frames, size_t pitch, size_t
     dim3 grid(strip_ctas, (b.h + rows - 1) / rows, count), block(L01_WARPS * 32);
     const double bytes = (5.0 * W * H + 4.0 * b.w * b.h) * count;     // 1 B read, 4 B + 1 B (a quarter of 4 B) written per pixel
     KLT_LAUNCH(ctx, "stream_level01", bytes,
-               (kernel<<<grid, block, 0, ctx->stream>>>(frames, pitch, frame_stride, img0, a.pitch, img1, b.pitch,
+               (stream_level01_kernel<<<grid, block, 0, ctx->stream>>>(frames, pitch, frame_stride, img0, a.pitch, img1, b.pitch,
                                                                        p->plane_floats, W, H, b.w, b.h, rows, n_strips, pf_rows, T)));
     return 1;
 }
@@ -1395,23 +1027,12 @@ int klt_stream_down2(klt_ctx *ctx, klt_pyr *p, int level, const klt_taps *taps, 
     const int n_strips = (b.w + 119) / 120;
     const int strip_ctas = (n_strips + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
     const double bytes = 4.0 * ((double)a.w * a.h + (double)b.w * b.h) * count;
-    // second generation on packed arithmetic; $KLT_B200_DOWN2=1 keeps the scalar kernel (A/B runs)
-    static const bool scalar_kernel = [] { const char *e = getenv("KLT_B200_DOWN2"); return e && e[0] == '1'; }();
-    if (!scalar_kernel) {
-        int rows2 = pick_rows_per_seg(ctx, stream_down2p_kernel, b.h, strip_ctas, count, 8);
-        if (!(rows2 & 1) && rows2 < b.h) rows2++;        // rows + 5 row pairs per segment: even, so no extra leading pair
-        dim3 grid2(strip_ctas, (b.h + rows2 - 1) / rows2, count), block2(WARPS_PER_CTA * 32);
-        KLT_LAUNCH(ctx, "stream_down2", bytes,
-                   (stream_down2p_kernel<<<grid2, block2, 0, ctx->stream>>>(p->level(0, first, level - 1), a.pitch, p->plane_floats,
-                                                                            a.w, a.h, p->level(0, first, level), b.pitch,
-                                                                            p->plane_floats, b.w, b.h, rows2, n_strips, T)));
-        return 1;
-    }
-    const int rows = pick_rows_per_seg(ctx, stream_down2_kernel, b.h, strip_ctas, count, 8);
+    int rows = pick_rows_per_seg(ctx, stream_down2p_kernel, b.h, strip_ctas, count, 8);
+    if (!(rows & 1) && rows < b.h) rows++;           // rows + 5 row pairs per segment: even, so no extra leading pair
     dim3 grid(strip_ctas, (b.h + rows - 1) / rows, count), block(WARPS_PER_CTA * 32);
     KLT_LAUNCH(ctx, "stream_down2", bytes,
-               (stream_down2_kernel<<<grid, block, 0, ctx->stream>>>(p->level(0, first, level - 1), a.pitch, p->plane_floats, a.w,
-                                                                     a.h, p->level(0, first, level), b.pitch, p->plane_floats, b.w,
-                                                                     b.h, rows, n_strips, T)));
+               (stream_down2p_kernel<<<grid, block, 0, ctx->stream>>>(p->level(0, first, level - 1), a.pitch, p->plane_floats,
+                                                                      a.w, a.h, p->level(0, first, level), b.pitch,
+                                                                      p->plane_floats, b.w, b.h, rows, n_strips, T)));
     return 1;
 }

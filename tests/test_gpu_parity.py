@@ -143,33 +143,14 @@ def test_pyramid_build_u8(gpu_ctx, oracle, cfg):
     pyr.close()
 
 
-_GEN_PROBE = r"""
-import sys, zlib, numpy as np
-sys.path.insert(0, %r)
-from pyfeaturetrack_b200 import _capi, klt, trackFeatures
-ctx = _capi.default_ctx()
-out = []
-for (H, W, L, batch) in [(1080, 1920, 3, 5), (200, 360, 2, 2), (64, 248, 2, 1), (540, 964, 3, 3)]:
-    frames = (np.random.default_rng(H + W).random((batch, H, W)) * 255).astype(np.uint8)
-    tc = klt.KLT_TrackingContext(); tc.nPyramidLevels, tc.subsampling = L, 2; tc.KLTUpdateTCBorder()
-    pyr = _capi.Pyramid(ctx, W, H, L, 2, batch)
-    pyr.build_u8(frames, trackFeatures._taps_for_one_image(tc), _capi.PRECISION_FAST_WINDOWED)
-    for b in range(batch):
-        for l in range(L):
-            a = pyr.download(0, l, b)
-            out.append((l, zlib.crc32(a.tobytes()), float(a.sum(dtype=np.float64)), float(np.abs(a).max())))
-    pyr.close()
-print(repr(out))
-"""
-
-
 @pytest.mark.parametrize("cfg", [dict(shape=(1080, 1920), L=3, batch=3), dict(shape=(200, 360), L=2, batch=2),
                                  dict(shape=(64, 248), L=2, batch=1), dict(shape=(540, 964), L=3, batch=2),
-                                 dict(shape=(2160, 3840), L=4, batch=1), dict(shape=(97, 132), L=2, batch=4)])
+                                 dict(shape=(2160, 3840), L=4, batch=1), dict(shape=(97, 132), L=2, batch=4),
+                                 dict(shape=(72, 116), L=2, batch=2)])
 def test_image_only_pyramids_vs_oracle(gpu_ctx, oracle, cfg):
     """The image-only (windowed) build -- the packed two-strip level-0 kernel and the packed decimation -- against the
-    oracle's pyramids: odd and even strip counts, a strip pair whose second strip lies outside the image, segments that
-    touch the top / bottom border and interior ones, widths that are not multiples of 120."""
+    oracle's pyramids: odd and even strip counts, a strip pair whose second strip lies outside the image, a single strip,
+    segments that touch the top / bottom border and interior ones, widths that are not multiples of 120."""
     from pyfeaturetrack_b200 import _capi, trackFeatures
     H, W = cfg["shape"]
     L, batch = cfg["L"], cfg["batch"]
@@ -187,34 +168,38 @@ def test_image_only_pyramids_vs_oracle(gpu_ctx, oracle, cfg):
     pyr.close()
 
 
-def test_kernel_generations_agree():
-    """$KLT_B200_SMOOTH0=1 / 2 / 3, $KLT_B200_DOWN2=1 and $KLT_B200_FUSED01=0 select the generations of the streaming kernels.
-    Every level-0 kernel (one strip per warp; two strips per warp on packed arithmetic; whole-row CTAs with bulk stores; the
-    fused level-0 + level-1 kernel) performs the same operations in the same order: level 0 is bit-identical.  The packed
-    decimation associates its sums differently from the scalar one, and the fused kernel decimates the smoothed
-    reflect-extended frame instead of the reflect-extended smoothed image: levels >= 1 agree to rounding."""
-    import ast
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = {}
-    variants = (("fused", {}), ("gen3", {"KLT_B200_FUSED01": "0"}), ("gen1", {"KLT_B200_FUSED01": "0", "KLT_B200_SMOOTH0": "1"}),
-                ("gen2", {"KLT_B200_FUSED01": "0", "KLT_B200_SMOOTH0": "2"}),
-                ("scalar", {"KLT_B200_FUSED01": "0", "KLT_B200_SMOOTH0": "1", "KLT_B200_DOWN2": "1"}))
-    for name, env in variants:
-        e = dict(os.environ)
-        for k in ("KLT_B200_SMOOTH0", "KLT_B200_DOWN2", "KLT_B200_FUSED01"):
-            e.pop(k, None)
-        e.update(env)
-        out = subprocess.run([sys.executable, "-c", _GEN_PROBE % root], env=e, capture_output=True, text=True, timeout=600)
-        assert out.returncode == 0, out.stderr[-2000:]
-        res[name] = ast.literal_eval(out.stdout.strip().splitlines()[-1])
-    assert res["gen3"] == res["gen1"] == res["gen2"]          # CRCs of every level: level 0 identical => all identical
-    for name in ("fused", "scalar"):
-        for (l1, c1, s1, m1), (l2, c2, s2, m2) in zip(res[name], res["gen3"]):
-            if l1 == 0:
-                assert c1 == c2, name
-            assert abs(s1 - s2) <= 1e-6 * max(abs(s1), 1.0) and abs(m1 - m2) <= 1e-5 * 255.0, name
+def test_kernel_generations_agree(gpu_ctx):
+    """The image-only (windowed) build starts with the fused level-0 + level-1 kernel (stream_level01) where it can, and
+    otherwise with the level-0 kernel (stream_smooth0x2) followed by the packed decimation (stream_down2).  The fused
+    kernel needs a frame pitch that is a multiple of 8, so the same frames, once contiguous and once in a buffer with 4
+    bytes of padding per row, take the two paths.  Both smooth level 0 with the same operations in the same order: level
+    0 is bit-identical.  The fused kernel decimates the smoothed reflect-extended frame instead of the reflect-extended
+    smoothed image: levels >= 1 agree to rounding."""
+    from pyfeaturetrack_b200 import _capi, trackFeatures
+    for (H, W, L, batch) in [(1080, 1920, 3, 5), (200, 360, 2, 2), (64, 248, 2, 1)]:
+        frames = (np.random.default_rng(H + W).random((batch, H, W)) * 255).astype(np.uint8)
+        padded = np.zeros((batch, H, W + 4), np.uint8)
+        padded[:, :, :W] = frames
+        taps = trackFeatures._taps_for_one_image(make_tc(nPyramidLevels=L, subsampling=2))
+        levels = []
+        for buf, first_kernel in ((frames, "stream_level01"), (padded, "stream_smooth0")):
+            pyr = _capi.Pyramid(gpu_ctx, W, H, L, 2, batch)
+            gpu_ctx.profile(True)
+            gpu_ctx.profile_reset()
+            try:
+                pyr.build_u8(buf, taps, _capi.PRECISION_FAST_WINDOWED)      # pitch: the buffer's row length
+                assert first_kernel in gpu_ctx.profile_read(), (H, W)
+            finally:
+                gpu_ctx.profile(False)
+            levels.append([[pyr.download(0, lvl, b) for lvl in range(L)] for b in range(batch)])
+            pyr.close()
+        for b in range(batch):
+            assert np.array_equal(levels[0][b][0], levels[1][b][0]), (H, W, b)
+            for lvl in range(1, L):
+                fused, split = levels[0][b][lvl], levels[1][b][lvl]
+                s1, s2 = fused.sum(dtype=np.float64), split.sum(dtype=np.float64)
+                assert abs(s1 - s2) <= 1e-6 * max(abs(s1), 1.0), (H, W, b, lvl)
+                assert np.abs(fused - split).max() <= 1e-5 * 255.0, (H, W, b, lvl)
 
 
 # ---- selection -----------------------------------------------------------------------------------------------------

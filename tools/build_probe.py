@@ -1,6 +1,6 @@
 """Pyramid-build probe: per-kernel CUDA-event times of image-only (windowed) and dense (fast) builds for several batch
-sizes, plus checksums of the built levels, so that two builds of the library (or two settings of $KLT_B200_SMOOTH0 /
-$KLT_B200_DOWN2) can be compared kernel by kernel.  python tools/build_probe.py [--batches 8,64] [--reps 20]"""
+sizes, plus checksums of the built levels, so that two builds of the library can be compared kernel by kernel.
+python tools/build_probe.py [--batches 8,64] [--reps 20]"""
 import argparse
 import json
 import os
@@ -61,8 +61,7 @@ def main():
             lv = [pyr.download(0, l, image=B - 1) for l in range(args.levels)]
             rec = {"batch": B, "mode": mode, "image": "%dx%d" % (W, H), "ms_per_build": round(ms_build, 4),
                    "frames_per_s": round(B / ms_build * 1e3, 1), "crc_levels": crc,
-                   "level_sums": [float(np.float64(a.sum(dtype=np.float64))) for a in lv],
-                   "smooth0": os.environ.get("KLT_B200_SMOOTH0", ""), "down2": os.environ.get("KLT_B200_DOWN2", "")}
+                   "level_sums": [float(np.float64(a.sum(dtype=np.float64))) for a in lv]}
             for k, v in prof.items():
                 ms = v["ms"] / v["launches"]
                 gbps = v["bytes"] / v["launches"] / ms * 1e-6
