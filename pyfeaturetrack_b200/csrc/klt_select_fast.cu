@@ -305,7 +305,7 @@ static int launch_fast(klt_ctx *ctx, const SelDev *S, int B, const float *img0, 
     if (rows > nrows) rows = nrows;
     const dim3 grid(strips, (nrows + rows - 1) / rows, B);
     const double bytes = (4.0 * S->W * S->H + 4.0 * S->ncand) * B;
-    KLT_LAUNCH(ctx, "eigen_fast", bytes, (eigen_fast_kernel<HH><<<grid, FS_THREADS, 0, ctx->stream>>>(img0, img_stride, pitch, *S, T, rows)));
+    KLT_LAUNCH(ctx, "eigen_fast_rows", bytes, (eigen_fast_kernel<HH><<<grid, FS_THREADS, 0, ctx->stream>>>(img0, img_stride, pitch, *S, T, rows)));
     return 1;
 }
 
