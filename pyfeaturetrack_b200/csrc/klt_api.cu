@@ -123,7 +123,6 @@ int klt_ctx_create(int device, void *stream, klt_ctx **out) {
     ctx->profiling = false;
     ctx->launches = 0;
     ctx->ws = nullptr; ctx->ws_bytes = 0;
-    ctx->level0_event = nullptr;
     ctx->own_stream = stream == nullptr;
     if (stream) ctx->stream = (cudaStream_t)stream;
     else if ((e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking)) != cudaSuccess) {
@@ -135,14 +134,13 @@ int klt_ctx_create(int device, void *stream, klt_ctx **out) {
     cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking);
     cudaStreamCreateWithFlags(&ctx->aux_stream, cudaStreamNonBlocking);
     for (int i = 0; i < 2; i++) cudaEventCreateWithFlags(&ctx->ov_ev[i], cudaEventDisableTiming);
-    ctx->iters_dev = nullptr;
     for (int i = 0; i < 16; i++) cudaEventCreateWithFlags(&ctx->chunk_ev[i], cudaEventDisableTiming);
     for (int i = 0; i < 2; i++) cudaEventCreateWithFlags(&ctx->half_free[i], cudaEventDisableTiming);
     ctx->half_next = 0;
     ctx->frames_dev = nullptr; ctx->frames_bytes = 0;
     ctx->async_flag_dev = nullptr;
     for (int i = 0; i < 16; i++) cudaEventCreateWithFlags(&ctx->marks[i], cudaEventDisableTiming);
-    if (cudaMalloc(&ctx->async_flag_dev, 256) == cudaSuccess) { cudaMemset(ctx->async_flag_dev, 0, 256); ctx->iters_dev = (unsigned long long *)(ctx->async_flag_dev + 16); }
+    if (cudaMalloc(&ctx->async_flag_dev, 256) == cudaSuccess) cudaMemset(ctx->async_flag_dev, 0, 256);
     ctx->num_sms = prop.multiProcessorCount;
     ctx->select_chunk = 4096;
     if (const char *e2 = getenv("KLT_B200_SELECT_CHUNK")) {
@@ -333,110 +331,92 @@ static int check_taps(klt_ctx *ctx, const klt_taps *t) {
     return KLT_OK;
 }
 
-// levels 1..L-1 and all gradients, given level 0 intensity already in place (level0_grad_done: the fused level-0
-// kernel has already written gradx/grady of level 0).  FAST precision takes the warp-streaming kernels where they
-// cover the configuration; everything else runs the generic tiled kernels.
-static int build_gradients(klt_ctx *ctx, klt_pyr *p, const klt_taps *taps, int precision, int first_level, int first, int count,
-                           int end_level = -1) {
-    int rc;
+// Host state of a build with the caller's KLT_PRECISION_*: the arithmetic (FAST_WINDOWED computes in FAST), the kernels,
+// and which gradient planes exist (none in an image-only FAST_WINDOWED build).  Builds, their lazy gradient passes and
+// graph replays of a build all keep it through this one function; it enqueues nothing.
+void klt_pyr_note_build(klt_pyr *p, const klt_taps *taps, int precision) {
+    const bool windowed = precision == KLT_PRECISION_FAST_WINDOWED;
+    p->precision = windowed ? KLT_PRECISION_FAST : precision;
+    p->hx->taps = *taps; p->hx->taps_valid = true;
+    p->hx->grad_valid = p->hx->grad0_valid = !windowed;
+}
+
+// build_levels: levels [from, n_levels) of images [first, first + count), each decimated from the level below;
+// build_grads: the gradient pairs of levels [from, to).  Both run with the arithmetic and kernels of the last build: FAST
+// arithmetic takes the warp-streaming kernel where it covers the level, everything else the generic tiled kernel.
+static int build_levels(klt_ctx *ctx, klt_pyr *p, int from, int first, int count) {
+    const klt_taps *taps = &p->hx->taps;
     const size_t stride = p->plane_floats;
-    const bool fast = precision == KLT_PRECISION_FAST;
-    if (end_level < 0) end_level = p->n_levels;
-    for (int l = first_level; l < end_level; l++) {
+    for (int l = from; l < p->n_levels; l++) {
+        const LevelDesc &a = p->lv[l - 1], &b = p->lv[l];
+        int rc = p->precision == KLT_PRECISION_FAST ? klt_stream_down2(ctx, p, l, taps, first, count) : 0;
+        if (rc < 0) return rc;
+        if (rc == 0 && (rc = klt_launch_pyr_down(ctx, p->level(0, first, l - 1), a.pitch, stride, a.w, a.h, p->level(0, first, l),
+                                                 b.pitch, stride, b.w, b.h, p->ss, count, &taps->pyramid, p->precision))) return rc;
+    }
+    return KLT_OK;
+}
+
+static int build_grads(klt_ctx *ctx, klt_pyr *p, int from, int to, int first, int count) {
+    const klt_taps *taps = &p->hx->taps;
+    const size_t stride = p->plane_floats;
+    for (int l = from; l < to; l++) {
         const LevelDesc &a = p->lv[l];
-        rc = fast ? klt_stream_grad(ctx, p, l, taps, first, count) : 0;
+        int rc = p->precision == KLT_PRECISION_FAST ? klt_stream_grad(ctx, p, l, taps, first, count) : 0;
         if (rc < 0) return rc;
         if (rc == 0 && (rc = klt_launch_grad_pair(ctx, p->level(0, first, l), a.pitch, stride, p->level(1, first, l),
                                                   p->level(2, first, l), a.pitch, stride, a.w, a.h, count, &taps->grad_gauss,
-                                                  &taps->grad_deriv, precision))) return rc;
+                                                  &taps->grad_deriv, p->precision))) return rc;
     }
     return KLT_OK;
 }
 
-// `windowed`: leave the gradient planes unwritten (KLT_PRECISION_FAST_WINDOWED)
-static int build_rest(klt_ctx *ctx, klt_pyr *p, const klt_taps *taps, int precision, bool level0_grad_done = false,
-                      int first = 0, int count = -1, bool windowed = false, int first_level = 1) {
-    if (count < 0) count = p->batch;
-    int rc;
-    const size_t stride = p->plane_floats;
-    const bool fast = precision == KLT_PRECISION_FAST;
-    for (int l = first_level; l < p->n_levels; l++) {
-        const LevelDesc &a = p->lv[l - 1], &b = p->lv[l];
-        rc = fast ? klt_stream_down2(ctx, p, l, taps, first, count) : 0;
-        if (rc < 0) return rc;
-        if (rc == 0 && (rc = klt_launch_pyr_down(ctx, p->level(0, first, l - 1), a.pitch, stride, a.w, a.h, p->level(0, first, l),
-                                                 b.pitch, stride, b.w, b.h, p->ss, count, &taps->pyramid, precision))) return rc;
-    }
-    if (windowed) return KLT_OK;
-    return build_gradients(ctx, p, taps, precision, level0_grad_done ? 1 : 0, first, count);
-}
-
-// bookkeeping of a build: `precision` as given by the caller; returns the arithmetic precision to run with
-int klt_begin_build(klt_pyr *p, const klt_taps *taps, int precision, bool *windowed) {
-    *windowed = precision == KLT_PRECISION_FAST_WINDOWED;
-    const int arith = *windowed ? KLT_PRECISION_FAST : precision;
-    p->precision = arith;
-    p->hx->taps = *taps; p->hx->taps_valid = true;
-    p->hx->grad_valid = p->hx->grad0_valid = !*windowed;
-    return arith;
-}
-
-int klt_pyr_ensure_gradients(klt_ctx *ctx, klt_pyr *p) {
-    if (!ctx || !p) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
+// gradient planes of levels [0, levels) of a built pyramid (an image-only build leaves them to its first reader; selection
+// on a tracking pyramid, KLTReplaceLostFeatures in sequentialMode, reads level 0 only).  Only klt_pyr_ensure_gradients
+// sets grad_valid: it sends tracking to the plane-based kernels, so a selection must leave an image-only pyramid on the
+// windowed tracker even when level 0 is its only level.
+int klt_ensure_gradients(klt_ctx *ctx, klt_pyr *p, int levels) {
     if (!p->hx || p->hx->grad_valid) return KLT_OK;
     if (!p->hx->taps_valid) return klt_fail(ctx, KLT_ERR_INVALID, "pyramid has not been built");
-    KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = build_gradients(ctx, p, &p->hx->taps, p->precision, p->hx->grad0_valid ? 1 : 0, 0, p->batch);
-    if (rc) return rc;
-    p->hx->grad_valid = p->hx->grad0_valid = true;
-    return KLT_OK;
-}
-
-// level 0 only: what selection on a tracking pyramid reads (KLTReplaceLostFeatures in sequentialMode)
-int klt_ensure_gradients_level0(klt_ctx *ctx, klt_pyr *p) {
-    if (!p->hx || p->hx->grad_valid || p->hx->grad0_valid) return KLT_OK;
-    if (!p->hx->taps_valid) return klt_fail(ctx, KLT_ERR_INVALID, "pyramid has not been built");
-    int rc = build_gradients(ctx, p, &p->hx->taps, p->precision, 0, 0, p->batch, 1);
+    int rc = build_grads(ctx, p, p->hx->grad0_valid ? 1 : 0, levels, 0, p->batch);
     if (rc) return rc;
     p->hx->grad0_valid = true;
     return KLT_OK;
 }
 
-// device frames -> pyramids for images [first, first+count); dframes points at image `first`
+int klt_pyr_ensure_gradients(klt_ctx *ctx, klt_pyr *p) {
+    if (!ctx || !p) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
+    KLT_CUDA(ctx, cudaSetDevice(ctx->device));
+    int rc = klt_ensure_gradients(ctx, p, p->n_levels);
+    if (rc == KLT_OK && p->hx) p->hx->grad_valid = true;
+    return rc;
+}
+
+// device frames -> pyramids for images [first, first+count); dframes points at image `first`.  level0_done (may be null) is
+// recorded right after the kernel that writes level 0, for a caller that forks work reading only that level.
 int klt_build_u8_device(klt_ctx *ctx, klt_pyr *p, const uint8_t *dframes, size_t pitch, size_t frame_stride,
-                        const klt_taps *taps, int precision, int first, int count, bool windowed) {
-    int rc;
+                        const klt_taps *taps, int precision, int first, int count, cudaEvent_t level0_done) {
+    klt_pyr_note_build(p, taps, precision);
+    const bool windowed = precision == KLT_PRECISION_FAST_WINDOWED;
+    int rc = 0, levels_done = 1;       // levels the level-0 step writes
+    bool grad0_done = false;           // ... and whether it also writes level 0's gradient pair
     if (windowed) {
-        // u8 -> smoothed image + level 1 in one pass
+        // u8 -> smoothed image + level 1 in one pass, else u8 -> smoothed image only
         // a caller that forks after level 0 (klt_sequence's eigenvalue pass) forks after the fused kernel instead: measured
         // 0.273 against 0.276 ms per step of 8 sequences with the two-kernel build, one launch fewer
-        rc = klt_stream_level01(ctx, dframes, pitch, frame_stride, p, taps, first, count);
-        if (rc < 0) return rc;
-        if (rc == 1) {
-            if (ctx->level0_event) KLT_CUDA(ctx, cudaEventRecord(ctx->level0_event, ctx->stream));
-            return build_rest(ctx, p, taps, precision, false, first, count, true, 2);
-        }
-        // u8 -> smoothed image only
-        rc = klt_stream_smooth0(ctx, dframes, pitch, frame_stride, p, taps, first, count);
-        if (rc < 0) return rc;
-        if (rc == 1) {
-            if (ctx->level0_event) KLT_CUDA(ctx, cudaEventRecord(ctx->level0_event, ctx->stream));
-            return build_rest(ctx, p, taps, precision, false, first, count, true);
-        }
+        if ((rc = klt_stream_level01(ctx, dframes, pitch, frame_stride, p, taps, first, count)) == 1) levels_done = 2;
+        else if (rc == 0) rc = klt_stream_smooth0(ctx, dframes, pitch, frame_stride, p, taps, first, count);
     } else if (precision == KLT_PRECISION_FAST) {
         // fused u8 -> smoothed image + gradient pair of level 0 (one read of the frame, three writes)
-        rc = klt_stream_level0(ctx, dframes, pitch, frame_stride, p, taps, first, count);
-        if (rc < 0) return rc;
-        if (rc == 1) {
-            if (ctx->level0_event) KLT_CUDA(ctx, cudaEventRecord(ctx->level0_event, ctx->stream));
-            return build_rest(ctx, p, taps, precision, true, first, count);
-        }
+        grad0_done = (rc = klt_stream_level0(ctx, dframes, pitch, frame_stride, p, taps, first, count)) == 1;
     }
+    if (rc < 0) return rc;
     // img.convert("F") + KLTComputeSmoothedImage (trackFeatures.py:165-166): one kernel, u8 in, f32 out
-    if ((rc = klt_launch_conv_sep_u8(ctx, dframes, pitch, frame_stride, p->level(0, first, 0), p->lv[0].pitch, p->plane_floats,
-                                     p->w, p->h, count, &taps->smooth, &taps->smooth, precision))) return rc;
-    if (ctx->level0_event) KLT_CUDA(ctx, cudaEventRecord(ctx->level0_event, ctx->stream));
-    return build_rest(ctx, p, taps, precision, false, first, count, windowed);
+    if (rc == 0 && (rc = klt_launch_conv_sep_u8(ctx, dframes, pitch, frame_stride, p->level(0, first, 0), p->lv[0].pitch,
+                                                p->plane_floats, p->w, p->h, count, &taps->smooth, &taps->smooth, p->precision))) return rc;
+    if (level0_done) KLT_CUDA(ctx, cudaEventRecord(level0_done, ctx->stream));
+    if ((rc = build_levels(ctx, p, levels_done, first, count))) return rc;
+    return windowed ? KLT_OK : build_grads(ctx, p, grad0_done ? 1 : 0, p->n_levels, first, count);
 }
 
 int klt_pyr_build_u8(klt_ctx *ctx, klt_pyr *p, const uint8_t *frames, size_t pitch, size_t frame_stride,
@@ -446,8 +426,6 @@ int klt_pyr_build_u8(klt_ctx *ctx, klt_pyr *p, const uint8_t *frames, size_t pit
     if ((rc = check_taps(ctx, taps))) return rc;
     if (pitch < (size_t)p->w) return klt_fail(ctx, KLT_ERR_INVALID, "pitch %zu smaller than width %d", pitch, p->w);
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-    bool windowed;
-    precision = klt_begin_build(p, taps, precision, &windowed);
     const uint8_t *dframes = frames;
     if (!klt_is_device_ptr(frames)) {
         const size_t bytes = (size_t)(p->batch - 1) * frame_stride + (size_t)(p->h - 1) * pitch + p->w;
@@ -455,7 +433,7 @@ int klt_pyr_build_u8(klt_ctx *ctx, klt_pyr *p, const uint8_t *frames, size_t pit
         KLT_CUDA(ctx, cudaMemcpyAsync(ctx->ws, frames, bytes, cudaMemcpyHostToDevice, ctx->stream));
         dframes = (const uint8_t *)ctx->ws;
     }
-    return klt_build_u8_device(ctx, p, dframes, pitch, frame_stride, taps, precision, 0, p->batch, windowed);
+    return klt_build_u8_device(ctx, p, dframes, pitch, frame_stride, taps, precision, 0, p->batch, nullptr);
 }
 
 int klt_pyr_build_f32(klt_ctx *ctx, klt_pyr *p, const float *images, size_t pitch, size_t frame_stride,
@@ -465,24 +443,24 @@ int klt_pyr_build_f32(klt_ctx *ctx, klt_pyr *p, const float *images, size_t pitc
     if ((rc = check_taps(ctx, taps))) return rc;
     if (pitch < (size_t)p->w) return klt_fail(ctx, KLT_ERR_INVALID, "pitch %zu smaller than width %d", pitch, p->w);
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-    bool windowed;
-    precision = klt_begin_build(p, taps, precision, &windowed);
+    klt_pyr_note_build(p, taps, precision);
     if (already_smoothed) {
         for (int b = 0; b < p->batch; b++)
             KLT_CUDA(ctx, cudaMemcpy2DAsync(p->level(0, b, 0), p->lv[0].pitch * sizeof(float), images + (size_t)b * frame_stride,
                                             pitch * sizeof(float), p->w * sizeof(float), p->h, cudaMemcpyDefault, ctx->stream));
-        return build_rest(ctx, p, taps, precision, false, 0, -1, windowed);
+    } else {
+        const float *dimg = images;
+        if (!klt_is_device_ptr(images)) {
+            const size_t elems = (size_t)(p->batch - 1) * frame_stride + (size_t)(p->h - 1) * pitch + p->w;
+            if ((rc = klt_ws_reserve(ctx, elems * sizeof(float)))) return rc;
+            KLT_CUDA(ctx, cudaMemcpyAsync(ctx->ws, images, elems * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+            dimg = (const float *)ctx->ws;
+        }
+        if ((rc = klt_launch_conv_sep_f32(ctx, dimg, pitch, frame_stride, p->level(0, 0, 0), p->lv[0].pitch, p->plane_floats, p->w,
+                                          p->h, p->batch, &taps->smooth, &taps->smooth, p->precision))) return rc;
     }
-    const float *dimg = images;
-    if (!klt_is_device_ptr(images)) {
-        const size_t elems = (size_t)(p->batch - 1) * frame_stride + (size_t)(p->h - 1) * pitch + p->w;
-        if ((rc = klt_ws_reserve(ctx, elems * sizeof(float)))) return rc;
-        KLT_CUDA(ctx, cudaMemcpyAsync(ctx->ws, images, elems * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-        dimg = (const float *)ctx->ws;
-    }
-    if ((rc = klt_launch_conv_sep_f32(ctx, dimg, pitch, frame_stride, p->level(0, 0, 0), p->lv[0].pitch, p->plane_floats, p->w,
-                                      p->h, p->batch, &taps->smooth, &taps->smooth, precision))) return rc;
-    return build_rest(ctx, p, taps, precision, false, 0, -1, windowed);
+    if ((rc = build_levels(ctx, p, 1, 0, p->batch))) return rc;
+    return precision == KLT_PRECISION_FAST_WINDOWED ? KLT_OK : build_grads(ctx, p, 0, p->n_levels, 0, p->batch);
 }
 
 int klt_pyr_download(klt_ctx *ctx, const klt_pyr *p, int image, int which, int level, float *out) {
@@ -548,7 +526,7 @@ int klt_select_good_features(klt_ctx *ctx, const klt_params *params, const klt_p
     if (pyr) {
         if (image < 0 || image >= pyr->batch) return klt_fail(ctx, KLT_ERR_INVALID, "image index out of range");
         if (pyr->batch == 1) return klt_select_batch(ctx, params, KLT_SELECT_STRICT, const_cast<klt_pyr *>(pyr), nullptr, nullptr, 0, 0, pyr->w, pyr->h, 1, n_features, replace, x, y, val, n_consumed);
-        int rc = klt_ensure_gradients_level0(ctx, const_cast<klt_pyr *>(pyr));      // image-only pyramids: build level 0's planes now
+        int rc = klt_ensure_gradients(ctx, const_cast<klt_pyr *>(pyr), 1);      // image-only pyramids: build level 0's planes now
         if (rc) return rc;
         return klt_select_batch(ctx, params, KLT_SELECT_STRICT, nullptr, pyr->level(1, image, 0), pyr->level(2, image, 0), 0, pyr->lv[0].pitch, pyr->w, pyr->h,
                                 1, n_features, replace, x, y, val, n_consumed);
@@ -881,14 +859,10 @@ static int track_pairs_impl(klt_ctx *ctx, const klt_params *params, const klt_ta
     const int half = ctx->half_next;
     ctx->half_next ^= 1;
     uint8_t *d1 = (uint8_t *)ctx->frames_dev + (size_t)half * ctx->frames_bytes, *d2 = d1 + set_stride;
-    int nchunks = B < 4 ? 1 : (B < 16 ? 2 : 4);
-    if (nchunks > 16) nchunks = 16;
+    const int nchunks = B < 4 ? 1 : (B < 16 ? 2 : 4);
     const int per_chunk = (B + nchunks - 1) / nchunks;
     // this half may still be read by the builds of the call before last
     KLT_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->half_free[half], 0));
-    bool windowed;
-    klt_begin_build(pyr1, taps, precision, &windowed);
-    precision = klt_begin_build(pyr2, taps, precision, &windowed);
     int k = 0;
     for (int first = 0; first < B; first += per_chunk, k++) {
         const int count = first + per_chunk <= B ? per_chunk : B - first;
@@ -902,8 +876,8 @@ static int track_pairs_impl(klt_ctx *ctx, const klt_params *params, const klt_ta
         const int count = first + per_chunk <= B ? per_chunk : B - first;
         const size_t off = (size_t)first * frame_stride;
         KLT_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->chunk_ev[k], 0));
-        if ((rc = klt_build_u8_device(ctx, pyr1, d1 + off, pitch, frame_stride, taps, precision, first, count, windowed))) return rc;
-        if ((rc = klt_build_u8_device(ctx, pyr2, d2 + off, pitch, frame_stride, taps, precision, first, count, windowed))) return rc;
+        if ((rc = klt_build_u8_device(ctx, pyr1, d1 + off, pitch, frame_stride, taps, precision, first, count, nullptr))) return rc;
+        if ((rc = klt_build_u8_device(ctx, pyr2, d2 + off, pitch, frame_stride, taps, precision, first, count, nullptr))) return rc;
     }
     KLT_CUDA(ctx, cudaEventRecord(ctx->half_free[half], ctx->stream));
     return track_impl(ctx, params, pyr1, pyr2, n_per_image, x, y, val, nullptr, nullptr, async);

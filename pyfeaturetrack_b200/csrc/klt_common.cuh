@@ -26,7 +26,7 @@ struct LevelDesc {
 
 // host-only part of a pyramid (kept behind a pointer so that klt_pyr stays a small by-value kernel argument)
 struct KltPyrHost {
-    klt_taps taps;            // kernels of the last build (the windowed tracker and lazy gradient builds need them)
+    klt_taps taps;            // kernels of the last build (its level loops, lazy gradient builds and the windowed tracker read them)
     bool taps_valid;
     bool grad_valid;          // gradient planes of ALL levels hold the gradients of the current images
     bool grad0_valid;         // at least level 0 does (selection on a tracking pyramid needs only that one)
@@ -78,8 +78,6 @@ struct klt_ctx {
     cudaStream_t copy_stream;
     cudaStream_t aux_stream;    // second compute stream: the second pyramid build of a device-resident klt_track_pairs_u8
     cudaEvent_t ov_ev[2];       // [0] entry, [1] "second pyramid built"
-    cudaEvent_t level0_event;   // if set, klt_build_u8_device records it right after the level-0 kernel (klt_sequence forks its eigenvalue pass there)
-    unsigned long long *iters_dev;   // device counter for calls that do not read it back
     cudaEvent_t chunk_ev[16];
     cudaEvent_t half_free[2];   // recorded on the compute stream once the builds have consumed that staging half
     int half_next;
@@ -125,14 +123,17 @@ static inline bool klt_pyr_has_gradients(const klt_pyr *p) { return !p->hx || p-
 
 int klt_make_taps(klt_ctx *ctx, const klt_kernel1d *k, TapsF *f, TapsD *d);
 
-// ---- klt_api.cu: pieces of the pyramid build that klt_sequence.cu reuses --------------------------------
+// ---- klt_api.cu: the pyramid build, shared with klt_select.cu and klt_sequence.cu ------------------------
 extern "C" {   // (defined inside klt_api.cu's extern "C" block; not part of the public ABI)
-// bookkeeping of a build: `precision` as given by the caller; returns the arithmetic precision to run with
-int klt_begin_build(klt_pyr *p, const klt_taps *taps, int precision, bool *windowed);
-// device frames -> pyramids for images [first, first+count); dframes points at image `first`
+// host state of a build with the caller's KLT_PRECISION_* (arithmetic, kernels, which gradient planes exist); enqueues
+// nothing, so a graph replay of a build calls it in place of the captured klt_build_u8_device
+void klt_pyr_note_build(klt_pyr *p, const klt_taps *taps, int precision);
+// device frames -> pyramids for images [first, first+count) with the caller's KLT_PRECISION_*; dframes points at image
+// `first`.  Records level0_done (may be null) right after the kernel that writes level 0.
 int klt_build_u8_device(klt_ctx *ctx, klt_pyr *p, const uint8_t *dframes, size_t pitch, size_t frame_stride,
-                        const klt_taps *taps, int precision, int first, int count, bool windowed);
-int klt_ensure_gradients_level0(klt_ctx *ctx, klt_pyr *p);
+                        const klt_taps *taps, int precision, int first, int count, cudaEvent_t level0_done);
+// gradient planes of levels [0, levels) of a built pyramid, built now where the last build left them out
+int klt_ensure_gradients(klt_ctx *ctx, klt_pyr *p, int levels);
 }
 
 // ---- launchers (klt_conv.cu) -- all pointers are DEVICE pointers, pitches in elements ----------------

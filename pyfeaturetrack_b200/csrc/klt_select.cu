@@ -878,6 +878,17 @@ int klt_sel_launch_eigen_strict(klt_ctx *ctx, const SelDev *S, int B, const floa
     return KLT_OK;
 }
 
+int klt_sel_launch_eigen(klt_ctx *ctx, const SelDev *S, int B, klt_pyr *pyr, int select_mode, float *sat) {
+    int rc;
+    if (select_mode == KLT_SELECT_FAST && pyr->hx->taps_valid) {
+        rc = klt_sel_launch_eigen_fast(ctx, S, B, pyr->level(0, 0, 0), pyr->plane_floats, pyr->lv[0].pitch, &pyr->hx->taps.grad_gauss,
+                                       &pyr->hx->taps.grad_deriv);
+        if (rc) return rc < 0 ? rc : KLT_OK;
+    }
+    if ((rc = klt_ensure_gradients(ctx, pyr, 1))) return rc;
+    return klt_sel_launch_eigen_strict(ctx, S, B, pyr->level(1, 0, 0), pyr->level(2, 0, 0), pyr->plane_floats, pyr->lv[0].pitch, sat);
+}
+
 // plan + scatter + walk on the eigenvalue maps and histograms of B images
 int klt_sel_launch_pick(klt_ctx *ctx, const SelDev *S, int B) {
     if (S->ncand) {
@@ -923,7 +934,6 @@ int klt_select_batch(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr
     if (rc) return rc;
     const bool host = !klt_is_device_ptr(x);
     if (host != !klt_is_device_ptr(y) || host != !klt_is_device_ptr(val)) return klt_fail(ctx, KLT_ERR_INVALID, "x, y, val must all be host or all be device");
-    const bool try_fast = select_mode == KLT_SELECT_FAST && pyr && pyr->hx && pyr->hx->taps_valid;
     if ((rc = klt_ws_reserve(ctx, klt_sel_workspace_bytes(&S, B, true, host)))) return rc;
     float *sat;
     klt_sel_carve(&S, B, true, host, (char *)ctx->ws, &sat);
@@ -937,19 +947,8 @@ int klt_select_batch(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr
     } else { S.fx = x; S.fy = y; S.fval = val; }
     if ((rc = klt_sel_prepare_kernels(ctx, &S))) return rc;
     if ((rc = klt_sel_launch_begin(ctx, &S, B))) return rc;
-    int done = 0;
-    if (try_fast) {
-        done = klt_sel_launch_eigen_fast(ctx, &S, B, pyr->level(0, 0, 0), pyr->plane_floats, pyr->lv[0].pitch, &pyr->hx->taps.grad_gauss,
-                                         &pyr->hx->taps.grad_deriv);
-        if (done < 0) return done;
-    }
-    if (!done) {
-        if (pyr) {
-            if ((rc = klt_ensure_gradients_level0(ctx, pyr))) return rc;      // image-only pyramids: build level 0's planes now
-            gx0 = pyr->level(1, 0, 0); gy0 = pyr->level(2, 0, 0); img_stride = pyr->plane_floats; pitch = pyr->lv[0].pitch;
-        }
-        if ((rc = klt_sel_launch_eigen_strict(ctx, &S, B, gx0, gy0, img_stride, pitch, sat))) return rc;
-    }
+    rc = pyr ? klt_sel_launch_eigen(ctx, &S, B, pyr, select_mode, sat) : klt_sel_launch_eigen_strict(ctx, &S, B, gx0, gy0, img_stride, pitch, sat);
+    if (rc) return rc;
     if ((rc = klt_sel_launch_pick(ctx, &S, B))) return rc;
     if (host) {
         KLT_CUDA(ctx, cudaMemcpyAsync(x, S.fx, total * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
@@ -974,22 +973,14 @@ int klt_eigen_maps(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr *
     if (nx_out) *nx_out = S.nx;
     if (ny_out) *ny_out = S.ny;
     if (!val || !S.ncand) return KLT_OK;
+    if (select_mode == KLT_SELECT_FAST && pyr->hx->taps_valid && !klt_sel_fast_covers(&S, &pyr->hx->taps.grad_gauss, &pyr->hx->taps.grad_deriv))
+        return klt_fail(ctx, KLT_ERR_UNSUPPORTED, "the fused eigenvalue pass does not cover this window / gradient kernel");
     if ((rc = klt_ws_reserve(ctx, klt_sel_workspace_bytes(&S, B, true, false)))) return rc;
     float *sat;
     klt_sel_carve(&S, B, true, false, (char *)ctx->ws, &sat);
     if ((rc = klt_sel_prepare_kernels(ctx, &S))) return rc;
     if ((rc = klt_sel_launch_begin(ctx, &S, B))) return rc;
-    int done = 0;
-    if (select_mode == KLT_SELECT_FAST && pyr->hx && pyr->hx->taps_valid) {
-        done = klt_sel_launch_eigen_fast(ctx, &S, B, pyr->level(0, 0, 0), pyr->plane_floats, pyr->lv[0].pitch, &pyr->hx->taps.grad_gauss,
-                                         &pyr->hx->taps.grad_deriv);
-        if (done < 0) return done;
-        if (!done) return klt_fail(ctx, KLT_ERR_UNSUPPORTED, "the fused eigenvalue pass does not cover this window / gradient kernel");
-    }
-    if (!done) {
-        if ((rc = klt_ensure_gradients_level0(ctx, pyr))) return rc;
-        if ((rc = klt_sel_launch_eigen_strict(ctx, &S, B, pyr->level(1, 0, 0), pyr->level(2, 0, 0), pyr->plane_floats, pyr->lv[0].pitch, sat))) return rc;
-    }
+    if ((rc = klt_sel_launch_eigen(ctx, &S, B, pyr, select_mode, sat))) return rc;
     KLT_CUDA(ctx, cudaMemcpyAsync(val, S.vmap, (size_t)B * S.ncand * sizeof(float), cudaMemcpyDefault, ctx->stream));
     KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return KLT_OK;

@@ -48,7 +48,11 @@ int klt_sel_prepare_kernels_scan(klt_ctx *ctx, const SelDev *S);
 int klt_sel_launch_begin(klt_ctx *ctx, const SelDev *S, int B);
 int klt_sel_launch_eigen_strict(klt_ctx *ctx, const SelDev *S, int B, const float *gx0, const float *gy0, size_t img_stride,
                                 size_t pitch, float *sat);
-// FAST eigenvalue map straight from the level-0 intensity planes (klt_select_fast.cu)
+// FAST eigenvalue map straight from the level-0 intensity planes (klt_select_fast.cu), where klt_sel_fast_covers says so
+bool klt_sel_fast_covers(const SelDev *S, const klt_kernel1d *gauss, const klt_kernel1d *deriv);
 int klt_sel_launch_eigen_fast(klt_ctx *ctx, const SelDev *S, int B, const float *img0, size_t img_stride, size_t pitch,
                               const klt_kernel1d *gauss, const klt_kernel1d *deriv);
+// eigenvalue maps of the level-0 planes of every image of a built pyramid: the fused pass if select_mode is KLT_SELECT_FAST
+// and it covers the configuration, else level 0's gradient planes (built now if the build left them out) and the table pass
+int klt_sel_launch_eigen(klt_ctx *ctx, const SelDev *S, int B, klt_pyr *pyr, int select_mode, float *sat);
 int klt_sel_launch_pick(klt_ctx *ctx, const SelDev *S, int B);

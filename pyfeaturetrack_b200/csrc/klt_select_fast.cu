@@ -309,16 +309,21 @@ static int launch_fast(klt_ctx *ctx, const SelDev *S, int B, const float *img0, 
     return 1;
 }
 
+// the fused pass covers 7-tap gradient kernels and square windows of half-size 1..7
+bool klt_sel_fast_covers(const SelDev *S, const klt_kernel1d *gauss, const klt_kernel1d *deriv) {
+    if (gauss->n != 2 * FS_R + 1 || deriv->n != 2 * FS_R + 1) return false;
+    if (S->hw != S->hh || S->hw < 1 || S->hw > 7) return false;
+    for (int k = 1; k <= 3; k++)            // the folded form needs the symmetry the reference's kernels have
+        if (fabs(gauss->taps[3 + k] - gauss->taps[3 - k]) > 1e-12 || fabs(deriv->taps[3 + k] + deriv->taps[3 - k]) > 1e-12) return false;
+    return fabs(deriv->taps[3]) <= 1e-12;
+}
+
 // 1 = launched, 0 = configuration not covered (caller builds gradient planes and takes the table-based pass), < 0 error
 int klt_sel_launch_eigen_fast(klt_ctx *ctx, const SelDev *S, int B, const float *img0, size_t img_stride, size_t pitch,
                               const klt_kernel1d *gauss, const klt_kernel1d *deriv) {
-    if (!gauss || !deriv || gauss->n != 2 * FS_R + 1 || deriv->n != 2 * FS_R + 1) return 0;
-    if (S->hw != S->hh || S->hw < 1 || S->hw > 7) return 0;
+    if (!klt_sel_fast_covers(S, gauss, deriv)) return 0;
     FastTaps T;
     for (int j = 0; j < 7; j++) { T.g[j] = (float)gauss->taps[6 - j]; T.d[j] = (float)deriv->taps[6 - j]; }
-    for (int k = 1; k <= 3; k++)            // the folded form needs the symmetry the reference's kernels have
-        if (fabs(gauss->taps[3 + k] - gauss->taps[3 - k]) > 1e-12 || fabs(deriv->taps[3 + k] + deriv->taps[3 - k]) > 1e-12) return 0;
-    if (fabs(deriv->taps[3]) > 1e-12) return 0;
     if (S->H < 16 && S->hh <= 3) {          // the quad kernel's one-bounce row reflection needs an image taller than its halo
         switch (S->hh) {
             case 1: return launch_fast<1>(ctx, S, B, img0, img_stride, pitch, T);

@@ -60,27 +60,11 @@ struct klt_sequence {
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-// eigenvalue maps of the level-0 planes of `p` (all images): the part of a selection that does not depend on the feature lists
-static int eigen_on(klt_ctx *ctx, klt_sequence *q, klt_pyr *p, const SelDev *S) {
-    int rc, done = 0;
-    if (q->select_mode == KLT_SELECT_FAST && q->fast_select_ok) {
-        done = klt_sel_launch_eigen_fast(ctx, S, q->B, p->level(0, 0, 0), p->plane_floats, p->lv[0].pitch, &q->taps.grad_gauss,
-                                         &q->taps.grad_deriv);
-        if (done < 0) return done;
-    }
-    if (!done) {
-        if ((rc = klt_ensure_gradients_level0(ctx, p))) return rc;
-        if ((rc = klt_sel_launch_eigen_strict(ctx, S, q->B, p->level(1, 0, 0), p->level(2, 0, 0), p->plane_floats, p->lv[0].pitch,
-                                              q->sat))) return rc;
-    }
-    return KLT_OK;
-}
-
 // selection on the level-0 planes of `p` (all images) into the sequence's feature lists, one stream
 static int select_on(klt_ctx *ctx, klt_sequence *q, klt_pyr *p, const SelDev *S) {
     int rc;
     if ((rc = klt_sel_launch_begin(ctx, S, q->B))) return rc;
-    if ((rc = eigen_on(ctx, q, p, S))) return rc;
+    if ((rc = klt_sel_launch_eigen(ctx, S, q->B, p, q->select_mode, q->sat))) return rc;
     return klt_sel_launch_pick(ctx, S, q->B);
 }
 
@@ -93,30 +77,26 @@ static SelDev sel_for_slot(const klt_sequence *q, int slot) {
 // FRONT of a step on ctx->stream (the caller points it at the stream it wants): frames in stage[par] -> pyramid `slot`,
 // and (replacement steps) its eigenvalue maps
 static int enqueue_front(klt_ctx *ctx, klt_sequence *q, int par, int slot, int replace) {
-    bool windowed;
-    const int arith = klt_begin_build(q->pyr[slot], &q->taps, q->precision, &windowed);
     const SelDev S = sel_for_slot(q, slot);
     int rc;
     // the fused fast eigenvalue pass reads the level-0 image only: it forks right after the level-0 kernel and runs beside the
     // decimations; the table-based pass needs the gradient planes, i.e. the whole build
-    const bool fork = replace && q->overlap && !ctx->profiling && q->eigen_stream && q->select_mode == KLT_SELECT_FAST && q->fast_select_ok;
-    ctx->level0_event = fork ? q->fork_ev : nullptr;
-    rc = klt_build_u8_device(ctx, q->pyr[slot], q->stage[par], q->cap_pitch, q->cap_stride, &q->taps, arith, 0, q->B, windowed);
-    ctx->level0_event = nullptr;
-    if (rc) return rc;
+    const bool fork = replace && q->overlap && !ctx->profiling && q->eigen_stream && q->fast_select_ok;
+    if ((rc = klt_build_u8_device(ctx, q->pyr[slot], q->stage[par], q->cap_pitch, q->cap_stride, &q->taps, q->precision, 0, q->B,
+                                  fork ? q->fork_ev : nullptr))) return rc;
     if (!replace) return KLT_OK;
     if (fork) {
         cudaStream_t mine = ctx->stream;
         KLT_CUDA(ctx, cudaStreamWaitEvent(q->eigen_stream, q->fork_ev, 0));
         ctx->stream = q->eigen_stream;
-        rc = eigen_on(ctx, q, q->pyr[slot], &S);
+        rc = klt_sel_launch_eigen(ctx, &S, q->B, q->pyr[slot], q->select_mode, q->sat);
         ctx->stream = mine;
         if (rc) return rc;
         KLT_CUDA(ctx, cudaEventRecord(q->join_ev, q->eigen_stream));
         KLT_CUDA(ctx, cudaStreamWaitEvent(mine, q->join_ev, 0));
         return KLT_OK;
     }
-    return eigen_on(ctx, q, q->pyr[slot], &S);
+    return klt_sel_launch_eigen(ctx, &S, q->B, q->pyr[slot], q->select_mode, q->sat);
 }
 
 // BACK of a step on ctx->stream: tracking prev -> slot and the list-dependent part of the replacement
@@ -204,9 +184,8 @@ static int run_half(klt_ctx *ctx, klt_sequence *q, int half, cudaStream_t stream
         }
         if (q->graph_ok[half][slot][rep]) {
             if (half == 0) {                               // host-side bookkeeping the captured calls would have done
-                bool windowed;
-                klt_begin_build(q->pyr[slot], &q->taps, q->precision, &windowed);
-                if (rep && !(q->select_mode == KLT_SELECT_FAST && q->fast_select_ok) && q->pyr[slot]->hx) q->pyr[slot]->hx->grad0_valid = true;
+                klt_pyr_note_build(q->pyr[slot], &q->taps, q->precision);
+                if (rep && !q->fast_select_ok) q->pyr[slot]->hx->grad0_valid = true;
             }
             const cudaError_t e = cudaGraphLaunch(q->graph[half][slot][rep], stream);
             if (e != cudaSuccess) { ctx->stream = saved; return klt_fail(ctx, KLT_ERR_CUDA, "cudaGraphLaunch failed: %s", cudaGetErrorString(e)); }
@@ -244,9 +223,7 @@ int klt_sequence_create(klt_ctx *ctx, const klt_params *params, const klt_taps *
     for (int i = 0; i < SEQ_ROT; i++)
         if ((rc = klt_pyr_create(ctx, w, h, params->n_levels, params->subsampling, n_sequences, &q->pyr[i]))) { klt_sequence_destroy(ctx, q); return rc; }
     if ((rc = klt_sel_geometry(ctx, params, w, h, n_features, 1, &q->S_rep))) { klt_sequence_destroy(ctx, q); return rc; }
-    // the fused fast eigen pass covers the default gradient kernel (7 taps) and square windows up to 15
-    q->fast_select_ok = select_mode == KLT_SELECT_FAST && taps->grad_gauss.n == 7 && taps->grad_deriv.n == 7 &&
-                        q->S_rep.hw == q->S_rep.hh && q->S_rep.hw >= 1 && q->S_rep.hw <= 7;
+    q->fast_select_ok = select_mode == KLT_SELECT_FAST && klt_sel_fast_covers(&q->S_rep, &taps->grad_gauss, &taps->grad_deriv);
     const bool need_sat = !q->fast_select_ok;
     const size_t total = (size_t)q->B * q->n;
     const size_t sel_b = klt_sel_workspace_bytes(&q->S_rep, q->B, need_sat, true);
@@ -321,9 +298,7 @@ int klt_sequence_start_u8(klt_ctx *ctx, klt_sequence *q, const uint8_t *frames, 
     if (q->front_stream) KLT_CUDA(ctx, cudaStreamSynchronize(q->front_stream));
     for (int i = 0; i < SEQ_ROT; i++) q->back_recorded[i] = false;
     if ((rc = stage_frames(ctx, q, par, frames, pitch, frame_stride, ctx->stream))) return rc;
-    bool windowed;
-    const int arith = klt_begin_build(q->pyr[slot], &q->taps, q->precision, &windowed);
-    if ((rc = klt_build_u8_device(ctx, q->pyr[slot], q->stage[par], pitch, frame_stride, &q->taps, arith, 0, q->B, windowed))) return rc;
+    if ((rc = klt_build_u8_device(ctx, q->pyr[slot], q->stage[par], pitch, frame_stride, &q->taps, q->precision, 0, q->B, nullptr))) return rc;
     KLT_CUDA(ctx, cudaEventRecord(q->stage_free[par], ctx->stream));
     if (select) {
         SelDev S = q->S_all;

@@ -349,11 +349,12 @@ def _oracle_sequence(oracle, p, frames, n, replace=True):
     return out
 
 
-def _run_sequence(ctx, tc, seqs, n, precision, select_mode, replace=True):
+def _run_sequence(ctx, tc, seqs, n, precision, select_mode, replace=True, taps=None):
     from pyfeaturetrack_b200 import _capi, selectGoodFeatures as sgf, trackFeatures as tf
     B, nfr = len(seqs), len(seqs[0])
     H, W = seqs[0][0].shape
-    q = _capi.Sequence(ctx, sgf.make_params(tc), tf._taps_for_one_image(tc), W, H, B, n, precision, select_mode)
+    taps = tf._taps_for_one_image(tc) if taps is None else taps
+    q = _capi.Sequence(ctx, sgf.make_params(tc), taps, W, H, B, n, precision, select_mode)
     q.start(np.ascontiguousarray(np.stack([s[0] for s in seqs])))
     out = [q.features()]
     for k in range(1, nfr):
@@ -492,14 +493,53 @@ def test_fullsize_golden_config_D_sequence(gpu_ctx, golden_fullsize):
             eq((got[k][0][s], got[k][1][s], got[k][2][s]), g[2 * k])                        # lists after replacement
 
 
+def test_sequence_fast_select_outside_the_fused_pass_equals_strict(gpu_ctx):
+    """The fused eigenvalue pass needs a symmetric 7-tap gradient smoother.  With one outer tap 1e-6 relative off it declines,
+    and a KLT_SELECT_FAST sequence must take the table-based pass instead, with its own summed-area-table workspace, on plain
+    launches and in graph replay: every list of every step equals the KLT_SELECT_STRICT run on the same taps and frames."""
+    from pyfeaturetrack_b200 import _capi, selectGoodFeatures as sgf, trackFeatures as tf
+    kw = dict(nPyramidLevels=3, subsampling=2, max_residue=10.0, sequentialMode=True)
+    tc = make_tc(**kw)
+    seqs = _sequence_frames(360, 480, 10, 3, speed=4.0)
+    H, W = seqs[0][0].shape
+    taps = tf._taps_for_one_image(tc)
+    assert taps.grad_gauss.n == 7
+    params = sgf.make_params(tc)
+    pyr = _capi.Pyramid(gpu_ctx, W, H, 3, 2, 1)
+    val = np.empty(H * W, np.float32)
+    nx, ny = C.c_int(), C.c_int()
+    codes = []
+    for perturb in (False, True):
+        if perturb:
+            taps.grad_gauss.taps[0] *= 1 + 1e-6
+        pyr.build_u8(np.ascontiguousarray(seqs[0][0]), taps, _capi.PRECISION_FAST_WINDOWED)
+        codes.append(_capi.lib().klt_eigen_map_batch(gpu_ctx.handle, C.byref(params), pyr.handle, _capi.SELECT_FAST,
+                                                     val.ctypes.data, C.byref(nx), C.byref(ny)))
+    pyr.close()
+    assert codes == [0, _capi.KLT_ERR_UNSUPPORTED]
+    runs = {}
+    for sel in (_capi.SELECT_FAST, _capi.SELECT_STRICT):
+        runs[sel], graph = _run_sequence(gpu_ctx, tc, seqs, 200, _capi.PRECISION_FAST_WINDOWED, sel, taps=taps)
+        assert graph
+    assert sum(int((o[3] != 0).sum()) for o in runs[_capi.SELECT_STRICT][1:]) > 0, "nothing was replaced"
+    for k, (got, want) in enumerate(zip(runs[_capi.SELECT_FAST], runs[_capi.SELECT_STRICT])):
+        for a, b in zip(got, want):
+            assert np.array_equal(a, b), k
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("precision,select", [("windowed", "fast"), ("fast", "strict"), ("strict", "strict")])
-def test_sequence_second_stream_changes_nothing(gpu_ctx, monkeypatch, precision, select):
+@pytest.mark.parametrize("precision,select,levels", [pytest.param("windowed", "fast", 3, id="windowed-fast"),
+                                                     pytest.param("fast", "strict", 3, id="fast-strict"),
+                                                     pytest.param("strict", "strict", 3, id="strict-strict"),
+                                                     pytest.param("windowed", "strict", 1, id="windowed-strict-one-level")])
+def test_sequence_second_stream_changes_nothing(gpu_ctx, monkeypatch, precision, select, levels):
     """The eigenvalue pass of a step runs on the context's second stream beside the decimations and the tracking kernel
     ($KLT_B200_SEQ_OVERLAP, on by default): every list of every frame must equal the single-stream run bit for bit, replayed
-    from the graph and with plain launches."""
+    from the graph and with plain launches.  A profiled run (plain launches, one stream) shows the tracker the pyramids'
+    precision selects; with one level, the level-0 gradient planes the table-based selection builds must not move an
+    image-only pyramid off the windowed tracker."""
     from pyfeaturetrack_b200 import _capi
-    kw = dict(nPyramidLevels=3, subsampling=2, max_residue=10.0, sequentialMode=True)
+    kw = dict(nPyramidLevels=levels, subsampling=2, max_residue=10.0, sequentialMode=True)
     tc = make_tc(**kw)
     seqs = _sequence_frames(360, 480, 9, 3, speed=4.0)
     prec = dict(windowed=_capi.PRECISION_FAST_WINDOWED, fast=_capi.PRECISION_FAST, strict=_capi.PRECISION_STRICT)[precision]
@@ -514,6 +554,16 @@ def test_sequence_second_stream_changes_nothing(gpu_ctx, monkeypatch, precision,
                 monkeypatch.setenv("KLT_B200_NO_GRAPH", "1")
             runs[(overlap, graph)], used = _run_sequence(gpu_ctx, tc, seqs, 200, prec, sel)
             assert used == graph
+    gpu_ctx.profile(True)
+    gpu_ctx.profile_reset()
+    try:
+        runs["profiled"], _ = _run_sequence(gpu_ctx, tc, seqs, 200, prec, sel)
+        kernels = gpu_ctx.profile_read()
+    finally:
+        gpu_ctx.profile(False)
+    tracker = dict(windowed="lk_windowed", fast="lk_track_rows", strict="lk_track")[precision]
+    assert [k for k in ("lk_windowed", "lk_track_rows", "lk_track") if k in kernels] == [tracker], sorted(kernels)
+    assert kernels[tracker]["launches"] == len(seqs[0]) - 1
     ref = runs[("0", False)]
     for key, got in runs.items():
         for k in range(len(ref)):
