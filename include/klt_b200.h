@@ -51,6 +51,8 @@ typedef enum klt_status {
 #define KLT_MAX_ITERATIONS (-3)
 #define KLT_OOB (-4)
 #define KLT_LARGE_RESIDUE (-5)
+/* beyond the reference: the forward-backward check rejected the feature (klt_track_features_fb) */
+#define KLT_FB_ERROR (-6)
 
 /* arithmetic mode of the convolution / pyramid kernels */
 #define KLT_PRECISION_FAST 0   /* fp32 FMA accumulation (<= 1e-6 relative-to-max of the reference images) */
@@ -233,6 +235,17 @@ int klt_eigen_map_batch(klt_ctx *ctx, const klt_params *params, klt_pyr *pyr, in
  * enqueues; that condition is then reported by the next klt_sync / klt_async_result on the context. */
 int klt_track_features(klt_ctx *ctx, const klt_params *params, const klt_pyr *pyr1, const klt_pyr *pyr2,
                        int n_per_image, double *x, double *y, int32_t *val, int64_t *n_iterations);
+/* ---- forward-backward check (Kalal, Mikolajczyk, Matas, ICPR 2010; beyond the reference and C-KLT).
+ * klt_track_features, then every feature it reports KLT_TRACKED at (xf, yf) is tracked back from pyr2 to pyr1 with the same
+ * params and kernels.  With e = sqrt(dx*dx + dy*dy) in double (dx = xb - x0, dy = yb - y0, (x0, y0) its position on entry),
+ * the feature becomes x = y = -1, val = KLT_FB_ERROR when the backward track is lost or !(e <= max_fb_error); otherwise it keeps
+ * the forward result.  A backward template that leaves the image rejects the feature and raises no KLT_ERR_ASSERT.
+ * max_fb_error: level-0 pixels, finite and > 0.  fb_error (optional, [batch][n_per_image]): (float)e where the backward track
+ * completed, -1 elsewhere.  x, y, val, fb_error host or device, same waiting / deferred-assert rules as klt_track_features;
+ * n_iterations counts both passes. */
+int klt_track_features_fb(klt_ctx *ctx, const klt_params *params, const klt_pyr *pyr1, const klt_pyr *pyr2,
+                          int n_per_image, float max_fb_error, double *x, double *y, int32_t *val, float *fb_error,
+                          int64_t *n_iterations);
 /* ---- affine consistency check: the block at trackFeatures.py:347-399.  The reference's callees there
  * (_KLTCreateFloatImage, _am_getSubFloatImage, _am_trackFeatureAffine) are undefined (NameError); these entry points
  * implement the C-KLT 1.3.4 routines of those names (parity against oracle/klt_oracle.c, unpinned by the reference).
@@ -334,6 +347,13 @@ int klt_sequence_select_stats(klt_ctx *ctx, klt_sequence *seq, int64_t *out);
 int klt_sequence_pyramid(klt_sequence *seq, klt_pyr **out);
 /* 1 once steps are replayed from CUDA graphs (0: plain launches, e.g. while profiling or with $KLT_B200_NO_GRAPH) */
 int klt_sequence_uses_graph(const klt_sequence *seq);
+/* from the next step on: max_fb_error > 0 runs the forward-backward check of klt_track_features_fb inside the step's tracking
+ * (before val_tracked is taken and before replacement, so rejected slots are refilled in the same step); 0 turns it off.
+ * Drops the captured graphs. */
+int klt_sequence_set_fb_check(klt_ctx *ctx, klt_sequence *seq, float max_fb_error);
+/* synchronous download of the last step's fb_error [n_sequences][n_features] (host or device; -1 where no backward track
+ * completed, everywhere when that step ran without the check) */
+int klt_sequence_get_fb_error(klt_ctx *ctx, klt_sequence *seq, float *out);
 
 #ifdef __cplusplus
 }

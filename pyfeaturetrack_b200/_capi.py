@@ -114,6 +114,8 @@ SIGNATURES = {
     "klt_select_good_features_batch": (_i, [_vp, C.POINTER(Params), _vp, _i, _i, _i, _dp, _dp, _ip]),
     "klt_eigen_map_batch": (_i, [_vp, C.POINTER(Params), _vp, _i, _fp, C.POINTER(_i), C.POINTER(_i)]),
     "klt_track_features": (_i, [_vp, C.POINTER(Params), _vp, _vp, _i, _dp, _dp, _ip, C.POINTER(C.c_int64)]),
+    "klt_track_features_fb": (_i, [_vp, C.POINTER(Params), _vp, _vp, _i, C.c_float, _dp, _dp, _ip, _fp,
+                                   C.POINTER(C.c_int64)]),
     "klt_affine_create": (_i, [_vp, _i, _i, _i, C.POINTER(_vp)]),
     "klt_affine_destroy": (_i, [_vp, _vp]),
     "klt_affine_reset": (_i, [_vp, _vp, _ip]),
@@ -142,6 +144,8 @@ SIGNATURES = {
     "klt_sequence_select_stats": (_i, [_vp, _vp, _vp]),
     "klt_sequence_pyramid": (_i, [_vp, C.POINTER(_vp)]),
     "klt_sequence_uses_graph": (_i, [_vp]),
+    "klt_sequence_set_fb_check": (_i, [_vp, _vp, C.c_float]),
+    "klt_sequence_get_fb_error": (_i, [_vp, _vp, _fp]),
 }
 
 
@@ -348,6 +352,17 @@ class Sequence:
 
     def uses_graph(self):
         return bool(lib().klt_sequence_uses_graph(self.handle))
+
+    def set_fb_check(self, max_fb_error):
+        """Forward-backward check inside every following step (max_fb_error > 0, level-0 pixels); 0 or None turns it off."""
+        self.ctx.check(lib().klt_sequence_set_fb_check(self.ctx.handle, self.handle,
+                                                       0.0 if max_fb_error is None else float(max_fb_error)))
+
+    def fb_error(self):
+        """float32 [n_sequences, n_features]: the last step's forward-backward distances (-1 where none was measured)."""
+        out = np.empty((self.B, self.n), np.float32)
+        self.ctx.check(lib().klt_sequence_get_fb_error(self.ctx.handle, self.handle, out.ctypes.data))
+        return out
 
     def close(self):
         if self.handle:

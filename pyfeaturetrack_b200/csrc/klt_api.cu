@@ -1,6 +1,7 @@
 // C ABI of libkltb200.so (see include/klt_b200.h): contexts, pyramids and the entry points that the Python
 // shims in pyfeaturetrack_b200/ bind with ctypes.  Host-side orchestration only; kernels live in
 // klt_conv.cu, klt_select.cu and klt_track.cu.
+#include <cfloat>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -564,9 +565,12 @@ static int check_track_args(klt_ctx *ctx, const klt_params *p, const klt_pyr *p1
     return KLT_OK;
 }
 
+// max_fb_error > 0: the forward-backward check after the forward track (fb_error may then be null, host or device)
 static int track_impl(klt_ctx *ctx, const klt_params *params, const klt_pyr *pyr1, const klt_pyr *pyr2, int n_per_image,
-                      double *x, double *y, int32_t *val, klt_affine *aff, int64_t *n_iterations, bool async = false) {
+                      double *x, double *y, int32_t *val, klt_affine *aff, int64_t *n_iterations, bool async = false,
+                      float max_fb_error = 0.f, float *fb_error = nullptr) {
     if (!ctx || !params || !pyr1 || !pyr2 || !x || !y || !val || n_per_image < 0) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
+    const bool fb = max_fb_error > 0.f;
     int rc;
     if ((rc = check_track_args(ctx, params, pyr1, pyr2))) return rc;
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
@@ -586,7 +590,8 @@ static int track_impl(klt_ctx *ctx, const klt_params *params, const klt_pyr *pyr
     const bool host = !klt_is_device_ptr(x);
     if (host != !klt_is_device_ptr(y) || host != !klt_is_device_ptr(val)) return klt_fail(ctx, KLT_ERR_INVALID, "x, y, val must all be host or all be device");
     const size_t fbytes = align_up(total * sizeof(double), 256);
-    if ((rc = klt_ws_reserve(ctx, 6 * fbytes + 256))) return rc;
+    // [iterations, assert word, backward assert word][x, y, val staging][affine: x_in, y_in, val_in | fb: x0, y0, vb, xb, yb, fb_error staging]
+    if ((rc = klt_ws_reserve(ctx, (fb ? 9 : 6) * fbytes + 256))) return rc;
     char *wsp = (char *)ctx->ws;
     unsigned long long *iters = (unsigned long long *)wsp;
     // calls that return without reading the flag back (asynchronous, or device arrays without n_iterations) raise the context's
@@ -611,13 +616,20 @@ static int track_impl(klt_ctx *ctx, const klt_params *params, const klt_pyr *pyr
         KLT_CUDA(ctx, cudaMemcpyAsync(y_in, dy, total * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
         KLT_CUDA(ctx, cudaMemcpyAsync(val_in, dval, total * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
     }
-    if ((rc = klt_launch_track(ctx, params, pyr1, pyr2, n_per_image, dx, dy, dval, iters, aflag))) return rc;
+    const bool fb_host = fb && fb_error && !klt_is_device_ptr(fb_error);
+    float *dfb = fb_host ? (float *)(wsp + 256 + 8 * fbytes) : fb_error;
+    if (fb) {
+        const FbArrays fa{(double *)(wsp + 256 + 3 * fbytes), (double *)(wsp + 256 + 4 * fbytes), (double *)(wsp + 256 + 6 * fbytes),
+                          (double *)(wsp + 256 + 7 * fbytes), (int32_t *)(wsp + 256 + 5 * fbytes), (int *)(wsp + 12)};
+        if ((rc = klt_launch_track_fb(ctx, params, pyr1, pyr2, n_per_image, max_fb_error, dx, dy, dval, fa, dfb, iters, aflag))) return rc;
+    } else if ((rc = klt_launch_track(ctx, params, pyr1, pyr2, n_per_image, dx, dy, dval, iters, aflag))) return rc;
     if (aff && (rc = klt_launch_affine(ctx, params, pyr1, pyr2, n_per_image, x_in, y_in, val_in, dx, dy, dval, aff, aflag))) return rc;
     if (host) {
         KLT_CUDA(ctx, cudaMemcpyAsync(x, dx, total * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
         KLT_CUDA(ctx, cudaMemcpyAsync(y, dy, total * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
         KLT_CUDA(ctx, cudaMemcpyAsync(val, dval, total * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
     }
+    if (fb_host) KLT_CUDA(ctx, cudaMemcpyAsync(fb_error, dfb, total * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     if (async) return KLT_OK;                    // results land when the stream gets there: klt_sync / klt_async_result
     if (host || n_iterations) {
         unsigned long long res[2] = {0, 0};
@@ -633,6 +645,13 @@ static int track_impl(klt_ctx *ctx, const klt_params *params, const klt_pyr *pyr
 int klt_track_features(klt_ctx *ctx, const klt_params *params, const klt_pyr *pyr1, const klt_pyr *pyr2, int n_per_image,
                        double *x, double *y, int32_t *val, int64_t *n_iterations) {
     return track_impl(ctx, params, pyr1, pyr2, n_per_image, x, y, val, nullptr, n_iterations);
+}
+
+int klt_track_features_fb(klt_ctx *ctx, const klt_params *params, const klt_pyr *pyr1, const klt_pyr *pyr2, int n_per_image,
+                          float max_fb_error, double *x, double *y, int32_t *val, float *fb_error, int64_t *n_iterations) {
+    if (!(max_fb_error > 0.f && max_fb_error <= FLT_MAX))
+        return klt_fail(ctx, KLT_ERR_INVALID, "max_fb_error must be finite and > 0 (got %g)", (double)max_fb_error);
+    return track_impl(ctx, params, pyr1, pyr2, n_per_image, x, y, val, nullptr, n_iterations, false, max_fb_error, fb_error);
 }
 
 int klt_track_features_affine(klt_ctx *ctx, const klt_params *params, const klt_pyr *pyr1, const klt_pyr *pyr2, int n_per_image,

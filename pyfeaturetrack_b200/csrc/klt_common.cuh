@@ -177,10 +177,19 @@ int klt_select_batch(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr
 int klt_eigen_maps(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr *pyr, float *val, int *nx_out, int *ny_out);
 
 // ---- klt_track.cu ------------------------------------------------------------------------------------
-// features of the images [first_image, first_image + n_images) of the batch (n_images < 0: all from first_image on)
+// features of the images [first_image, first_image + n_images) of the batch (n_images < 0: all from first_image on);
+// assert_marks_feature: see TrackArgs
 int klt_launch_track(klt_ctx *ctx, const klt_params *p, const klt_pyr *p1, const klt_pyr *p2, int n_per_image,
                      double *x_dev, double *y_dev, int32_t *val_dev, unsigned long long *iters_dev, int *assert_dev,
-                     int first_image = 0, int n_images = -1);
+                     int first_image = 0, int n_images = -1, int assert_marks_feature = 0);
+// device scratch of the forward-backward check, [batch][n_per_image] each; scratch_assert: the backward pass's assert word
+struct FbArrays { double *x0, *y0, *xb, *yb; int32_t *vb; int *scratch_assert; };
+// klt_launch_track p1 -> p2 with the forward-backward check: (x0, y0) saved, forward track, fb_prepare, the backward track
+// p2 -> p1 on (xb, yb, vb) (its template assertions mark the feature and raise only *scratch_assert), fb_check.  fb_error may
+// be null.  All pointers are device pointers; graph-capturable.
+int klt_launch_track_fb(klt_ctx *ctx, const klt_params *p, const klt_pyr *p1, const klt_pyr *p2, int n_per_image,
+                        float max_fb_error, double *x, double *y, int32_t *val, const FbArrays &fa, float *fb_error,
+                        unsigned long long *iters_dev, int *assert_dev);
 int klt_launch_extract_patch(klt_ctx *ctx, const float *img, size_t pitch, int w, int h, float x, float y,
                              int height, int width, float *out_dev, int *ok_dev);
 int klt_launch_iterate(klt_ctx *ctx, const klt_params *p, const float *tpatch_dev, const float *img2, const float *gx2,

@@ -9,16 +9,18 @@
 // A step has two halves with different inputs:
 //   FRONT  (needs only the new frames)     pyramid build + eigenvalue maps of the new frames (the latter on a third stream
 //                                          beside the decimations, forked right after the level-0 kernel)
-//   BACK   (needs FRONT + the lists of     tracking prev -> cur, status copy, pre-marking of the survivors, histogram, plan,
-//           the previous step)             scatter, greedy walk
+//   BACK   (needs FRONT + the lists of     tracking prev -> cur (with the forward-backward check: then back cur -> prev),
+//           the previous step)             status copy, pre-marking of the survivors, histogram, plan, scatter, greedy walk
 // FRONT runs on the sequence's own stream, BACK on the context's: when the caller does not wait between steps, FRONT of frame
 // k + 1 overlaps BACK of frame k (the walk and the plan are one CTA per sequence; the eigenvalue pass fills the other SMs).
 // That needs three pyramid batches and three eigenvalue maps in rotation (BACK(k) still tracks out of the pyramid FRONT(k + 2)
 // will overwrite, hence FRONT(k) waits for BACK(k - 2)).  Each half is captured into a CUDA graph per rotation slot once it has
 // run as plain launches; from then on a step is two graph launches and four event operations.  Host frames are uploaded on
 // the copy stream into the staging buffer of the step's rotation slot.  $KLT_B200_SEQ_OVERLAP=0 (and profiling) puts everything on one stream.
+#include <cfloat>
 #include <cstdlib>
 #include <cstring>
+#include <vector>
 
 #include "klt_common.cuh"
 #include "klt_select.cuh"
@@ -56,6 +58,12 @@ struct klt_sequence {
     bool graph_ok[2][SEQ_ROT][2];
     int warm[2][SEQ_ROT][2];
     int64_t graph_launches[2][SEQ_ROT][2];
+    // forward-backward check (klt_sequence_set_fb_check): threshold (0 = off) and its arrays, allocated on first use
+    float fb_max;
+    bool fb_ran;                     // the last step ran the check (fb_err is current)
+    char *fb_block;
+    FbArrays fb;
+    float *fb_err;
 };
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -102,7 +110,11 @@ static int enqueue_front(klt_ctx *ctx, klt_sequence *q, int par, int slot, int r
 // BACK of a step on ctx->stream: tracking prev -> slot and the list-dependent part of the replacement
 static int enqueue_back(klt_ctx *ctx, klt_sequence *q, int prev, int slot, int replace) {
     int rc;
-    if ((rc = klt_launch_track(ctx, &q->params, q->pyr[prev], q->pyr[slot], q->n, q->fx, q->fy, q->fval, q->iters, q->aflag))) return rc;
+    // both pyramids stay alive until BACK ends (rotation of three), so the backward pass needs no further synchronisation
+    if (q->fb_max > 0.f) {
+        if ((rc = klt_launch_track_fb(ctx, &q->params, q->pyr[prev], q->pyr[slot], q->n, q->fb_max, q->fx, q->fy, q->fval, q->fb,
+                                      q->fb_err, q->iters, q->aflag))) return rc;
+    } else if ((rc = klt_launch_track(ctx, &q->params, q->pyr[prev], q->pyr[slot], q->n, q->fx, q->fy, q->fval, q->iters, q->aflag))) return rc;
     KLT_CUDA(ctx, cudaMemcpyAsync(q->fval_tracked, q->fval, (size_t)q->B * q->n * sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream));
     if (!replace) return KLT_OK;
     const SelDev S = sel_for_slot(q, slot);
@@ -285,6 +297,7 @@ int klt_sequence_destroy(klt_ctx *ctx, klt_sequence *q) {
     if (q->front_stream) cudaStreamDestroy(q->front_stream);
     if (q->eigen_stream) cudaStreamDestroy(q->eigen_stream);
     if (q->block) cudaFree(q->block);
+    if (q->fb_block) cudaFree(q->fb_block);
     delete q;
     return KLT_OK;
 }
@@ -308,6 +321,7 @@ int klt_sequence_start_u8(klt_ctx *ctx, klt_sequence *q, const uint8_t *frames, 
     KLT_CUDA(ctx, cudaEventRecord(q->back_done[slot], ctx->stream));
     q->back_recorded[slot] = true;
     q->cur = slot; q->started = 1; q->steps = 0;
+    q->fb_ran = false;
     return KLT_OK;
 }
 
@@ -357,6 +371,7 @@ int klt_sequence_step_u8(klt_ctx *ctx, klt_sequence *q, const uint8_t *frames, s
     q->back_recorded[slot] = true;
     q->cur = slot;
     q->steps++;
+    q->fb_ran = q->fb_max > 0.f;
     return copy_out(ctx, q, x, y, val, val_tracked);
 }
 
@@ -390,6 +405,43 @@ int klt_sequence_select_stats(klt_ctx *ctx, klt_sequence *q, int64_t *out) {
 int klt_sequence_pyramid(klt_sequence *q, klt_pyr **out) {
     if (!q || !out) return KLT_ERR_INVALID;
     *out = q->pyr[q->cur];
+    return KLT_OK;
+}
+
+int klt_sequence_set_fb_check(klt_ctx *ctx, klt_sequence *q, float max_fb_error) {
+    if (!ctx || !q) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
+    if (!(max_fb_error == 0.f || (max_fb_error > 0.f && max_fb_error <= FLT_MAX)))
+        return klt_fail(ctx, KLT_ERR_INVALID, "max_fb_error must be 0 (off) or finite and > 0 (got %g)", (double)max_fb_error);
+    KLT_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (max_fb_error > 0.f && !q->fb_block) {
+        const size_t total = (size_t)q->B * q->n, db = align_up(total * sizeof(double), 256), ib = align_up(total * sizeof(int), 256);
+        const size_t bytes = 4 * db + 2 * ib + 256;
+        cudaError_t e = cudaMalloc(&q->fb_block, bytes);
+        if (e != cudaSuccess) { q->fb_block = nullptr; return klt_fail(ctx, KLT_ERR_NOMEM, "cudaMalloc(%zu) for the forward-backward arrays failed: %s", bytes, cudaGetErrorString(e)); }
+        char *b = q->fb_block;
+        q->fb.x0 = (double *)b; b += db;
+        q->fb.y0 = (double *)b; b += db;
+        q->fb.xb = (double *)b; b += db;
+        q->fb.yb = (double *)b; b += db;
+        q->fb.vb = (int32_t *)b; b += ib;
+        q->fb_err = (float *)b; b += ib;
+        q->fb.scratch_assert = (int *)b;
+    }
+    if (max_fb_error != q->fb_max) drop_graphs(q);      // the captured BACK halves carry the check and its threshold
+    q->fb_max = max_fb_error;
+    return KLT_OK;
+}
+
+int klt_sequence_get_fb_error(klt_ctx *ctx, klt_sequence *q, float *out) {
+    if (!ctx || !q || !out) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
+    const size_t total = (size_t)q->B * q->n;
+    if (q->fb_ran) {
+        KLT_CUDA(ctx, cudaMemcpyAsync(out, q->fb_err, total * sizeof(float), cudaMemcpyDefault, ctx->stream));
+    } else {
+        std::vector<float> none(total, -1.f);
+        KLT_CUDA(ctx, cudaMemcpyAsync(out, none.data(), total * sizeof(float), cudaMemcpyDefault, ctx->stream));
+    }
+    KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return KLT_OK;
 }
 

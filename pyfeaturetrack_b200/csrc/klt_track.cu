@@ -254,7 +254,10 @@ lk_track_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ xs, do
 
     if (lane == 0) {
         if (my_iters) atomicAdd(iters_total, (unsigned long long)my_iters);
-        if (st == KLT_INTERNAL_ASSERT) return;   // host raises; feature left untouched
+        if (st == KLT_INTERNAL_ASSERT) {         // host raises; feature left untouched
+            if (A.assert_marks_feature) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = KLT_OOB; }
+            return;
+        }
         const int W0 = A.p1.lv[0].w, H0 = A.p1.lv[0].h;
         const bool oob = xout < A.borderx || xout > __dsub_rn((double)(W0 - 1), A.borderx) || yout < A.bordery ||
                          yout > __dsub_rn((double)(H0 - 1), A.bordery);                      // _outOfBounds :140-141
@@ -452,7 +455,10 @@ lk_track_rows_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ x
     }
     if (was_alive && j == 0) {
         if (my_iters) atomicAdd(iters_total, (unsigned long long)my_iters);
-        if (st == KLT_INTERNAL_ASSERT) return;
+        if (st == KLT_INTERNAL_ASSERT) {
+            if (A.assert_marks_feature) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = KLT_OOB; }
+            return;
+        }
         const int W0 = A.p1.lv[0].w, H0 = A.p1.lv[0].h;
         const bool oob = xout < A.borderx || xout > (double)(W0 - 1) - A.borderx || yout < A.bordery ||
                          yout > (double)(H0 - 1) - A.bordery;
@@ -473,10 +479,11 @@ static int launch_rows(klt_ctx *ctx, const TrackArgs &A, double *x, double *y, i
 
 int klt_launch_track(klt_ctx *ctx, const klt_params *p, const klt_pyr *p1, const klt_pyr *p2, int n_per_image,
                      double *x_dev, double *y_dev, int32_t *val_dev, unsigned long long *iters_dev, int *assert_dev,
-                     int first_image, int n_images) {
+                     int first_image, int n_images, int assert_marks_feature) {
     // bit-exact arithmetic only pays off on bit-exact (STRICT) pyramids
     const bool exact = p1->precision == KLT_PRECISION_STRICT && p2->precision == KLT_PRECISION_STRICT;
     TrackArgs A;
+    A.assert_marks_feature = assert_marks_feature;
     A.p1 = *p1; A.p2 = *p2;
     A.w = p->window_width; A.h = p->window_height;
     A.n_levels = p->n_levels; A.ss = p->subsampling;
@@ -515,6 +522,61 @@ int klt_launch_track(klt_ctx *ctx, const klt_params *p, const klt_pyr *p1, const
     KLT_CUDA(ctx, cudaFuncSetAttribute(lk_track_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     const int blocks = (A.total - A.f_begin + warps - 1) / warps;
     KLT_LAUNCH(ctx, "lk_track", 0.0, (lk_track_kernel<<<blocks, warps * 32, smem, ctx->stream>>>(A, x_dev, y_dev, val_dev, iters_dev, assert_dev)));
+    return KLT_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Forward-backward check (Kalal, Mikolajczyk, Matas, ICPR 2010; no counterpart in the reference or in C-KLT).  The backward
+// pass is an ordinary klt_launch_track with the two pyramids swapped; these two element-wise kernels surround it.
+// ---------------------------------------------------------------------------------------------------------------------
+// the forward result becomes the backward pass's input (features the forward pass lost keep val < 0: the tracker skips them)
+__global__ void fb_prepare_kernel(int total, const double *__restrict__ x, const double *__restrict__ y,
+                                  const int32_t *__restrict__ val, double *__restrict__ xb, double *__restrict__ yb,
+                                  int32_t *__restrict__ vb) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= total) return;
+    xb[f] = x[f]; yb[f] = y[f]; vb[f] = val[f];
+}
+
+// decision: a forward-tracked feature whose backward track was lost, or came back farther than max_fb_error from where it
+// started, becomes (-1, -1, KLT_FB_ERROR).  e = sqrt(dx*dx + dy*dy) in double without FMA (NumPy's result bit for bit).
+__global__ void fb_check_kernel(int total, float max_fb_error, const double *__restrict__ x0, const double *__restrict__ y0,
+                                const double *__restrict__ xb, const double *__restrict__ yb, const int32_t *__restrict__ vb,
+                                double *__restrict__ x, double *__restrict__ y, int32_t *__restrict__ val,
+                                float *__restrict__ fb_error) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= total) return;
+    float fe = -1.f;
+    if (val[f] == KLT_TRACKED) {
+        bool reject = true;
+        if (vb[f] == KLT_TRACKED) {
+            const double dx = __dsub_rn(xb[f], x0[f]), dy = __dsub_rn(yb[f], y0[f]);
+            const double e = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
+            fe = (float)e;
+            reject = !(e <= (double)max_fb_error);
+        }
+        if (reject) { x[f] = -1.0; y[f] = -1.0; val[f] = KLT_FB_ERROR; }
+    }
+    if (fb_error) fb_error[f] = fe;
+}
+
+int klt_launch_track_fb(klt_ctx *ctx, const klt_params *p, const klt_pyr *p1, const klt_pyr *p2, int n_per_image,
+                        float max_fb_error, double *x, double *y, int32_t *val, const FbArrays &fa, float *fb_error,
+                        unsigned long long *iters_dev, int *assert_dev) {
+    const int total = n_per_image * p1->batch;
+    if (total <= 0) return KLT_OK;
+    const int blocks = (total + 255) / 256;
+    int rc;
+    // (x0, y0): the start positions, which the forward track overwrites
+    KLT_CUDA(ctx, cudaMemcpyAsync(fa.x0, x, total * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+    KLT_CUDA(ctx, cudaMemcpyAsync(fa.y0, y, total * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+    if ((rc = klt_launch_track(ctx, p, p1, p2, n_per_image, x, y, val, iters_dev, assert_dev))) return rc;
+    KLT_LAUNCH(ctx, "fb_prepare", 36.0 * total,
+               (fb_prepare_kernel<<<blocks, 256, 0, ctx->stream>>>(total, x, y, val, fa.xb, fa.yb, fa.vb)));
+    if ((rc = klt_launch_track(ctx, p, p2, p1, n_per_image, fa.xb, fa.yb, fa.vb, iters_dev, fa.scratch_assert, 0, -1, 1))) return rc;
+    KLT_LAUNCH(ctx, "fb_check", 76.0 * total,
+               (fb_check_kernel<<<blocks, 256, 0, ctx->stream>>>(total, max_fb_error, fa.x0, fa.y0, fa.xb, fa.yb, fa.vb, x, y, val,
+                                                                 fb_error)));
     return KLT_OK;
 }
 

@@ -17,6 +17,8 @@ struct TrackArgs {
     int n_per_image, total;     // features per image; END of the feature range of this launch
     int f_begin;                // first feature of this launch (a sub-range of the batch: [f_begin, total))
     int lighting_insensitive;   // gain / bias normalisation of trackFeaturesUtils.pyx:152-239 (exact-order kernel only)
+    int assert_marks_feature;   // 1: a feature whose template leaves the image is written (-1, -1, KLT_OOB) instead of being
+                                // left untouched (the backward pass of the forward-backward check; the flag is still raised)
 };
 
 // gradient kernels of the two pyramids (the reference's kernel cache can hand different ones to the two images,

@@ -418,7 +418,10 @@ lk_windowed_kernel(const __grid_constant__ TrackArgs A, const __grid_constant__ 
     }
     if (was_alive && q == 0) {
         if (my_iters) atomicAdd(iters_total, (unsigned long long)my_iters);
-        if (st == KLT_INTERNAL_ASSERT) return;
+        if (st == KLT_INTERNAL_ASSERT) {
+            if (A.assert_marks_feature) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = KLT_OOB; }
+            return;
+        }
         const int W0 = A.p1.lv[0].w, H0 = A.p1.lv[0].h;
         const bool oob = xout < A.borderx || xout > (double)(W0 - 1) - A.borderx || yout < A.bordery ||
                          yout > (double)(H0 - 1) - A.bordery;

@@ -15,6 +15,7 @@ class kltState:
     KLT_MAX_ITERATIONS = -3
     KLT_OOB = -4
     KLT_LARGE_RESIDUE = -5
+    KLT_FB_ERROR = -6            # beyond the reference: rejected by the forward-backward check (tc.max_fb_error)
 
 
 def _fix_window(tc, who):
@@ -47,6 +48,8 @@ _TC_DEFAULTS = (
     ("affineConsistencyCheck", -1), ("affine_window_width", 15), ("affine_window_height", 15),
     ("affine_max_iterations", 10), ("affine_max_residue", 10.), ("affine_min_displacement", 0.02),
     ("affine_max_displacement_differ", 1.5),
+    # beyond the reference: forward-backward check (level-0 pixels); None switches it off
+    ("max_fb_error", None),
 )
 # search_range / window_halfwidth <= bound  ->  (nPyramidLevels, subsampling)   (klt.py:105-117)
 _PYRAMID_STEPS = ((3.0, 2, 2), (5.0, 2, 4), (9.0, 2, 8))

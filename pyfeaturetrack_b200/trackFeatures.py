@@ -165,9 +165,11 @@ def KLTTrackFeatures(tc, img1, img2, featurelist):
             KLTCountRemainingFeatures(featurelist), ncols, nrows))
     _fix_window(tc, "Tracking context")
     use_affine = tc.affineConsistencyCheck >= 0
-    if tc.lighting_insensitive and use_affine:
+    max_fb_error = getattr(tc, "max_fb_error", None)
+    if (tc.lighting_insensitive or max_fb_error is not None) and use_affine:
         # the reference raises for lighting_insensitive alone (trackFeaturesUtils.pyx:435); this build implements the
-        # mode from the C the reference carries as comments (:152-239) -- but not together with the affine check
+        # mode from the C the reference carries as comments (:152-239) -- but not together with the affine check, and
+        # neither is the forward-backward check (beyond the reference)
         raise Exception("Not implemented")
     if use_affine and tc.affineConsistencyCheck > 2:
         raise ValueError("affineConsistencyCheck must be -1, 0, 1 or 2")
@@ -199,6 +201,11 @@ def KLTTrackFeatures(tc, img1, img2, featurelist):
         ctx.check(_capi.lib().klt_track_features_affine(ctx.handle, C.byref(params), pyramid1.pyr.handle,
                                                        pyramid2.pyr.handle, len(featurelist), x.ctypes.data,
                                                        y.ctypes.data, val.ctypes.data, aff.handle, None))
+    elif max_fb_error is not None:
+        # forward-backward check: rejected features come back with val = kltState.KLT_FB_ERROR
+        ctx.check(_capi.lib().klt_track_features_fb(ctx.handle, C.byref(params), pyramid1.pyr.handle, pyramid2.pyr.handle,
+                                                   len(featurelist), float(max_fb_error), x.ctypes.data, y.ctypes.data,
+                                                   val.ctypes.data, None, None))
     else:
         ctx.check(_capi.lib().klt_track_features(ctx.handle, C.byref(params), pyramid1.pyr.handle, pyramid2.pyr.handle,
                                                 len(featurelist), x.ctypes.data, y.ctypes.data, val.ctypes.data, None))
