@@ -218,6 +218,17 @@ int klt_select_good_features(klt_ctx *ctx, const klt_params *params, const klt_p
  * arrays are updated in place and the call returns without waiting).  select_mode: KLT_SELECT_STRICT / KLT_SELECT_FAST. */
 int klt_select_good_features_batch(klt_ctx *ctx, const klt_params *params, klt_pyr *pyr, int n_features, int replace,
                                    int select_mode, double *x, double *y, int32_t *val);
+/* ---- selection mask (beyond the reference, which has none; cf. the mask of OpenCV's goodFeaturesToTrack).
+ * klt_select_good_features_batch restricted to the pixels a caller allows: mask uint8 [batch][h][mask_pitch] (pitch in elements,
+ * >= w; mask_stride elements between images, 0 = one mask for every image), host or device, NONZERO = allowed.  A candidate at
+ * level-0 pixel (x, y) with mask[y][x] == 0 is never selected and suppresses nothing: the result is the reference's with that
+ * candidate removed from its pointlist (equivalently, with its eigenvalue set to 0).  In replacement mode surviving features keep
+ * their slots wherever they are and still suppress their mindist neighbourhood; only the new features obey the mask.
+ * mask == NULL is klt_select_good_features_batch.  Same host / device and waiting rules; a device mask must stay untouched
+ * until the stream has consumed it.  KLT_ERR_INVALID if mask_pitch < w. */
+int klt_select_good_features_batch_masked(klt_ctx *ctx, const klt_params *params, klt_pyr *pyr, int n_features, int replace,
+                                          int select_mode, const uint8_t *mask, size_t mask_pitch, size_t mask_stride, double *x,
+                                          double *y, int32_t *val);
 
 /* The minimum-eigenvalue maps alone, for every image of a pyramid batch, by either method: what ScanImageForGoodFeatures
  * returns as pointlistval (goodFeaturesUtils.pyx:53-71), val [batch][ny][nx] (host or device; NULL: only report nx, ny). */
@@ -354,6 +365,13 @@ int klt_sequence_set_fb_check(klt_ctx *ctx, klt_sequence *seq, float max_fb_erro
 /* synchronous download of the last step's fb_error [n_sequences][n_features] (host or device; -1 where no backward track
  * completed, everywhere when that step ran without the check) */
 int klt_sequence_get_fb_error(klt_ctx *ctx, klt_sequence *seq, float *out);
+/* selection mask of every following replacement and of the selection of klt_sequence_start_u8(select != 0) (beyond the
+ * reference; semantics of klt_select_good_features_batch_masked, tracking is not affected): mask uint8
+ * [n_sequences][h][mask_pitch], mask_stride elements apart (0 = one mask for every sequence), host or device, nonzero = allowed.
+ * The mask is converted once, on the context's stream behind the steps already enqueued, into a map the sequence owns; the
+ * caller's buffer is free again when the stream has passed this call.  mask == NULL turns the mask off.  Turning it on or off
+ * drops the captured graphs; replacing a set mask does not, so a mask that changes every frame keeps the graph replay. */
+int klt_sequence_set_mask(klt_ctx *ctx, klt_sequence *seq, const uint8_t *mask, size_t mask_pitch, size_t mask_stride);
 
 #ifdef __cplusplus
 }

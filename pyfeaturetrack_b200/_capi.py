@@ -112,6 +112,7 @@ SIGNATURES = {
     "klt_select_good_features": (_i, [_vp, C.POINTER(Params), _vp, _i, _fp, _fp, _i, _i, _i, _i, _dp, _dp, _ip,
                                       C.POINTER(C.c_int64)]),
     "klt_select_good_features_batch": (_i, [_vp, C.POINTER(Params), _vp, _i, _i, _i, _dp, _dp, _ip]),
+    "klt_select_good_features_batch_masked": (_i, [_vp, C.POINTER(Params), _vp, _i, _i, _i, _u8p, _sz, _sz, _dp, _dp, _ip]),
     "klt_eigen_map_batch": (_i, [_vp, C.POINTER(Params), _vp, _i, _fp, C.POINTER(_i), C.POINTER(_i)]),
     "klt_track_features": (_i, [_vp, C.POINTER(Params), _vp, _vp, _i, _dp, _dp, _ip, C.POINTER(C.c_int64)]),
     "klt_track_features_fb": (_i, [_vp, C.POINTER(Params), _vp, _vp, _i, C.c_float, _dp, _dp, _ip, _fp,
@@ -146,6 +147,7 @@ SIGNATURES = {
     "klt_sequence_uses_graph": (_i, [_vp]),
     "klt_sequence_set_fb_check": (_i, [_vp, _vp, C.c_float]),
     "klt_sequence_get_fb_error": (_i, [_vp, _vp, _fp]),
+    "klt_sequence_set_mask": (_i, [_vp, _vp, _u8p, _sz, _sz]),
 }
 
 
@@ -363,6 +365,29 @@ class Sequence:
         out = np.empty((self.B, self.n), np.float32)
         self.ctx.check(lib().klt_sequence_get_fb_error(self.ctx.handle, self.handle, out.ctypes.data))
         return out
+
+    def set_mask(self, mask, pitch=None, stride=None):
+        """Selection mask of every following replacement (and of start(select=True)); nonzero = new features allowed there.
+        mask: None (off), a (H, W) array shared by every sequence, a (n_sequences, H, W) array, or a device pointer with an
+        explicit pitch and stride (elements; stride 0 = shared).  Tracking is not affected."""
+        if mask is None:
+            self.ctx.check(lib().klt_sequence_set_mask(self.ctx.handle, self.handle, None, 0, 0))
+            return
+        if isinstance(mask, np.ndarray):
+            m = np.ascontiguousarray(mask != 0 if mask.dtype != np.uint8 else mask, np.uint8)
+            if m.shape == (self.h, self.w):
+                stride = 0
+            elif m.shape == (self.B, self.h, self.w):
+                stride = self.h * self.w
+            else:
+                raise ValueError("mask shape %s: expected (%d, %d) or (%d, %d, %d)" % (m.shape, self.h, self.w, self.B, self.h,
+                                                                                       self.w))
+            self._mask_keep = m          # (the conversion is enqueued behind the steps in flight)
+            self.ctx.check(lib().klt_sequence_set_mask(self.ctx.handle, self.handle, m.ctypes.data, self.w, stride))
+            return
+        if pitch is None or stride is None:
+            raise ValueError("a device mask needs an explicit pitch and stride")
+        self.ctx.check(lib().klt_sequence_set_mask(self.ctx.handle, self.handle, int(mask), int(pitch), int(stride)))
 
     def close(self):
         if self.handle:

@@ -540,10 +540,17 @@ int klt_select_good_features(klt_ctx *ctx, const klt_params *params, const klt_p
 
 int klt_select_good_features_batch(klt_ctx *ctx, const klt_params *params, klt_pyr *pyr, int n_features, int replace,
                                    int select_mode, double *x, double *y, int32_t *val) {
+    return klt_select_good_features_batch_masked(ctx, params, pyr, n_features, replace, select_mode, nullptr, 0, 0, x, y, val);
+}
+
+int klt_select_good_features_batch_masked(klt_ctx *ctx, const klt_params *params, klt_pyr *pyr, int n_features, int replace,
+                                          int select_mode, const uint8_t *mask, size_t mask_pitch, size_t mask_stride, double *x,
+                                          double *y, int32_t *val) {
     if (!ctx || !params || !pyr || !x || !y || !val || n_features < 0) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
     if (select_mode != KLT_SELECT_STRICT && select_mode != KLT_SELECT_FAST) return klt_fail(ctx, KLT_ERR_INVALID, "select_mode must be KLT_SELECT_STRICT or KLT_SELECT_FAST");
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-    return klt_select_batch(ctx, params, select_mode, pyr, nullptr, nullptr, 0, 0, pyr->w, pyr->h, pyr->batch, n_features, replace, x, y, val, nullptr);
+    return klt_select_batch(ctx, params, select_mode, pyr, nullptr, nullptr, 0, 0, pyr->w, pyr->h, pyr->batch, n_features, replace, x, y, val, nullptr,
+                            mask, mask_pitch, mask_stride);
 }
 
 int klt_eigen_map_batch(klt_ctx *ctx, const klt_params *params, klt_pyr *pyr, int select_mode, float *val, int *nx, int *ny) {

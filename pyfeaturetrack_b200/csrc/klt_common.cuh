@@ -169,10 +169,12 @@ int klt_stream_down2(klt_ctx *ctx, klt_pyr *p, int level, const klt_taps *taps, 
 int klt_launch_scan(klt_ctx *ctx, const float *gx, const float *gy, size_t pitch, int w, int h, int bx, int by,
                     int hw, int hh, int skip, float *val_dev /* [ny][nx] */, int nx, int ny);
 // full selection for every image of `pyr` (or, pyr == NULL, for B explicit device gradient images img_stride apart);
-// x, y, val: [B][n_features] host or device
+// x, y, val: [B][n_features] host or device; mask (optional, host or device): uint8 [B][h][mask_pitch], mask_stride apart
+// (0: one mask for all images), nonzero = candidates allowed there
 int klt_select_batch(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr *pyr, const float *gx0, const float *gy0,
                      size_t img_stride, size_t pitch, int w, int h, int B, int n_features, int replace, double *x, double *y,
-                     int32_t *val, int64_t *n_consumed);
+                     int32_t *val, int64_t *n_consumed, const uint8_t *mask = nullptr, size_t mask_pitch = 0,
+                     size_t mask_stride = 0);
 
 int klt_eigen_maps(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr *pyr, float *val, int *nx_out, int *ny_out);
 

@@ -437,6 +437,39 @@ premark_kernel(const __grid_constant__ SelDev S) {
     }
 }
 
+// ---- caller's selection mask -> pre-mark map (beyond the reference) ----------------------------------------------------
+// map[b][y * W + x] = (mask[b * stride + y * pitch + x] == 0): a masked-out pixel is pre-marked like a pixel a survivor
+// suppresses.  Every byte of the image's map_stride is written (the padding with 0), so the map needs no memset first.
+// vec (W, pitch, stride multiples of 16, mask 16-byte aligned): 16 map bytes per thread, never across a row; else 1.
+__global__ void __launch_bounds__(256)
+mask_premap_kernel(const unsigned char *__restrict__ mask, size_t pitch, size_t stride, int W, int H, size_t map_stride, int vec,
+                   unsigned char *__restrict__ premap) {
+    const unsigned char *m = mask + (size_t)blockIdx.y * stride;
+    unsigned char *map = premap + (size_t)blockIdx.y * map_stride;
+    const unsigned int plane = (unsigned int)W * (unsigned int)H;          // < 2^26 (8191 x 8191)
+    const unsigned int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (vec) {
+        const unsigned int o = 16u * t;
+        if (o >= map_stride) return;
+        uint4 r = make_uint4(0u, 0u, 0u, 0u);
+        if (o < plane) {
+            const unsigned int y = o / (unsigned int)W, x = o - y * (unsigned int)W;
+            const uint4 v = *reinterpret_cast<const uint4 *>(m + (size_t)y * pitch + x);
+            r.x = __vcmpeq4(v.x, 0u) & 0x01010101u; r.y = __vcmpeq4(v.y, 0u) & 0x01010101u;
+            r.z = __vcmpeq4(v.z, 0u) & 0x01010101u; r.w = __vcmpeq4(v.w, 0u) & 0x01010101u;
+        }
+        *reinterpret_cast<uint4 *>(map + o) = r;
+    } else {
+        if (t >= map_stride) return;
+        unsigned char r = 0;
+        if (t < plane) {
+            const unsigned int y = t / (unsigned int)W, x = t - y * (unsigned int)W;
+            r = m[(size_t)y * pitch + x] == 0 ? 1 : 0;
+        }
+        map[t] = r;
+    }
+}
+
 // ---- the walk: sort + greedy minimum-distance suppression (_enforceMinimumDistance) -----------------------------------
 // Accepted features are remembered in a grid of cells of side cs = r + 1 (r = mindist - 1): two features in one cell would
 // be closer than mindist, so a cell holds at most one and a candidate only has to look at its 3x3 cell neighbourhood
@@ -796,21 +829,21 @@ int klt_sel_geometry(klt_ctx *ctx, const klt_params *p, int w, int h, int n_feat
     return KLT_OK;
 }
 
-size_t klt_sel_workspace_bytes(const SelDev *S, int B, bool strict_sat, bool own_features) {
+size_t klt_sel_workspace_bytes(const SelDev *S, int B, bool strict_sat, bool own_features, bool masked) {
     size_t t = 0;
     if (strict_sat) t += align_up((size_t)B * 3 * S->W * S->H * sizeof(float), 256);
     t += align_up((size_t)B * (S->ncand + 1) * sizeof(float), 256);              // vmap
     t += align_up((size_t)B * (SEL_BINS * 3 + 1) * sizeof(unsigned int), 256);   // hist, cursor, offs
     t += align_up((size_t)B * (SEL_PLAN_WORDS * sizeof(unsigned int) + SEL_STATUS_WORDS * sizeof(unsigned long long)), 256);
     t += 2 * align_up((size_t)B * S->key_stride * sizeof(unsigned long long), 256);
-    if (S->replace) t += align_up((size_t)B * S->map_stride, 256);
+    if (S->replace || masked) t += align_up((size_t)B * S->map_stride, 256);
     if (!S->grid_in_smem) t += align_up((size_t)B * S->grid_stride * sizeof(unsigned short), 256) + align_up((size_t)B * S->grid_stride * sizeof(unsigned int), 256);
     t += align_up((size_t)B * S->n_features * sizeof(int) + 64, 256);            // free slots
     if (own_features) t += align_up((size_t)B * S->n_features * (2 * sizeof(double) + sizeof(int)) + 64, 256);
     return t + 1024;
 }
 
-void klt_sel_carve(SelDev *S, int B, bool strict_sat, bool own_features, char *base, float **sat) {
+void klt_sel_carve(SelDev *S, int B, bool strict_sat, bool own_features, char *base, float **sat, bool masked) {
     char *p = base;
     auto take = [&](size_t bytes) { char *q = p; p += align_up(bytes, 256); return q; };
     if (sat) *sat = nullptr;
@@ -822,7 +855,7 @@ void klt_sel_carve(SelDev *S, int B, bool strict_sat, bool own_features, char *b
     S->status = (unsigned long long *)ps; S->plan = (unsigned int *)(ps + (size_t)B * SEL_STATUS_WORDS * sizeof(unsigned long long));
     S->keys = (unsigned long long *)take((size_t)B * S->key_stride * sizeof(unsigned long long));
     S->keys2 = (unsigned long long *)take((size_t)B * S->key_stride * sizeof(unsigned long long));
-    S->premap = S->replace ? (unsigned char *)take((size_t)B * S->map_stride) : nullptr;
+    S->premap = (S->replace || masked) ? (unsigned char *)take((size_t)B * S->map_stride) : nullptr;
     S->grid_global = S->grid_in_smem ? nullptr : (unsigned short *)take((size_t)B * S->grid_stride * sizeof(unsigned short));
     S->cellmin_global = S->grid_in_smem ? nullptr : (unsigned int *)take((size_t)B * S->grid_stride * sizeof(unsigned int));
     S->free_slots = (int *)take((size_t)B * S->n_features * sizeof(int) + 64);
@@ -846,12 +879,31 @@ int klt_sel_prepare_kernels(klt_ctx *ctx, const SelDev *S) {
     return KLT_OK;
 }
 
-// histogram reset + (replacement mode) pre-marking of the surviving features; must precede the eigen pass
-int klt_sel_launch_begin(klt_ctx *ctx, const SelDev *S, int B) {
+int klt_launch_mask_premap(klt_ctx *ctx, const unsigned char *mask, size_t pitch, size_t stride, int W, int H, size_t map_stride,
+                           int B, unsigned char *premap) {
+    const int vec = (W % 16) == 0 && (pitch % 16) == 0 && (stride % 16) == 0 && (map_stride % 16) == 0 &&
+                    ((reinterpret_cast<uintptr_t>(mask) | reinterpret_cast<uintptr_t>(premap)) & 15) == 0;
+    const size_t threads = vec ? map_stride / 16 : map_stride;
+    const dim3 grid((unsigned int)((threads + 255) / 256), B);
+    KLT_LAUNCH(ctx, "mask_premap", ((double)W * H + (double)map_stride) * B,
+               (mask_premap_kernel<<<grid, 256, 0, ctx->stream>>>(mask, pitch, stride, W, H, map_stride, vec, premap)));
+    return KLT_OK;
+}
+
+// histogram reset + the pre-mark map: seeded from the caller's mask (m->mask: converted now; m->seed: copied) or cleared,
+// then, in replacement mode, pre-marking of the surviving features; must precede the eigen pass
+int klt_sel_launch_begin(klt_ctx *ctx, const SelDev *S, int B, const SelMask *m) {
     KLT_CUDA(ctx, cudaMemsetAsync(S->hist, 0, (size_t)B * SEL_BINS * sizeof(unsigned int), ctx->stream));
-    if (S->replace) {
-        KLT_CUDA(ctx, cudaMemsetAsync(S->premap, 0, (size_t)B * S->map_stride, ctx->stream));
-        if (S->r >= 0 && S->n_features > 0)
+    if (S->premap) {
+        int rc;
+        if (m && m->mask) {
+            if ((rc = klt_launch_mask_premap(ctx, m->mask, m->pitch, m->stride, S->W, S->H, S->map_stride, B, S->premap))) return rc;
+        } else if (m && m->seed) {
+            KLT_CUDA(ctx, cudaMemcpyAsync(S->premap, m->seed, (size_t)B * S->map_stride, cudaMemcpyDeviceToDevice, ctx->stream));
+        } else {
+            KLT_CUDA(ctx, cudaMemsetAsync(S->premap, 0, (size_t)B * S->map_stride, ctx->stream));
+        }
+        if (S->replace && S->r >= 0 && S->n_features > 0)
             KLT_LAUNCH(ctx, "premark", (double)B * S->map_stride, (premark_kernel<<<dim3(S->n_features, B), 128, 0, ctx->stream>>>(*S)));
     }
     return KLT_OK;
@@ -928,15 +980,27 @@ int klt_sel_prepare_kernels_scan(klt_ctx *ctx, const SelDev *S) {
 // Source: the level-0 planes of `pyr` (all its images), or explicit device gradient images (pyr == NULL, B images img_stride apart).
 int klt_select_batch(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr *pyr, const float *gx0, const float *gy0,
                      size_t img_stride, size_t pitch, int w, int h, int B, int n_features, int replace, double *x, double *y,
-                     int32_t *val, int64_t *n_consumed) {
+                     int32_t *val, int64_t *n_consumed, const uint8_t *mask, size_t mask_pitch, size_t mask_stride) {
     SelDev S;
     int rc = klt_sel_geometry(ctx, p, w, h, n_features, replace, &S);
     if (rc) return rc;
     const bool host = !klt_is_device_ptr(x);
     if (host != !klt_is_device_ptr(y) || host != !klt_is_device_ptr(val)) return klt_fail(ctx, KLT_ERR_INVALID, "x, y, val must all be host or all be device");
-    if ((rc = klt_ws_reserve(ctx, klt_sel_workspace_bytes(&S, B, true, host)))) return rc;
+    const bool masked = mask != nullptr;
+    if (masked && mask_pitch < (size_t)w) return klt_fail(ctx, KLT_ERR_INVALID, "mask_pitch %zu smaller than width %d", mask_pitch, w);
+    // a host mask is uploaded behind the selection workspace
+    const bool mask_host = masked && !klt_is_device_ptr(mask);
+    const size_t mask_bytes = masked ? (size_t)(mask_stride ? B - 1 : 0) * mask_stride + (size_t)(h - 1) * mask_pitch + w : 0;
+    const size_t sel_b = klt_sel_workspace_bytes(&S, B, true, host, masked);
+    if ((rc = klt_ws_reserve(ctx, sel_b + (mask_host ? align_up(mask_bytes, 256) : 0)))) return rc;
     float *sat;
-    klt_sel_carve(&S, B, true, host, (char *)ctx->ws, &sat);
+    klt_sel_carve(&S, B, true, host, (char *)ctx->ws, &sat, masked);
+    SelMask sm = {mask, mask_pitch, mask_stride, nullptr};
+    if (mask_host) {
+        unsigned char *d = (unsigned char *)ctx->ws + sel_b;
+        KLT_CUDA(ctx, cudaMemcpyAsync(d, mask, mask_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        sm.mask = d;
+    }
     const size_t total = (size_t)B * n_features;
     if (host) {
         if (replace) {
@@ -946,7 +1010,7 @@ int klt_select_batch(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr
         }
     } else { S.fx = x; S.fy = y; S.fval = val; }
     if ((rc = klt_sel_prepare_kernels(ctx, &S))) return rc;
-    if ((rc = klt_sel_launch_begin(ctx, &S, B))) return rc;
+    if ((rc = klt_sel_launch_begin(ctx, &S, B, masked ? &sm : nullptr))) return rc;
     rc = pyr ? klt_sel_launch_eigen(ctx, &S, B, pyr, select_mode, sat) : klt_sel_launch_eigen_strict(ctx, &S, B, gx0, gy0, img_stride, pitch, sat);
     if (rc) return rc;
     if ((rc = klt_sel_launch_pick(ctx, &S, B))) return rc;

@@ -26,7 +26,7 @@ struct SelDev {
     unsigned int *plan;               // [B][SEL_PLAN_WORDS]
     unsigned long long *status;       // [B][SEL_STATUS_WORDS]
     unsigned long long *keys, *keys2; // [B][key_stride]
-    unsigned char *premap;            // [B][map_stride], replacement mode only
+    unsigned char *premap;            // [B][map_stride], replacement mode or a masked selection
     unsigned short *grid_global;      // [B][grid_stride] when the cell grid does not fit in shared memory
     unsigned int *cellmin_global;     // [B][grid_stride] ditto, the per-cell minimum live rank of the walk's rounds
     int *free_slots;                  // [B][n_features]
@@ -40,12 +40,25 @@ __device__ __forceinline__ int eig_rbin(float v) {
     return min(max(rb, 0), SEL_BINS - 1);
 }
 
+// Where the pre-mark map of a selection starts from (klt_sel_launch_begin).  The map is premap != nullptr in replacement mode
+// and whenever the selection is masked; a set byte removes the candidate at that pixel from the histogram, the keys and the
+// walk's fallback gather.  With neither field set the map starts cleared.
+struct SelMask {
+    const unsigned char *mask;        // caller's mask [B or 1][H][pitch] (device), nonzero = allowed: converted by mask_premap
+    size_t pitch, stride;             // in elements; stride 0 = one mask for every image
+    const unsigned char *seed;        // or a map [B][map_stride] converted earlier (klt_sequence_set_mask): copied
+};
+
 int klt_sel_geometry(klt_ctx *ctx, const klt_params *p, int w, int h, int n_features, int replace, SelDev *S);
-size_t klt_sel_workspace_bytes(const SelDev *S, int B, bool strict_sat, bool own_features);
-void klt_sel_carve(SelDev *S, int B, bool strict_sat, bool own_features, char *base, float **sat);
+// masked: reserve / carve the pre-mark map also in SELECTING_ALL mode
+size_t klt_sel_workspace_bytes(const SelDev *S, int B, bool strict_sat, bool own_features, bool masked = false);
+void klt_sel_carve(SelDev *S, int B, bool strict_sat, bool own_features, char *base, float **sat, bool masked = false);
 int klt_sel_prepare_kernels(klt_ctx *ctx, const SelDev *S);          // cudaFuncSetAttribute calls: outside stream capture
 int klt_sel_prepare_kernels_scan(klt_ctx *ctx, const SelDev *S);
-int klt_sel_launch_begin(klt_ctx *ctx, const SelDev *S, int B);
+int klt_sel_launch_begin(klt_ctx *ctx, const SelDev *S, int B, const SelMask *m = nullptr);
+// premap[b][y * W + x] = (mask[b * stride + y * pitch + x] == 0) for B images, every byte of map_stride written (device pointers)
+int klt_launch_mask_premap(klt_ctx *ctx, const unsigned char *mask, size_t pitch, size_t stride, int W, int H, size_t map_stride,
+                           int B, unsigned char *premap);
 int klt_sel_launch_eigen_strict(klt_ctx *ctx, const SelDev *S, int B, const float *gx0, const float *gy0, size_t img_stride,
                                 size_t pitch, float *sat);
 // FAST eigenvalue map straight from the level-0 intensity planes (klt_select_fast.cu), where klt_sel_fast_covers says so

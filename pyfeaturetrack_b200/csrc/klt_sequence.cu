@@ -64,14 +64,27 @@ struct klt_sequence {
     char *fb_block;
     FbArrays fb;
     float *fb_err;
+    // selection mask (klt_sequence_set_mask): the pre-mark map it seeds, [B][map_stride], allocated on first use (its address
+    // never changes, so the captured BACK halves keep copying from it), and the device staging of host masks
+    bool mask_on;
+    unsigned char *mask_seed;
+    unsigned char *mask_up;
+    size_t mask_up_bytes;
 };
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // selection on the level-0 planes of `p` (all images) into the sequence's feature lists, one stream
+// where the pre-mark map of a selection starts: the mask's map while a mask is set, else cleared
+static SelMask mask_of(const klt_sequence *q) {
+    SelMask m = {nullptr, 0, 0, q->mask_on ? q->mask_seed : nullptr};
+    return m;
+}
+
 static int select_on(klt_ctx *ctx, klt_sequence *q, klt_pyr *p, const SelDev *S) {
     int rc;
-    if ((rc = klt_sel_launch_begin(ctx, S, q->B))) return rc;
+    const SelMask m = mask_of(q);
+    if ((rc = klt_sel_launch_begin(ctx, S, q->B, &m))) return rc;
     if ((rc = klt_sel_launch_eigen(ctx, S, q->B, p, q->select_mode, q->sat))) return rc;
     return klt_sel_launch_pick(ctx, S, q->B);
 }
@@ -118,7 +131,8 @@ static int enqueue_back(klt_ctx *ctx, klt_sequence *q, int prev, int slot, int r
     KLT_CUDA(ctx, cudaMemcpyAsync(q->fval_tracked, q->fval, (size_t)q->B * q->n * sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream));
     if (!replace) return KLT_OK;
     const SelDev S = sel_for_slot(q, slot);
-    if ((rc = klt_sel_launch_begin(ctx, &S, q->B))) return rc;
+    const SelMask m = mask_of(q);
+    if ((rc = klt_sel_launch_begin(ctx, &S, q->B, &m))) return rc;
     return klt_sel_launch_pick(ctx, &S, q->B);
 }
 
@@ -298,6 +312,8 @@ int klt_sequence_destroy(klt_ctx *ctx, klt_sequence *q) {
     if (q->eigen_stream) cudaStreamDestroy(q->eigen_stream);
     if (q->block) cudaFree(q->block);
     if (q->fb_block) cudaFree(q->fb_block);
+    if (q->mask_seed) cudaFree(q->mask_seed);
+    if (q->mask_up) cudaFree(q->mask_up);
     delete q;
     return KLT_OK;
 }
@@ -442,6 +458,42 @@ int klt_sequence_get_fb_error(klt_ctx *ctx, klt_sequence *q, float *out) {
         KLT_CUDA(ctx, cudaMemcpyAsync(out, none.data(), total * sizeof(float), cudaMemcpyDefault, ctx->stream));
     }
     KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return KLT_OK;
+}
+
+int klt_sequence_set_mask(klt_ctx *ctx, klt_sequence *q, const uint8_t *mask, size_t mask_pitch, size_t mask_stride) {
+    if (!ctx || !q) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
+    KLT_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (!mask) {
+        if (q->mask_on) drop_graphs(q);          // the captured BACK halves copy the map instead of clearing it
+        q->mask_on = false;
+        q->S_all.premap = nullptr;
+        return KLT_OK;
+    }
+    if (mask_pitch < (size_t)q->w) return klt_fail(ctx, KLT_ERR_INVALID, "mask_pitch %zu smaller than width %d", mask_pitch, q->w);
+    const SelDev &S = q->S_rep;
+    if (!q->mask_seed) {
+        const cudaError_t e = cudaMalloc(&q->mask_seed, (size_t)q->B * S.map_stride);
+        if (e != cudaSuccess) { q->mask_seed = nullptr; return klt_fail(ctx, KLT_ERR_NOMEM, "cudaMalloc for the mask map failed: %s", cudaGetErrorString(e)); }
+    }
+    const unsigned char *src = mask;
+    if (!klt_is_device_ptr(mask)) {
+        const size_t bytes = (size_t)(mask_stride ? q->B - 1 : 0) * mask_stride + (size_t)(q->h - 1) * mask_pitch + q->w;
+        if (bytes > q->mask_up_bytes) {
+            KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));     // an earlier conversion may still read the old buffer
+            if (q->mask_up) KLT_CUDA(ctx, cudaFree(q->mask_up));
+            q->mask_up = nullptr; q->mask_up_bytes = 0;
+            KLT_CUDA(ctx, cudaMalloc(&q->mask_up, bytes));
+            q->mask_up_bytes = bytes;
+        }
+        KLT_CUDA(ctx, cudaMemcpyAsync(q->mask_up, mask, bytes, cudaMemcpyHostToDevice, ctx->stream));
+        src = q->mask_up;
+    }
+    int rc;
+    if ((rc = klt_launch_mask_premap(ctx, src, mask_pitch, mask_stride, q->w, q->h, S.map_stride, q->B, q->mask_seed))) return rc;
+    if (!q->mask_on) drop_graphs(q);
+    q->mask_on = true;
+    q->S_all.premap = q->S_rep.premap;          // SELECTING_ALL reads the same map (no pre-marking there)
     return KLT_OK;
 }
 

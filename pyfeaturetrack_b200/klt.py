@@ -50,6 +50,8 @@ _TC_DEFAULTS = (
     ("affine_max_displacement_differ", 1.5),
     # beyond the reference: forward-backward check (level-0 pixels); None switches it off
     ("max_fb_error", None),
+    # beyond the reference: (nrows, ncols) array, nonzero where selection may place new features; None = everywhere
+    ("selection_mask", None),
 )
 # search_range / window_halfwidth <= bound  ->  (nPyramidLevels, subsampling)   (klt.py:105-117)
 _PYRAMID_STEPS = ((3.0, 2, 2), (5.0, 2, 4), (9.0, 2, 8))

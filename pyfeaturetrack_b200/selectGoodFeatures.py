@@ -138,15 +138,35 @@ _AFFINE_RESET = dict(aff_img=None, aff_img_gradx=None, aff_img_grady=None, aff_x
                      aff_Ayx=0.0, aff_Axy=0.0, aff_Ayy=1.0)
 
 
+def _selection_mask(tc, ncols, nrows):
+    """tc.selection_mask as uint8 [nrows, ncols] (nonzero = new features allowed there), or None."""
+    m = getattr(tc, "selection_mask", None)
+    if m is None:
+        return None
+    m = np.asarray(m)
+    if m.shape != (nrows, ncols):
+        KLTError("(_KLTSelectGoodFeatures) Size of tc.selection_mask ({0}) is different from size of image ({1} by {2})".format(
+            " by ".join(str(s) for s in m.shape[::-1]), ncols, nrows))
+    return np.ascontiguousarray(m != 0, np.uint8)
+
+
 def _select_on_device(tc, pyr, nFeatures, featurelist, overwriteAllFeatures):
-    """Scan + sort + _enforceMinimumDistance on level-0 gradients of `pyr` (selectGoodFeatures.py:215-246)."""
+    """Scan + sort + _enforceMinimumDistance on level-0 gradients of `pyr` (selectGoodFeatures.py:215-246), restricted to
+    tc.selection_mask where one is set (beyond the reference)."""
     ctx = pyr.ctx
+    mask = _selection_mask(tc, pyr.w, pyr.h)
     x, y, val = _gather(featurelist, nFeatures, overwriteAllFeatures)
     old_val = val.copy()
     params = make_params(tc)
-    ctx.check(_capi.lib().klt_select_good_features_batch(ctx.handle, C.byref(params), pyr.handle, nFeatures,
-                                                        0 if overwriteAllFeatures else 1, config.select_mode_code(),
-                                                        x.ctypes.data, y.ctypes.data, val.ctypes.data))
+    if mask is None:
+        ctx.check(_capi.lib().klt_select_good_features_batch(ctx.handle, C.byref(params), pyr.handle, nFeatures,
+                                                            0 if overwriteAllFeatures else 1, config.select_mode_code(),
+                                                            x.ctypes.data, y.ctypes.data, val.ctypes.data))
+    else:
+        ctx.check(_capi.lib().klt_select_good_features_batch_masked(ctx.handle, C.byref(params), pyr.handle, nFeatures,
+                                                                   0 if overwriteAllFeatures else 1, config.select_mode_code(),
+                                                                   mask.ctypes.data, pyr.w, 0, x.ctypes.data, y.ctypes.data,
+                                                                   val.ctypes.data))
     ctx.mark_synced()          # host arrays: the call waited for the stream
     _scatter(featurelist, x, y, val, old_val, overwriteAllFeatures)
     return featurelist
