@@ -92,8 +92,7 @@ __device__ __forceinline__ int iterate_exact(const float *T, const float *Tgx, c
     const float fhw = (float)hw, fhh = (float)hh, fnc = (float)nc, fnr = (float)nr;
     int status = KLT_TRACKED;
     while (true) {
-        if (__fsub_rn(x2, fhw) < 0.f || __fsub_rn(fnc, __fadd_rn(x2, fhw)) < 1.001f ||
-            __fsub_rn(y2, fhh) < 0.f || __fsub_rn(fnr, __fadd_rn(y2, fhh)) < 1.001f) { status = KLT_OOB; break; }
+        if (!lk_window_inside_f(x2, y2, fhw, fhh, fnc, fnr)) { status = KLT_OOB; break; }
         const int ix = (int)x2, iy = (int)y2;
         const float ax = __double2float_rn(__dsub_rn((double)x2, (double)ix));
         const float ay = __double2float_rn(__dsub_rn((double)y2, (double)iy));
@@ -173,7 +172,7 @@ lk_track_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ xs, do
     const double ss = (double)A.ss;
 
     double xloc = xs[f], yloc = ys[f];
-    for (int r = A.n_levels - 1; r >= 0; r--) { xloc = __ddiv_rn(xloc, ss); yloc = __ddiv_rn(yloc, ss); }   // :260-262
+    lk_top_level(xloc, yloc, A.n_levels, ss);
     double xout = xloc, yout = yloc;
     int st = KLT_TRACKED;
     unsigned int my_iters = 0;
@@ -189,7 +188,7 @@ lk_track_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ xs, do
         const float x1 = __double2float_rn(xloc), y1 = __double2float_rn(yloc);
         {
             const int ix = (int)x1, iy = (int)y1;
-            if (!(ix - hw >= 0 && iy - hh >= 0 && ix + hw + 2 <= nc && iy + hh + 2 <= nr)) {   // pyx:35
+            if (!lk_template_inside(ix, iy, hw, hh, nc, nr)) {
                 if (lane == 0) { atomicExch(assert_flag, 1); }
                 st = KLT_INTERNAL_ASSERT;
                 break;
@@ -214,10 +213,8 @@ lk_track_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ xs, do
         int status = status0;
         my_iters += iteration;
 
-        // ---- back in _trackFeature (trackFeatures.py:108-136): doubles, hw = width/2 ----
-        const double x2d = (double)x2, y2d = (double)y2, hwd = A.w / 2.0, hhd = A.h / 2.0;
-        if (__dsub_rn(x2d, hwd) < 0.0 || __dsub_rn((double)nc, __dadd_rn(x2d, hwd)) < 1.001 ||
-            __dsub_rn(y2d, hhd) < 0.0 || __dsub_rn((double)nr, __dadd_rn(y2d, hhd)) < 1.001) status = KLT_OOB;
+        // ---- back in _trackFeature (trackFeatures.py:108-136) ----
+        if (!lk_window_inside_d(x2, y2, A.w, A.h, nc, nr)) status = KLT_OOB;
         if (status == KLT_TRACKED && A.has_max_residue) {
             const int ix = (int)x2, iy = (int)y2;
             const float ax = __double2float_rn(__dsub_rn((double)x2, (double)ix));
@@ -244,27 +241,11 @@ lk_track_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ xs, do
             if (res > A.max_residue) status = KLT_LARGE_RESIDUE;
             __syncwarp();
         }
-        xout = x2d; yout = y2d;
-        if (A.retain) st = KLT_TRACKED;
-        else if (status == KLT_SMALL_DET || status == KLT_OOB || status == KLT_LARGE_RESIDUE) st = status;
-        else if (iteration >= A.max_iterations) st = KLT_MAX_ITERATIONS;
-        else st = KLT_TRACKED;
-        if (st == KLT_SMALL_DET || st == KLT_OOB) break;                                     // :284-285
+        xout = (double)x2; yout = (double)y2;
+        st = lk_level_verdict(A, status, iteration);
+        if (lk_level_lost(st)) break;
     }
-
-    if (lane == 0) {
-        if (my_iters) atomicAdd(iters_total, (unsigned long long)my_iters);
-        if (st == KLT_INTERNAL_ASSERT) {         // host raises; feature left untouched
-            if (A.assert_marks_feature) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = KLT_OOB; }
-            return;
-        }
-        const int W0 = A.p1.lv[0].w, H0 = A.p1.lv[0].h;
-        const bool oob = xout < A.borderx || xout > __dsub_rn((double)(W0 - 1), A.borderx) || yout < A.bordery ||
-                         yout > __dsub_rn((double)(H0 - 1), A.bordery);                      // _outOfBounds :140-141
-        if (st == KLT_OOB || oob) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = KLT_OOB; }
-        else if (st == KLT_SMALL_DET || st == KLT_LARGE_RESIDUE || st == KLT_MAX_ITERATIONS) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = st; }
-        else { xs[f] = xout; ys[f] = yout; vals[f] = KLT_TRACKED; }
-    }
+    if (lane == 0) lk_write_feature(A, f, st, xout, yout, my_iters, xs, ys, vals, iters_total);
 }
 
 
@@ -283,7 +264,7 @@ lk_track_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ xs, do
 // lane of the warp must call these (the shuffles are warp-wide); `ld` says whether this lane really loads.
 template <int W>
 __device__ __forceinline__ void patch_col(const float *__restrict__ img, int pitch, int ix, int iy, int i, bool ld,
-                                          float w00, float w01, float w10, float w11, float (&out)[W]) {
+                                          const Bilinear &w, float (&out)[W]) {
     const float *p = img + (ld ? (size_t)(iy - W / 2) * pitch + (ix - W / 2 + i) : 0);
     float a[W + 1], b[W + 1];
 #pragma unroll
@@ -291,7 +272,7 @@ __device__ __forceinline__ void patch_col(const float *__restrict__ img, int pit
 #pragma unroll
     for (int j = 0; j < W + 1; j++) b[j] = __shfl_down_sync(0xffffffffu, a[j], 1);
 #pragma unroll
-    for (int j = 0; j < W; j++) out[j] = fmaf(w11, b[j + 1], fmaf(w10, a[j + 1], fmaf(w01, b[j], w00 * a[j])));
+    for (int j = 0; j < W; j++) out[j] = w(a[j], b[j], a[j + 1], b[j + 1]);
 }
 
 // the three patches (image, gradx, grady) of one position: all 3*(W+1) loads are issued before the first use, so one
@@ -299,8 +280,7 @@ __device__ __forceinline__ void patch_col(const float *__restrict__ img, int pit
 template <int W>
 __device__ __forceinline__ void patch_col3(const float *__restrict__ i0, const float *__restrict__ i1,
                                            const float *__restrict__ i2, int pitch, int ix, int iy, int i, bool ld,
-                                           float w00, float w01, float w10, float w11, float (&o0)[W], float (&o1)[W],
-                                           float (&o2)[W]) {
+                                           const Bilinear &w, float (&o0)[W], float (&o1)[W], float (&o2)[W]) {
     const size_t off = ld ? (size_t)(iy - W / 2) * pitch + (ix - W / 2 + i) : 0;
     const float *p0 = i0 + off, *p1 = i1 + off, *p2 = i2 + off;
     float a0[W + 1], b0[W + 1], a1[W + 1], b1[W + 1], a2[W + 1], b2[W + 1];
@@ -319,9 +299,9 @@ __device__ __forceinline__ void patch_col3(const float *__restrict__ i0, const f
     }
 #pragma unroll
     for (int j = 0; j < W; j++) {
-        o0[j] = fmaf(w11, b0[j + 1], fmaf(w10, a0[j + 1], fmaf(w01, b0[j], w00 * a0[j])));
-        o1[j] = fmaf(w11, b1[j + 1], fmaf(w10, a1[j + 1], fmaf(w01, b1[j], w00 * a1[j])));
-        o2[j] = fmaf(w11, b2[j + 1], fmaf(w10, a2[j + 1], fmaf(w01, b2[j], w00 * a2[j])));
+        o0[j] = w(a0[j], b0[j], a0[j + 1], b0[j + 1]);
+        o1[j] = w(a1[j], b1[j], a1[j + 1], b1[j + 1]);
+        o2[j] = w(a2[j], b2[j], a2[j + 1], b2[j + 1]);
     }
 }
 
@@ -350,7 +330,7 @@ lk_track_rows_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ x
     constexpr int hw = W / 2;
     const double ss = (double)A.ss;
     double xloc = alive ? xs[f] : 0.0, yloc = alive ? ys[f] : 0.0;
-    for (int r = A.n_levels - 1; r >= 0; r--) { xloc /= ss; yloc /= ss; }
+    lk_top_level(xloc, yloc, A.n_levels, ss);
     double xout = xloc, yout = yloc;
     int st = KLT_TRACKED;
     unsigned int my_iters = 0;
@@ -365,16 +345,13 @@ lk_track_rows_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ x
         {
             const float x1 = (float)xloc, y1 = (float)yloc;
             const int ix = (int)x1, iy = (int)y1;
-            if (alive && !(ix - hw >= 0 && iy - hw >= 0 && ix + hw + 2 <= nc && iy + hw + 2 <= nr)) {   // pyx:35
+            if (alive && !lk_template_inside(ix, iy, hw, hw, nc, nr)) {
                 if (j == 0) atomicExch(assert_flag, 1);
                 st = KLT_INTERNAL_ASSERT;
                 alive = false;
             }
-            {
-                const float ax = x1 - (float)ix, ay = y1 - (float)iy;
-                const float w11 = ax * ay, w01 = ax - w11, w10 = ay - w11, w00 = 1.f - ax - ay + w11;
-                patch_col3<W>(I1, GX1, GY1, pitch, ix, iy, j, alive && col_ld, w00, w01, w10, w11, T, Tgx, Tgy);
-            }
+            patch_col3<W>(I1, GX1, GY1, pitch, ix, iy, j, alive && col_ld, Bilinear(x1 - (float)ix, y1 - (float)iy), T, Tgx,
+                          Tgy);
             if (!(alive && row_ok)) {
 #pragma unroll
                 for (int i = 0; i < W; i++) { T[i] = 0.f; Tgx[i] = 0.f; Tgy[i] = 0.f; }
@@ -385,17 +362,16 @@ lk_track_rows_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ x
         const float fnc = (float)nc, fnr = (float)nr, fhw = (float)hw;
         bool iterating = alive;
         while (__any_sync(0xffffffffu, iterating)) {
-            if (iterating && (x2 - fhw < 0.f || fnc - (x2 + fhw) < 1.001f || y2 - fhw < 0.f || fnr - (y2 + fhw) < 1.001f)) {
+            if (iterating && !lk_window_inside_f(x2, y2, fhw, fhw, fnc, fnr)) {
                 status = KLT_OOB;
                 iterating = false;
             }
             float gxx = 0.f, gxy = 0.f, gyy = 0.f, ex = 0.f, ey = 0.f;
             {
                 const int ix = (int)x2, iy = (int)y2;
-                const float ax = x2 - (float)ix, ay = y2 - (float)iy;
-                const float w11 = ax * ay, w01 = ax - w11, w10 = ay - w11, w00 = 1.f - ax - ay + w11;
                 float P[W], Px[W], Py[W];
-                patch_col3<W>(I2, GX2, GY2, pitch, ix, iy, j, iterating && col_ld, w00, w01, w10, w11, P, Px, Py);
+                patch_col3<W>(I2, GX2, GY2, pitch, ix, iy, j, iterating && col_ld, Bilinear(x2 - (float)ix, y2 - (float)iy), P,
+                              Px, Py);
                 if (iterating && row_ok) {
 #pragma unroll
                     for (int i = 0; i < W; i++) {
@@ -422,20 +398,14 @@ lk_track_rows_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ x
             }
         }
         my_iters += iteration;
-        if (alive) {
-            const double x2d = (double)x2, y2d = (double)y2, hwd = W / 2.0;
-            if (x2d - hwd < 0.0 || (double)nc - (x2d + hwd) < 1.001 || y2d - hwd < 0.0 || (double)nr - (y2d + hwd) < 1.001)
-                status = KLT_OOB;
-        }
+        if (alive && !lk_window_inside_d(x2, y2, W, W, nc, nr)) status = KLT_OOB;
         const bool need_res = alive && status == KLT_TRACKED && A.has_max_residue;
         if (__any_sync(0xffffffffu, need_res)) {
             float res = 0.f;
             {
                 const int ix = (int)x2, iy = (int)y2;
-                const float ax = x2 - (float)ix, ay = y2 - (float)iy;
-                const float w11 = ax * ay, w01 = ax - w11, w10 = ay - w11, w00 = 1.f - ax - ay + w11;
                 float P[W];
-                patch_col<W>(I2, pitch, ix, iy, j, need_res && col_ld, w00, w01, w10, w11, P);
+                patch_col<W>(I2, pitch, ix, iy, j, need_res && col_ld, Bilinear(x2 - (float)ix, y2 - (float)iy), P);
                 if (need_res && row_ok) {
 #pragma unroll
                     for (int i = 0; i < W; i++) res += fabsf(T[i] - P[i]);
@@ -446,26 +416,11 @@ lk_track_rows_kernel(const __grid_constant__ TrackArgs A, double *__restrict__ x
         }
         if (alive) {
             xout = (double)x2; yout = (double)y2;
-            if (A.retain) st = KLT_TRACKED;
-            else if (status == KLT_SMALL_DET || status == KLT_OOB || status == KLT_LARGE_RESIDUE) st = status;
-            else if (iteration >= A.max_iterations) st = KLT_MAX_ITERATIONS;
-            else st = KLT_TRACKED;
-            if (st == KLT_SMALL_DET || st == KLT_OOB) alive = false;                           // :284-285
+            st = lk_level_verdict(A, status, iteration);
+            if (lk_level_lost(st)) alive = false;
         }
     }
-    if (was_alive && j == 0) {
-        if (my_iters) atomicAdd(iters_total, (unsigned long long)my_iters);
-        if (st == KLT_INTERNAL_ASSERT) {
-            if (A.assert_marks_feature) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = KLT_OOB; }
-            return;
-        }
-        const int W0 = A.p1.lv[0].w, H0 = A.p1.lv[0].h;
-        const bool oob = xout < A.borderx || xout > (double)(W0 - 1) - A.borderx || yout < A.bordery ||
-                         yout > (double)(H0 - 1) - A.bordery;
-        if (st == KLT_OOB || oob) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = KLT_OOB; }
-        else if (st == KLT_SMALL_DET || st == KLT_LARGE_RESIDUE || st == KLT_MAX_ITERATIONS) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = st; }
-        else { xs[f] = xout; ys[f] = yout; vals[f] = KLT_TRACKED; }
-    }
+    if (was_alive && j == 0) lk_write_feature(A, f, st, xout, yout, my_iters, xs, ys, vals, iters_total);
 }
 
 template <int W>
@@ -584,7 +539,7 @@ int klt_launch_track_fb(klt_ctx *ctx, const klt_params *p, const klt_pyr *p1, co
 __global__ void extract_patch_kernel(const float *__restrict__ img, int pitch, int nc, int nr, float x, float y,
                                      int height, int width, float *__restrict__ out, int *__restrict__ ok) {
     const int ix = (int)x, iy = (int)y, hw = width / 2, hh = height / 2;
-    if (!(ix - hw >= 0 && iy - hh >= 0 && ix + hw + 2 <= nc && iy + hh + 2 <= nr)) {
+    if (!lk_template_inside(ix, iy, hw, hh, nc, nr)) {
         if (threadIdx.x == 0) *ok = 0;
         return;
     }
@@ -630,7 +585,7 @@ int klt_launch_iterate(klt_ctx *ctx, const klt_params *p, const float *tpatch_de
 __global__ void patch_combine_kernel(const float *__restrict__ p1, const float *__restrict__ img, int pitch, int nc, int nr,
                                      float x, float y, int height, int width, int mode, float *__restrict__ out, int *__restrict__ ok) {
     const int ix = (int)x, iy = (int)y, hw = width / 2, hh = height / 2;
-    if (!(ix - hw >= 0 && iy - hh >= 0 && ix + hw + 2 <= nc && iy + hh + 2 <= nr)) {
+    if (!lk_template_inside(ix, iy, hw, hh, nc, nr)) {
         if (threadIdx.x == 0) *ok = 0;
         return;
     }

@@ -113,18 +113,16 @@ __device__ __forceinline__ void stage_reflect(float *__restrict__ dst, const flo
     }
 }
 
-__device__ __forceinline__ float bil(const float *p, int P, float w00, float w01, float w10, float w11) {
-    return fmaf(w11, p[P + 1], fmaf(w10, p[P], fmaf(w01, p[1], w00 * p[0])));
-}
+__device__ __forceinline__ float bil(const float *p, int P, const Bilinear &w) { return w(p[0], p[1], p[P], p[P + 1]); }
 // bilinear sample of an interleaved (gx, gy) plane: four 64-bit loads for both gradients; P = pitch in pairs
-__device__ __forceinline__ float2 bil2(const float *p, int P, float w00, float w01, float w10, float w11) {
+__device__ __forceinline__ float2 bil2(const float *p, int P, const Bilinear &w) {
     const float2 a = *reinterpret_cast<const float2 *>(p), b = *reinterpret_cast<const float2 *>(p + 2);
     const float2 c = *reinterpret_cast<const float2 *>(p + 2 * P), d = *reinterpret_cast<const float2 *>(p + 2 * P + 2);
-    return make_float2(fmaf(w11, d.x, fmaf(w10, c.x, fmaf(w01, b.x, w00 * a.x))),
-                       fmaf(w11, d.y, fmaf(w10, c.y, fmaf(w01, b.y, w00 * a.y))));
+    return make_float2(w(a.x, b.x, c.x, d.x), w(a.y, b.y, c.y, d.y));
 }
 
-// sum over the LPF lanes of a feature, result in every lane of the group
+// sum over the LPF lanes of a feature, result in every lane of the group.  Not lk_track_rows' group_sum: that one
+// pairs the lanes in the opposite order, and the order is part of the rounded result.
 template <int LPF>
 __device__ __forceinline__ float group_sum(float v) {
 #pragma unroll
@@ -222,9 +220,9 @@ lk_windowed_kernel(const __grid_constant__ TrackArgs A, const __grid_constant__ 
     const float *const plane1 = A.p1.base + (size_t)image * A.p1.plane_floats;      // intensity planes of this feature's pair
     const float *const plane2 = A.p2.base + (size_t)image * A.p2.plane_floats;
     constexpr int hw = W / 2;
-    const double ss = (double)A.ss, inv_ss = 1.0 / ss;        // subsampling is a power of two: x * inv_ss == x / ss exactly
+    const double ss = (double)A.ss;
     double xloc = alive ? xs[f] : 0.0, yloc = alive ? ys[f] : 0.0;
-    for (int r = A.n_levels - 1; r >= 0; r--) { xloc *= inv_ss; yloc *= inv_ss; }
+    lk_top_level(xloc, yloc, A.n_levels, ss);
     double xout = xloc, yout = yloc;
     int st = KLT_TRACKED;
     unsigned int my_iters = 0;
@@ -245,7 +243,7 @@ lk_windowed_kernel(const __grid_constant__ TrackArgs A, const __grid_constant__ 
         const int nc = A.p1.lv[r].w, nr = A.p1.lv[r].h, pitch = A.p1.lv[r].pitch;
         const float x1 = (float)xloc, y1 = (float)yloc;
         const int ix1 = (int)x1, iy1 = (int)y1;
-        if (alive && !(ix1 - hw >= 0 && iy1 - hw >= 0 && ix1 + hw + 2 <= nc && iy1 + hw + 2 <= nr)) {   // pyx:35
+        if (alive && !lk_template_inside(ix1, iy1, hw, hw, nc, nr)) {
             if (q == 0) atomicExch(assert_flag, 1);
             st = KLT_INTERNAL_ASSERT;
             alive = false;
@@ -257,7 +255,7 @@ lk_windowed_kernel(const __grid_constant__ TrackArgs A, const __grid_constant__ 
         // MARGIN pixels inside.  (gix, giy): window position the gradients in shared memory belong to.
         int rx0 = (int)x2 - hw - MARGIN, ry0 = (int)y2 - hw - MARGIN;
         int gix = -0x40000000, giy = -0x40000000;
-        const bool start_inside = alive && !(x2 - fhw < 0.f || fnc - (x2 + fhw) < 1.001f || y2 - fhw < 0.f || fnr - (y2 + fhw) < 1.001f);
+        const bool start_inside = alive && lk_window_inside_f(x2, y2, fhw, fhw, fnc, fnr);
 
         // ---- one memory round trip: both regions of this level (TMA boxes; 'reflect' regions by element) ----
         // issue(do1, do2): group-uniform flags; returns whether the group has to wait on its mbarrier
@@ -308,15 +306,14 @@ lk_windowed_kernel(const __grid_constant__ TrackArgs A, const __grid_constant__ 
         // ---- template: the first image's window, gradients interpolated like the image (trackFeatures.py:87-92) ----
         float T[C::PX], Tgx[C::PX], Tgy[C::PX];
         {
-            const float ax = x1 - (float)ix1, ay = y1 - (float)iy1;
-            const float w11 = ax * ay, w01 = ax - w11, w10 = ay - w11, w00 = 1.f - ax - ay + w11;
+            const Bilinear w(x1 - (float)ix1, y1 - (float)iy1);
 #pragma unroll
             for (int i = 0; i < C::PX; i++) {
                 const bool on = alive && col_on && (C::RPR * i + rr < W);
                 T[i] = 0.f; Tgx[i] = 0.f; Tgy[i] = 0.f;
                 if (on) {
-                    T[i] = bil(i1 + (C::RPR * i + rr + RG) * C::P1 + pc + RG, C::P1, w00, w01, w10, w11);
-                    const float2 tg = bil2(g1 + po + 2 * C::RPR * i * C::GP, C::GP, w00, w01, w10, w11);
+                    T[i] = bil(i1 + (C::RPR * i + rr + RG) * C::P1 + pc + RG, C::P1, w);
+                    const float2 tg = bil2(g1 + po + 2 * C::RPR * i * C::GP, C::GP, w);
                     Tgx[i] = tg.x; Tgy[i] = tg.y;
                 }
             }
@@ -326,7 +323,7 @@ lk_windowed_kernel(const __grid_constant__ TrackArgs A, const __grid_constant__ 
         int ox = MARGIN, oy = MARGIN;
         bool iterating = alive;
         for (;;) {
-            if (iterating && (x2 - fhw < 0.f || fnc - (x2 + fhw) < 1.001f || y2 - fhw < 0.f || fnr - (y2 + fhw) < 1.001f)) {
+            if (iterating && !lk_window_inside_f(x2, y2, fhw, fhw, fnc, fnr)) {
                 status = KLT_OOB;
                 iterating = false;
             }
@@ -344,16 +341,15 @@ lk_windowed_kernel(const __grid_constant__ TrackArgs A, const __grid_constant__ 
                 gradient_pair<W, C::P2>(i2 + oy * C::P2 + ox, tpl, g2, moved, K.g2, K.d2, th2, q);
                 if (moved) { gix = ix; giy = iy; }
             }
-            const float ax = x2 - (float)ix, ay = y2 - (float)iy;
-            const float w11 = ax * ay, w01 = ax - w11, w10 = ay - w11, w00 = 1.f - ax - ay + w11;
+            const Bilinear w(x2 - (float)ix, y2 - (float)iy);
             const float *bi = i2 + (oy + rr + RG) * C::P2 + ox + pc + RG;
             float gxx = 0.f, gxy = 0.f, gyy = 0.f, ex = 0.f, ey = 0.f;
             if (iterating && col_on) {
 #pragma unroll
                 for (int i = 0; i < C::PX; i++) {
                     if (C::RPR * (i + 1) <= W || C::RPR * i + rr < W) {      // (compile-time true except in the last round)
-                        const float Pv = bil(bi + C::RPR * i * C::P2, C::P2, w00, w01, w10, w11);
-                        const float2 Pg = bil2(g2 + po + 2 * C::RPR * i * C::GP, C::GP, w00, w01, w10, w11);
+                        const float Pv = bil(bi + C::RPR * i * C::P2, C::P2, w);
+                        const float2 Pg = bil2(g2 + po + 2 * C::RPR * i * C::GP, C::GP, w);
                         const float diff = T[i] - Pv, gx = Tgx[i] + Pg.x, gy = Tgy[i] + Pg.y;
                         gxx = fmaf(gx, gx, gxx); gxy = fmaf(gx, gy, gxy); gyy = fmaf(gy, gy, gyy);
                         ex = fmaf(diff, gx, ex); ey = fmaf(diff, gy, ey);
@@ -378,11 +374,7 @@ lk_windowed_kernel(const __grid_constant__ TrackArgs A, const __grid_constant__ 
             }
         }
         my_iters += iteration;
-        if (alive) {
-            const double x2d = (double)x2, y2d = (double)y2, hwd = W / 2.0;
-            if (x2d - hwd < 0.0 || (double)nc - (x2d + hwd) < 1.001 || y2d - hwd < 0.0 || (double)nr - (y2d + hwd) < 1.001)
-                status = KLT_OOB;
-        }
+        if (alive && !lk_window_inside_d(x2, y2, W, W, nc, nr)) status = KLT_OOB;
         const bool need_res = alive && status == KLT_TRACKED && A.has_max_residue;
         if (__any_sync(FULL, need_res)) {
             const int ix = (int)x2, iy = (int)y2;
@@ -393,15 +385,14 @@ lk_windowed_kernel(const __grid_constant__ TrackArgs A, const __grid_constant__ 
                 if (left) { rx0 = ix - hw - MARGIN; ry0 = iy - hw - MARGIN; ox = MARGIN; oy = MARGIN; }
                 arrive(issue(false, left));
             }
-            const float ax = x2 - (float)ix, ay = y2 - (float)iy;
-            const float w11 = ax * ay, w01 = ax - w11, w10 = ay - w11, w00 = 1.f - ax - ay + w11;
+            const Bilinear w(x2 - (float)ix, y2 - (float)iy);
             const float *bi = i2 + (oy + rr + RG) * C::P2 + ox + pc + RG;
             float res = 0.f;
             if (need_res && col_on) {
 #pragma unroll
                 for (int i = 0; i < C::PX; i++)
                     if (C::RPR * (i + 1) <= W || C::RPR * i + rr < W)
-                        res += fabsf(T[i] - bil(bi + C::RPR * i * C::P2, C::P2, w00, w01, w10, w11));
+                        res += fabsf(T[i] - bil(bi + C::RPR * i * C::P2, C::P2, w));
             }
             res = group_sum<C::LPF>(res) / (float)(W * W);
             if (need_res && res > A.max_residue) status = KLT_LARGE_RESIDUE;
@@ -409,26 +400,11 @@ lk_windowed_kernel(const __grid_constant__ TrackArgs A, const __grid_constant__ 
         __syncwarp();                              // all lanes are done with the regions before the next level overwrites them
         if (alive) {
             xout = (double)x2; yout = (double)y2;
-            if (A.retain) st = KLT_TRACKED;
-            else if (status == KLT_SMALL_DET || status == KLT_OOB || status == KLT_LARGE_RESIDUE) st = status;
-            else if (iteration >= A.max_iterations) st = KLT_MAX_ITERATIONS;
-            else st = KLT_TRACKED;
-            if (st == KLT_SMALL_DET || st == KLT_OOB) alive = false;                           // :284-285
+            st = lk_level_verdict(A, status, iteration);
+            if (lk_level_lost(st)) alive = false;
         }
     }
-    if (was_alive && q == 0) {
-        if (my_iters) atomicAdd(iters_total, (unsigned long long)my_iters);
-        if (st == KLT_INTERNAL_ASSERT) {
-            if (A.assert_marks_feature) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = KLT_OOB; }
-            return;
-        }
-        const int W0 = A.p1.lv[0].w, H0 = A.p1.lv[0].h;
-        const bool oob = xout < A.borderx || xout > (double)(W0 - 1) - A.borderx || yout < A.bordery ||
-                         yout > (double)(H0 - 1) - A.bordery;
-        if (st == KLT_OOB || oob) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = KLT_OOB; }
-        else if (st == KLT_SMALL_DET || st == KLT_LARGE_RESIDUE || st == KLT_MAX_ITERATIONS) { xs[f] = -1.0; ys[f] = -1.0; vals[f] = st; }
-        else { xs[f] = xout; ys[f] = yout; vals[f] = KLT_TRACKED; }
-    }
+    if (was_alive && q == 0) lk_write_feature(A, f, st, xout, yout, my_iters, xs, ys, vals, iters_total);
 }
 
 // ---- host side: tensor maps ---------------------------------------------------------------------------------------
