@@ -38,8 +38,6 @@ int klt_ws_reserve(klt_ctx *ctx, size_t bytes) {
     return KLT_OK;
 }
 
-static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
 int klt_prof_begin(klt_ctx *ctx, const char *name, double bytes) {
     if (!ctx->profiling) return -1;
     int rec = -1;
@@ -224,32 +222,19 @@ int klt_timer_elapsed_ms(klt_ctx *ctx, float *ms) {
 }
 
 // ---- operator level ---------------------------------------------------------------------------------------
-// Stages host images in the workspace when needed.  Layout: [in][out0][out1].
-static int stage_in(klt_ctx *ctx, const float *in, size_t n, size_t slot, size_t nslots, const float **dev) {
-    const size_t plane = align_up(n * sizeof(float), 256);
-    int rc = klt_ws_reserve(ctx, nslots * plane);
-    if (rc) return rc;
-    float *d = (float *)((char *)ctx->ws + slot * plane);
-    KLT_CUDA(ctx, cudaMemcpyAsync(d, in, n * sizeof(float), cudaMemcpyDefault, ctx->stream));
-    *dev = d;
-    return KLT_OK;
-}
-
 int klt_convolve_separable_f32(klt_ctx *ctx, const float *in, int w, int h, const klt_kernel1d *hk,
                                const klt_kernel1d *vk, int precision, float *out) {
     if (!ctx || !in || !out || w <= 0 || h <= 0) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)w * h, plane = align_up(n * sizeof(float), 256);
-    int rc = klt_ws_reserve(ctx, 2 * plane);
-    if (rc) return rc;
-    const float *din = in;
-    float *dout = out;
-    const bool in_host = !klt_is_device_ptr(in), out_host = !klt_is_device_ptr(out);
-    if (in_host && (rc = stage_in(ctx, in, n, 0, 2, &din))) return rc;
-    if (out_host) dout = (float *)((char *)ctx->ws + plane);
-    if ((rc = klt_launch_conv_sep_f32(ctx, din, w, 0, dout, w, 0, w, h, 1, hk, vk, precision))) return rc;
-    if (out_host) {
-        KLT_CUDA(ctx, cudaMemcpyAsync(out, dout, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    const size_t n = (size_t)w * h;
+    KltArg<const float> din = klt_arg(in, n);
+    KltArg<float> dout = klt_arg(out, n);
+    int rc;
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { din.place(c); dout.place(c); }))) return rc;
+    if ((rc = klt_stage_in(ctx, din))) return rc;
+    if ((rc = klt_launch_conv_sep_f32(ctx, din.dev, w, 0, dout.dev, w, 0, w, h, 1, hk, vk, precision))) return rc;
+    if (dout.host) {
+        if ((rc = klt_stage_out(ctx, dout))) return rc;
         KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     }
     return KLT_OK;
@@ -263,19 +248,16 @@ int klt_gradients_f32(klt_ctx *ctx, const float *in, int w, int h, const klt_ker
                       int precision, float *gradx, float *grady) {
     if (!ctx || !in || !gradx || !grady || w <= 0 || h <= 0) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)w * h, plane = align_up(n * sizeof(float), 256);
-    int rc = klt_ws_reserve(ctx, 3 * plane);
-    if (rc) return rc;
-    const float *din = in;
-    const bool in_host = !klt_is_device_ptr(in), out_host = !klt_is_device_ptr(gradx);
-    if (out_host != !klt_is_device_ptr(grady)) return klt_fail(ctx, KLT_ERR_INVALID, "gradx and grady must both be host or both be device");
-    if (in_host && (rc = stage_in(ctx, in, n, 0, 3, &din))) return rc;
-    float *dgx = out_host ? (float *)((char *)ctx->ws + plane) : gradx;
-    float *dgy = out_host ? (float *)((char *)ctx->ws + 2 * plane) : grady;
-    if ((rc = klt_launch_grad_pair(ctx, din, w, 0, dgx, dgy, w, 0, w, h, 1, gauss, deriv, precision))) return rc;
-    if (out_host) {
-        KLT_CUDA(ctx, cudaMemcpyAsync(gradx, dgx, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(grady, dgy, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    const size_t n = (size_t)w * h;
+    KltArg<const float> din = klt_arg(in, n);
+    KltArg<float> dgx = klt_arg(gradx, n), dgy = klt_arg(grady, n);
+    if (dgx.host != dgy.host) return klt_fail(ctx, KLT_ERR_INVALID, "gradx and grady must both be host or both be device");
+    int rc;
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { din.place(c); dgx.place(c); dgy.place(c); }))) return rc;
+    if ((rc = klt_stage_in(ctx, din))) return rc;
+    if ((rc = klt_launch_grad_pair(ctx, din.dev, w, 0, dgx.dev, dgy.dev, w, 0, w, h, 1, gauss, deriv, precision))) return rc;
+    if (dgx.host) {
+        if ((rc = klt_stage_out(ctx, dgx)) || (rc = klt_stage_out(ctx, dgy))) return rc;
         KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     }
     return KLT_OK;
@@ -427,14 +409,9 @@ int klt_pyr_build_u8(klt_ctx *ctx, klt_pyr *p, const uint8_t *frames, size_t pit
     if ((rc = check_taps(ctx, taps))) return rc;
     if (pitch < (size_t)p->w) return klt_fail(ctx, KLT_ERR_INVALID, "pitch %zu smaller than width %d", pitch, p->w);
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-    const uint8_t *dframes = frames;
-    if (!klt_is_device_ptr(frames)) {
-        const size_t bytes = (size_t)(p->batch - 1) * frame_stride + (size_t)(p->h - 1) * pitch + p->w;
-        if ((rc = klt_ws_reserve(ctx, bytes))) return rc;
-        KLT_CUDA(ctx, cudaMemcpyAsync(ctx->ws, frames, bytes, cudaMemcpyHostToDevice, ctx->stream));
-        dframes = (const uint8_t *)ctx->ws;
-    }
-    return klt_build_u8_device(ctx, p, dframes, pitch, frame_stride, taps, precision, 0, p->batch, nullptr);
+    KltArg<const uint8_t> df = klt_arg(frames, (size_t)(p->batch - 1) * frame_stride + (size_t)(p->h - 1) * pitch + p->w);
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { df.place(c); })) || (rc = klt_stage_in(ctx, df))) return rc;
+    return klt_build_u8_device(ctx, p, df.dev, pitch, frame_stride, taps, precision, 0, p->batch, nullptr);
 }
 
 int klt_pyr_build_f32(klt_ctx *ctx, klt_pyr *p, const float *images, size_t pitch, size_t frame_stride,
@@ -450,14 +427,9 @@ int klt_pyr_build_f32(klt_ctx *ctx, klt_pyr *p, const float *images, size_t pitc
             KLT_CUDA(ctx, cudaMemcpy2DAsync(p->level(0, b, 0), p->lv[0].pitch * sizeof(float), images + (size_t)b * frame_stride,
                                             pitch * sizeof(float), p->w * sizeof(float), p->h, cudaMemcpyDefault, ctx->stream));
     } else {
-        const float *dimg = images;
-        if (!klt_is_device_ptr(images)) {
-            const size_t elems = (size_t)(p->batch - 1) * frame_stride + (size_t)(p->h - 1) * pitch + p->w;
-            if ((rc = klt_ws_reserve(ctx, elems * sizeof(float)))) return rc;
-            KLT_CUDA(ctx, cudaMemcpyAsync(ctx->ws, images, elems * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-            dimg = (const float *)ctx->ws;
-        }
-        if ((rc = klt_launch_conv_sep_f32(ctx, dimg, pitch, frame_stride, p->level(0, 0, 0), p->lv[0].pitch, p->plane_floats, p->w,
+        KltArg<const float> dimg = klt_arg(images, (size_t)(p->batch - 1) * frame_stride + (size_t)(p->h - 1) * pitch + p->w);
+        if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { dimg.place(c); })) || (rc = klt_stage_in(ctx, dimg))) return rc;
+        if ((rc = klt_launch_conv_sep_f32(ctx, dimg.dev, pitch, frame_stride, p->level(0, 0, 0), p->lv[0].pitch, p->plane_floats, p->w,
                                           p->h, p->batch, &taps->smooth, &taps->smooth, p->precision))) return rc;
     }
     if ((rc = build_levels(ctx, p, 1, 0, p->batch))) return rc;
@@ -496,25 +468,16 @@ int klt_scan_good_features(klt_ctx *ctx, const float *gradx, const float *grady,
     int nx = 0, ny = 0;
     if (w - borderx > borderx) nx = (w - 2 * borderx + step - 1) / step;
     if (h - bordery > bordery) ny = (h - 2 * bordery + step - 1) / step;
-    const size_t n = (size_t)w * h, plane = align_up(n * sizeof(float), 256);
-    int rc = klt_ws_reserve(ctx, 6 * plane);
-    if (rc) return rc;
-    char *wsp = (char *)ctx->ws;
-    float *dval = (float *)(wsp + 3 * plane);
-    const float *dgx = gradx, *dgy = grady;
-    if (!klt_is_device_ptr(gradx)) {
-        float *d = (float *)(wsp + 4 * plane);
-        KLT_CUDA(ctx, cudaMemcpyAsync(d, gradx, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-        dgx = d;
-    }
-    if (!klt_is_device_ptr(grady)) {
-        float *d = (float *)(wsp + 5 * plane);
-        KLT_CUDA(ctx, cudaMemcpyAsync(d, grady, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-        dgy = d;
-    }
-    if ((rc = klt_launch_scan(ctx, dgx, dgy, w, w, h, borderx, bordery, window_hw, window_hh, n_skipped_pixels, dval, nx, ny))) return rc;
-    if (nx > 0 && ny > 0)
-        KLT_CUDA(ctx, cudaMemcpyAsync(val, dval, (size_t)nx * ny * sizeof(float), cudaMemcpyDefault, ctx->stream));
+    const size_t n = (size_t)w * h;
+    KltArg<const float> dgx = klt_arg(gradx, n), dgy = klt_arg(grady, n);
+    KltArg<float> dval = klt_arg_staged(val, (size_t)nx * ny);
+    float *sat;
+    int rc;
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { sat = c.take<float>(3 * n); dval.place(c); dgx.place(c); dgy.place(c); }))) return rc;
+    if ((rc = klt_stage_in(ctx, dgx)) || (rc = klt_stage_in(ctx, dgy))) return rc;
+    if ((rc = klt_launch_scan(ctx, dgx.dev, dgy.dev, w, w, h, borderx, bordery, window_hw, window_hh, n_skipped_pixels, sat, dval.dev,
+                              nx, ny))) return rc;
+    if (nx > 0 && ny > 0 && (rc = klt_stage_out(ctx, dval))) return rc;
     KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return KLT_OK;
 }
@@ -594,56 +557,49 @@ static int track_impl(klt_ctx *ctx, const klt_params *params, const klt_pyr *pyr
         if (params->affine_consistency_check < 0 || params->affine_consistency_check > 2) return klt_fail(ctx, KLT_ERR_INVALID, "affine_consistency_check must be 0, 1 or 2");
         if (params->affine_window_width != aff->aw || params->affine_window_height != aff->ah) return klt_fail(ctx, KLT_ERR_INVALID, "affine window differs from the affine state's");
     }
-    const bool host = !klt_is_device_ptr(x);
-    if (host != !klt_is_device_ptr(y) || host != !klt_is_device_ptr(val)) return klt_fail(ctx, KLT_ERR_INVALID, "x, y, val must all be host or all be device");
-    const size_t fbytes = align_up(total * sizeof(double), 256);
-    // [iterations, assert word, backward assert word][x, y, val staging][affine: x_in, y_in, val_in | fb: x0, y0, vb, xb, yb, fb_error staging]
-    if ((rc = klt_ws_reserve(ctx, (fb ? 9 : 6) * fbytes + 256))) return rc;
-    char *wsp = (char *)ctx->ws;
-    unsigned long long *iters = (unsigned long long *)wsp;
+    KltFeatures f;
+    if ((rc = klt_features(ctx, x, y, val, total, &f))) return rc;
+    KltArg<float> dfb = klt_arg(fb ? fb_error : nullptr, total);
+    KltTrackStatus *st = nullptr;
+    double *x_in = nullptr, *y_in = nullptr;      // the affine block's pre-track positions (xloc, yloc) and which features were live
+    int32_t *val_in = nullptr;
+    FbArrays fa{};
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) {
+            st = c.take<KltTrackStatus>(1);
+            f.place(c);
+            if (aff) { x_in = c.take<double>(total); y_in = c.take<double>(total); val_in = c.take<int32_t>(total); }
+            if (fb) {
+                fa.x0 = c.take<double>(total); fa.y0 = c.take<double>(total); fa.xb = c.take<double>(total); fa.yb = c.take<double>(total);
+                fa.vb = c.take<int32_t>(total);
+            }
+            dfb.place(c);
+        }))) return rc;
+    fa.scratch_assert = &st->scratch_assert;
     // calls that return without reading the flag back (asynchronous, or device arrays without n_iterations) raise the context's
     // sticky flag instead: klt_sync / klt_async_result report it
-    const bool deferred = async || (!host && !n_iterations);
+    const bool deferred = async || (!f.x.host && !n_iterations);
     if (deferred && !ctx->async_flag_dev) return klt_fail(ctx, KLT_ERR_NOMEM, "the context has no status word");
-    int *aflag = deferred ? ctx->async_flag_dev : (int *)(wsp + 8);
-    double *dx = x, *dy = y;
-    int32_t *dval = val;
-    KLT_CUDA(ctx, cudaMemsetAsync(wsp, 0, 16, ctx->stream));
-    if (host) {
-        dx = (double *)(wsp + 256); dy = (double *)(wsp + 256 + fbytes); dval = (int32_t *)(wsp + 256 + 2 * fbytes);
-        KLT_CUDA(ctx, cudaMemcpyAsync(dx, x, total * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(dy, y, total * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(dval, val, total * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+    int *aflag = deferred ? ctx->async_flag_dev : &st->asserted;
+    KLT_CUDA(ctx, cudaMemsetAsync(st, 0, sizeof *st, ctx->stream));
+    if ((rc = klt_stage_in(ctx, f))) return rc;
+    if (aff) {
+        KLT_CUDA(ctx, cudaMemcpyAsync(x_in, f.x.dev, total * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        KLT_CUDA(ctx, cudaMemcpyAsync(y_in, f.y.dev, total * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        KLT_CUDA(ctx, cudaMemcpyAsync(val_in, f.val.dev, total * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
     }
-    double *x_in = nullptr, *y_in = nullptr;
-    int32_t *val_in = nullptr;
-    if (aff) {   // the affine block needs the pre-track positions (xloc, yloc) and which features were live
-        x_in = (double *)(wsp + 256 + 3 * fbytes); y_in = (double *)(wsp + 256 + 4 * fbytes); val_in = (int32_t *)(wsp + 256 + 5 * fbytes);
-        KLT_CUDA(ctx, cudaMemcpyAsync(x_in, dx, total * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(y_in, dy, total * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(val_in, dval, total * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
-    }
-    const bool fb_host = fb && fb_error && !klt_is_device_ptr(fb_error);
-    float *dfb = fb_host ? (float *)(wsp + 256 + 8 * fbytes) : fb_error;
     if (fb) {
-        const FbArrays fa{(double *)(wsp + 256 + 3 * fbytes), (double *)(wsp + 256 + 4 * fbytes), (double *)(wsp + 256 + 6 * fbytes),
-                          (double *)(wsp + 256 + 7 * fbytes), (int32_t *)(wsp + 256 + 5 * fbytes), (int *)(wsp + 12)};
-        if ((rc = klt_launch_track_fb(ctx, params, pyr1, pyr2, n_per_image, max_fb_error, dx, dy, dval, fa, dfb, iters, aflag))) return rc;
-    } else if ((rc = klt_launch_track(ctx, params, pyr1, pyr2, n_per_image, dx, dy, dval, iters, aflag))) return rc;
-    if (aff && (rc = klt_launch_affine(ctx, params, pyr1, pyr2, n_per_image, x_in, y_in, val_in, dx, dy, dval, aff, aflag))) return rc;
-    if (host) {
-        KLT_CUDA(ctx, cudaMemcpyAsync(x, dx, total * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(y, dy, total * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(val, dval, total * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    }
-    if (fb_host) KLT_CUDA(ctx, cudaMemcpyAsync(fb_error, dfb, total * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+        if ((rc = klt_launch_track_fb(ctx, params, pyr1, pyr2, n_per_image, max_fb_error, f.x.dev, f.y.dev, f.val.dev, fa, dfb.dev,
+                                      &st->iters, aflag))) return rc;
+    } else if ((rc = klt_launch_track(ctx, params, pyr1, pyr2, n_per_image, f.x.dev, f.y.dev, f.val.dev, &st->iters, aflag))) return rc;
+    if (aff && (rc = klt_launch_affine(ctx, params, pyr1, pyr2, n_per_image, x_in, y_in, val_in, f.x.dev, f.y.dev, f.val.dev, aff, aflag))) return rc;
+    if ((rc = klt_stage_out(ctx, f)) || (rc = klt_stage_out(ctx, dfb))) return rc;
     if (async) return KLT_OK;                    // results land when the stream gets there: klt_sync / klt_async_result
-    if (host || n_iterations) {
-        unsigned long long res[2] = {0, 0};
-        KLT_CUDA(ctx, cudaMemcpyAsync(res, wsp, 16, cudaMemcpyDeviceToHost, ctx->stream));
+    if (f.x.host || n_iterations) {
+        KltTrackStatus res{};
+        KLT_CUDA(ctx, cudaMemcpyAsync(&res, st, sizeof res, cudaMemcpyDeviceToHost, ctx->stream));
         KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        if (n_iterations) *n_iterations = (int64_t)res[0];
-        if ((int)(res[1] & 0xffffffffull))
+        if (n_iterations) *n_iterations = (int64_t)res.iters;
+        if (res.asserted)
             return klt_fail(ctx, KLT_ERR_ASSERT, "a feature window leaves the image at a pyramid level: the reference raises AssertionError (trackFeaturesUtils.pyx:35)");
     }
     return KLT_OK;
@@ -673,17 +629,15 @@ int klt_affine_create(klt_ctx *ctx, int n, int aw, int ah, klt_affine **out) {
     klt_affine *a = new klt_affine();
     a->n = n; a->aw = aw; a->ah = ah;
     const size_t tn = (size_t)(aw + 2) * (ah + 2);
-    const size_t b_has = align_up((size_t)n * 4 + 4, 256), b_f = align_up((size_t)n * 4 + 4, 256), b_A = align_up((size_t)n * 16 + 16, 256);
-    const size_t bytes = b_has + 2 * b_f + b_A + (size_t)n * 3 * tn * 4 + 256;
-    cudaError_t e = cudaMalloc(&a->block, bytes);
-    if (e != cudaSuccess) { delete a; return klt_fail(ctx, KLT_ERR_NOMEM, "cudaMalloc(%zu) for affine state failed: %s", bytes, cudaGetErrorString(e)); }
-    char *b = (char *)a->block;
-    a->has = (int *)b; b += b_has;
-    a->aff_x = (float *)b; b += b_f;
-    a->aff_y = (float *)b; b += b_f;
-    a->A = (float *)b; b += b_A;
-    a->tmpl = (float *)b;
-    int rc = klt_launch_affine_reset(ctx, a, nullptr);
+    int rc = klt_alloc_layout(ctx, &a->block, "affine state", [&](KltCarver &c) {
+        a->has = c.take<int>((size_t)n + 1);
+        a->aff_x = c.take<float>((size_t)n + 1);
+        a->aff_y = c.take<float>((size_t)n + 1);
+        a->A = c.take<float>(4 * (size_t)n + 4);
+        a->tmpl = c.take<float>((size_t)n * 3 * tn + 64);
+    });
+    if (rc) { delete a; return rc; }
+    rc = klt_launch_affine_reset(ctx, a, nullptr);
     if (rc) { cudaFree(a->block); delete a; return rc; }
     *out = a;
     return KLT_OK;
@@ -701,10 +655,10 @@ int klt_affine_reset(klt_ctx *ctx, klt_affine *a, const int32_t *mask) {
     if (!ctx || !a) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
     if (!mask) return klt_launch_affine_reset(ctx, a, nullptr);
-    int rc = klt_ws_reserve(ctx, (size_t)a->n * 4 + 256);
-    if (rc) return rc;
-    KLT_CUDA(ctx, cudaMemcpyAsync(ctx->ws, mask, (size_t)a->n * 4, cudaMemcpyDefault, ctx->stream));
-    return klt_launch_affine_reset(ctx, a, (const int *)ctx->ws);
+    KltArg<const int32_t> dmask = klt_arg_staged(mask, (size_t)a->n);
+    int rc;
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { dmask.place(c); })) || (rc = klt_stage_in(ctx, dmask))) return rc;
+    return klt_launch_affine_reset(ctx, a, (const int *)dmask.dev);
 }
 
 int klt_affine_download(klt_ctx *ctx, const klt_affine *a, int32_t *has_template, float *aff_x, float *aff_y, float *A) {
@@ -729,20 +683,15 @@ int klt_affine_download_template(klt_ctx *ctx, const klt_affine *a, int slot, fl
 int klt_extract_patch(klt_ctx *ctx, const float *img, int w, int h, float x, float y, int height, int width, float *out) {
     if (!ctx || !img || !out || w <= 0 || h <= 0 || width < 1 || height < 1) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)w * h, plane = align_up(n * sizeof(float), 256), pbytes = align_up((size_t)width * height * sizeof(float), 256);
-    int rc = klt_ws_reserve(ctx, plane + pbytes + 256);
-    if (rc) return rc;
-    char *wsp = (char *)ctx->ws;
-    const float *dimg = img;
-    if (!klt_is_device_ptr(img)) {
-        KLT_CUDA(ctx, cudaMemcpyAsync(wsp, img, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-        dimg = (const float *)wsp;
-    }
-    float *dout = (float *)(wsp + plane);
-    int *dok = (int *)(wsp + plane + pbytes);
-    if ((rc = klt_launch_extract_patch(ctx, dimg, w, w, h, x, y, height, width, dout, dok))) return rc;
+    KltArg<const float> dimg = klt_arg(img, (size_t)w * h);
+    KltArg<float> dout = klt_arg_staged(out, (size_t)width * height);
+    int *dok;
+    int rc;
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { dimg.place(c); dout.place(c); dok = c.take<int>(1); }))) return rc;
+    if ((rc = klt_stage_in(ctx, dimg))) return rc;
+    if ((rc = klt_launch_extract_patch(ctx, dimg.dev, w, w, h, x, y, height, width, dout.dev, dok))) return rc;
     int ok = 0;
-    KLT_CUDA(ctx, cudaMemcpyAsync(out, dout, (size_t)width * height * sizeof(float), cudaMemcpyDefault, ctx->stream));
+    if ((rc = klt_stage_out(ctx, dout))) return rc;
     KLT_CUDA(ctx, cudaMemcpyAsync(&ok, dok, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     if (!ok) return klt_fail(ctx, KLT_ERR_ASSERT, "patch out of bounds (trackFeaturesUtils.pyx:35)");
@@ -750,14 +699,6 @@ int klt_extract_patch(klt_ctx *ctx, const float *img, int w, int h, float x, flo
 }
 
 // ---- operator-level entry points of the reference's Cython modules --------------------------------------------------
-static int stage_image(klt_ctx *ctx, const float *img, size_t n, char *slot, const float **dev) {
-    *dev = img;
-    if (!klt_is_device_ptr(img)) {
-        KLT_CUDA(ctx, cudaMemcpyAsync(slot, img, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-        *dev = (const float *)slot;
-    }
-    return KLT_OK;
-}
 
 int klt_track_iterate(klt_ctx *ctx, const klt_params *params, float x2, float y2, const float *gx_patch, const float *gy_patch,
                       const float *img_patch, const float *img2, const float *gradx2, const float *grady2, int w, int h,
@@ -767,20 +708,17 @@ int klt_track_iterate(klt_ctx *ctx, const klt_params *params, float x2, float y2
     if (params->lighting_insensitive) return klt_fail(ctx, KLT_ERR_UNSUPPORTED, "lighting_insensitive: Not implemented (trackFeaturesUtils.pyx:435)");
     if (params->window_width != params->window_height) return klt_fail(ctx, KLT_ERR_UNSUPPORTED, "non-square windows are refused (quirk Q10)");
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)w * h, plane = align_up(n * sizeof(float), 256);
-    const size_t pn = (size_t)params->window_width * params->window_height, pbytes = align_up(3 * pn * sizeof(float), 256);
-    int rc = klt_ws_reserve(ctx, 3 * plane + pbytes + 256);
-    if (rc) return rc;
-    char *wsp = (char *)ctx->ws;
-    const float *d2, *dgx, *dgy;
-    if ((rc = stage_image(ctx, img2, n, wsp, &d2))) return rc;
-    if ((rc = stage_image(ctx, gradx2, n, wsp + plane, &dgx))) return rc;
-    if ((rc = stage_image(ctx, grady2, n, wsp + 2 * plane, &dgy))) return rc;
-    float *tp = (float *)(wsp + 3 * plane), *dout = (float *)(wsp + 3 * plane + pbytes);
+    const size_t n = (size_t)w * h, pn = (size_t)params->window_width * params->window_height;
+    KltArg<const float> d2 = klt_arg(img2, n), dgx = klt_arg(gradx2, n), dgy = klt_arg(grady2, n);
+    float *tp, *dout;                   // tp: the three patches back to back
+    int rc;
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { d2.place(c); dgx.place(c); dgy.place(c); tp = c.take<float>(3 * pn); dout = c.take<float>(4); })))
+        return rc;
+    if ((rc = klt_stage_in(ctx, d2)) || (rc = klt_stage_in(ctx, dgx)) || (rc = klt_stage_in(ctx, dgy))) return rc;
     KLT_CUDA(ctx, cudaMemcpyAsync(tp, img_patch, pn * sizeof(float), cudaMemcpyDefault, ctx->stream));
     KLT_CUDA(ctx, cudaMemcpyAsync(tp + pn, gx_patch, pn * sizeof(float), cudaMemcpyDefault, ctx->stream));
     KLT_CUDA(ctx, cudaMemcpyAsync(tp + 2 * pn, gy_patch, pn * sizeof(float), cudaMemcpyDefault, ctx->stream));
-    if ((rc = klt_launch_iterate(ctx, params, tp, d2, dgx, dgy, w, h, x2, y2, dout))) return rc;
+    if ((rc = klt_launch_iterate(ctx, params, tp, d2.dev, dgx.dev, dgy.dev, w, h, x2, y2, dout))) return rc;
     float res[4];
     KLT_CUDA(ctx, cudaMemcpyAsync(res, dout, sizeof(res), cudaMemcpyDeviceToHost, ctx->stream));
     KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -796,18 +734,16 @@ int klt_patch_combine(klt_ctx *ctx, const float *patch1, const float *img2, int 
     if (!ctx || !patch1 || !img2 || !out || w <= 0 || h <= 0 || width < 1 || height < 1 || mode < 0 || mode > 1)
         return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)w * h, plane = align_up(n * sizeof(float), 256), pn = (size_t)width * height, pbytes = align_up(pn * sizeof(float), 256);
-    int rc = klt_ws_reserve(ctx, plane + 2 * pbytes + 256);
-    if (rc) return rc;
-    char *wsp = (char *)ctx->ws;
-    const float *dimg;
-    if ((rc = stage_image(ctx, img2, n, wsp, &dimg))) return rc;
-    float *dp1 = (float *)(wsp + plane), *dout = (float *)(wsp + plane + pbytes);
-    int *dok = (int *)(wsp + plane + 2 * pbytes);
-    KLT_CUDA(ctx, cudaMemcpyAsync(dp1, patch1, pn * sizeof(float), cudaMemcpyDefault, ctx->stream));
-    if ((rc = klt_launch_patch_combine(ctx, dp1, dimg, w, h, x2, y2, height, width, mode, dout, dok))) return rc;
+    const size_t pn = (size_t)width * height;
+    KltArg<const float> dimg = klt_arg(img2, (size_t)w * h), dp1 = klt_arg_staged(patch1, pn);
+    KltArg<float> dout = klt_arg_staged(out, pn);
+    int *dok;
+    int rc;
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { dimg.place(c); dp1.place(c); dout.place(c); dok = c.take<int>(1); }))) return rc;
+    if ((rc = klt_stage_in(ctx, dimg)) || (rc = klt_stage_in(ctx, dp1))) return rc;
+    if ((rc = klt_launch_patch_combine(ctx, dp1.dev, dimg.dev, w, h, x2, y2, height, width, mode, dout.dev, dok))) return rc;
     int ok = 0;
-    KLT_CUDA(ctx, cudaMemcpyAsync(out, dout, pn * sizeof(float), cudaMemcpyDefault, ctx->stream));
+    if ((rc = klt_stage_out(ctx, dout))) return rc;
     KLT_CUDA(ctx, cudaMemcpyAsync(&ok, dok, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     if (!ok) return klt_fail(ctx, KLT_ERR_ASSERT, "patch out of bounds (trackFeaturesUtils.pyx:35)");

@@ -116,8 +116,103 @@ void klt_prof_end(klt_ctx *ctx, int token);
         KLT_CHECK_LAUNCH(ctx);                                  \
     } while (0)
 
-int klt_ws_reserve(klt_ctx *ctx, size_t bytes);          // grow-only workspace
+// Grow-only workspace.  Every extern "C" entry point that uses ctx->ws reserves it once, for its whole layout (klt_ws_layout),
+// before it enqueues anything into it, and nothing it calls reserves again: a reserve that grows frees the old block, and
+// with it whatever the caller has already staged there.
+int klt_ws_reserve(klt_ctx *ctx, size_t bytes);
 bool klt_is_device_ptr(const void *p);
+
+static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// Bump carver of one device block into 256-byte aligned buffers.  A layout is written once, as code that takes its buffers
+// from a carver: run on a null base it only counts the bytes (off), run on the block it hands out the pointers.
+struct KltCarver {
+    char *base;
+    size_t off;
+    template <class T> T *take(size_t count) {
+        T *p = base ? (T *)(base + off) : nullptr;
+        off += align_up(count * sizeof(T), 256);
+        return p;
+    }
+};
+
+// layout(KltCarver &) sizes the workspace, which is reserved, then carves ctx->ws
+template <class F> int klt_ws_layout(klt_ctx *ctx, F &&layout) {
+    KltCarver c{nullptr, 0};
+    layout(c);
+    int rc = klt_ws_reserve(ctx, c.off);
+    if (rc) return rc;
+    c = KltCarver{(char *)ctx->ws, 0};
+    layout(c);
+    return KLT_OK;
+}
+
+// layout(KltCarver &) sizes one new allocation *block (what: the error message's name for it), then carves it
+template <class F> int klt_alloc_layout(klt_ctx *ctx, void **block, const char *what, F &&layout) {
+    KltCarver c{nullptr, 0};
+    layout(c);
+    cudaError_t e = cudaMalloc(block, c.off);
+    if (e != cudaSuccess) {
+        *block = nullptr;
+        return klt_fail(ctx, KLT_ERR_NOMEM, "cudaMalloc(%zu) for %s failed: %s", c.off, what, cudaGetErrorString(e));
+    }
+    c = KltCarver{(char *)*block, 0};
+    layout(c);
+    return KLT_OK;
+}
+
+// A "host or device" array of a call.  klt_arg classifies the pointer once: a device array is used in place (dev == user), a
+// host array gets a slot in the call's layout (place).  klt_arg_staged always goes through a slot.  klt_stage_in fills the
+// slot from the caller's array, klt_stage_out copies it back, both on ctx->stream; without a slot they do nothing.
+template <class T> struct KltArg {
+    T *user;
+    size_t n;
+    bool host;
+    T *dev;
+    void place(KltCarver &c) { if (host) dev = c.take<T>(n); }
+};
+template <class T> KltArg<T> klt_arg(T *p, size_t n) { return {p, n, p && !klt_is_device_ptr(p), p}; }
+template <class T> KltArg<T> klt_arg_staged(T *p, size_t n) { return {p, n, true, p}; }
+template <class T> int klt_stage_in(klt_ctx *ctx, const KltArg<T> &a) {
+    if (a.host) KLT_CUDA(ctx, cudaMemcpyAsync((void *)a.dev, a.user, a.n * sizeof(T), cudaMemcpyDefault, ctx->stream));
+    return KLT_OK;
+}
+template <class T> int klt_stage_out(klt_ctx *ctx, const KltArg<T> &a) {
+    if (a.host) KLT_CUDA(ctx, cudaMemcpyAsync(a.user, a.dev, a.n * sizeof(T), cudaMemcpyDefault, ctx->stream));
+    return KLT_OK;
+}
+
+// the x, y, val arrays of a feature call
+struct KltFeatures {
+    KltArg<double> x, y;
+    KltArg<int32_t> val;
+    void place(KltCarver &c) { x.place(c); y.place(c); val.place(c); }
+};
+// classifies x, y and val, which must all be host or all be device
+static inline int klt_features(klt_ctx *ctx, double *x, double *y, int32_t *val, size_t n, KltFeatures *f) {
+    *f = KltFeatures{klt_arg(x, n), klt_arg(y, n), klt_arg(val, n)};
+    if (f->y.host != f->x.host || f->val.host != f->x.host)
+        return klt_fail(ctx, KLT_ERR_INVALID, "x, y, val must all be host or all be device");
+    return KLT_OK;
+}
+static inline int klt_stage_in(klt_ctx *ctx, const KltFeatures &f) {
+    int rc;
+    if ((rc = klt_stage_in(ctx, f.x)) || (rc = klt_stage_in(ctx, f.y)) || (rc = klt_stage_in(ctx, f.val))) return rc;
+    return KLT_OK;
+}
+static inline int klt_stage_out(klt_ctx *ctx, const KltFeatures &f) {
+    int rc;
+    if ((rc = klt_stage_out(ctx, f.x)) || (rc = klt_stage_out(ctx, f.y)) || (rc = klt_stage_out(ctx, f.val))) return rc;
+    return KLT_OK;
+}
+
+// Status words of tracking: one call's (track_impl) or a sequence's since its last klt_sequence_sync.  Cleared by one memset
+// and read back by one copy; the kernels get plain pointers to the fields.
+struct KltTrackStatus {
+    unsigned long long iters;     // Newton iterations
+    int asserted;                 // a feature window left the image (the reference raises AssertionError)
+    int scratch_assert;           // the backward pass's assert word under the forward-backward check (marks features only)
+};
 
 static inline bool klt_pyr_has_gradients(const klt_pyr *p) { return !p->hx || p->hx->grad_valid; }
 
@@ -166,8 +261,9 @@ int klt_stream_grad(klt_ctx *ctx, klt_pyr *p, int level, const klt_taps *taps, i
 int klt_stream_down2(klt_ctx *ctx, klt_pyr *p, int level, const klt_taps *taps, int first, int count);
 
 // ---- klt_select.cu -----------------------------------------------------------------------------------
+// sat_dev: the summed-area tables, [3][w * h]
 int klt_launch_scan(klt_ctx *ctx, const float *gx, const float *gy, size_t pitch, int w, int h, int bx, int by,
-                    int hw, int hh, int skip, float *val_dev /* [ny][nx] */, int nx, int ny);
+                    int hw, int hh, int skip, float *sat_dev, float *val_dev /* [ny][nx] */, int nx, int ny);
 // full selection for every image of `pyr` (or, pyr == NULL, for B explicit device gradient images img_stride apart);
 // x, y, val: [B][n_features] host or device; mask (optional, host or device): uint8 [B][h][mask_pitch], mask_stride apart
 // (0: one mask for all images), nonzero = candidates allowed there

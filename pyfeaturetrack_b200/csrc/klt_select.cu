@@ -789,7 +789,6 @@ select_walk_kernel(const __grid_constant__ SelDev S, int presorted) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 int klt_sel_geometry(klt_ctx *ctx, const klt_params *p, int w, int h, int n_features, int replace, SelDev *S) {
     if (w > 8191 || h > 8191) return klt_fail(ctx, KLT_ERR_UNSUPPORTED, "image larger than 8191 pixels per side");
@@ -829,40 +828,22 @@ int klt_sel_geometry(klt_ctx *ctx, const klt_params *p, int w, int h, int n_feat
     return KLT_OK;
 }
 
-size_t klt_sel_workspace_bytes(const SelDev *S, int B, bool strict_sat, bool own_features, bool masked) {
-    size_t t = 0;
-    if (strict_sat) t += align_up((size_t)B * 3 * S->W * S->H * sizeof(float), 256);
-    t += align_up((size_t)B * (S->ncand + 1) * sizeof(float), 256);              // vmap
-    t += align_up((size_t)B * (SEL_BINS * 3 + 1) * sizeof(unsigned int), 256);   // hist, cursor, offs
-    t += align_up((size_t)B * (SEL_PLAN_WORDS * sizeof(unsigned int) + SEL_STATUS_WORDS * sizeof(unsigned long long)), 256);
-    t += 2 * align_up((size_t)B * S->key_stride * sizeof(unsigned long long), 256);
-    if (S->replace || masked) t += align_up((size_t)B * S->map_stride, 256);
-    if (!S->grid_in_smem) t += align_up((size_t)B * S->grid_stride * sizeof(unsigned short), 256) + align_up((size_t)B * S->grid_stride * sizeof(unsigned int), 256);
-    t += align_up((size_t)B * S->n_features * sizeof(int) + 64, 256);            // free slots
-    if (own_features) t += align_up((size_t)B * S->n_features * (2 * sizeof(double) + sizeof(int)) + 64, 256);
-    return t + 1024;
-}
-
-void klt_sel_carve(SelDev *S, int B, bool strict_sat, bool own_features, char *base, float **sat, bool masked) {
-    char *p = base;
-    auto take = [&](size_t bytes) { char *q = p; p += align_up(bytes, 256); return q; };
-    if (sat) *sat = nullptr;
-    if (strict_sat) { float *s = (float *)take((size_t)B * 3 * S->W * S->H * sizeof(float)); if (sat) *sat = s; }
-    S->vmap = (float *)take((size_t)B * (S->ncand + 1) * sizeof(float));
-    unsigned int *h3 = (unsigned int *)take((size_t)B * (SEL_BINS * 3 + 1) * sizeof(unsigned int));
-    S->hist = h3; S->cursor = h3 + (size_t)B * SEL_BINS; S->offs = h3 + (size_t)2 * B * SEL_BINS;      // offs: [B][SEL_BINS + 1]
-    char *ps = take((size_t)B * (SEL_PLAN_WORDS * sizeof(unsigned int) + SEL_STATUS_WORDS * sizeof(unsigned long long)));
-    S->status = (unsigned long long *)ps; S->plan = (unsigned int *)(ps + (size_t)B * SEL_STATUS_WORDS * sizeof(unsigned long long));
-    S->keys = (unsigned long long *)take((size_t)B * S->key_stride * sizeof(unsigned long long));
-    S->keys2 = (unsigned long long *)take((size_t)B * S->key_stride * sizeof(unsigned long long));
-    S->premap = (S->replace || masked) ? (unsigned char *)take((size_t)B * S->map_stride) : nullptr;
-    S->grid_global = S->grid_in_smem ? nullptr : (unsigned short *)take((size_t)B * S->grid_stride * sizeof(unsigned short));
-    S->cellmin_global = S->grid_in_smem ? nullptr : (unsigned int *)take((size_t)B * S->grid_stride * sizeof(unsigned int));
-    S->free_slots = (int *)take((size_t)B * S->n_features * sizeof(int) + 64);
-    if (own_features) {
-        char *f = take((size_t)B * S->n_features * (2 * sizeof(double) + sizeof(int)) + 64);
-        S->fx = (double *)f; S->fy = S->fx + (size_t)B * S->n_features; S->fval = (int *)(S->fy + (size_t)B * S->n_features);
-    }
+float *klt_sel_layout(KltCarver &c, SelDev *S, int B, bool strict_sat, bool masked) {
+    float *sat = strict_sat ? c.take<float>((size_t)B * 3 * S->W * S->H) : nullptr;
+    S->vmap = c.take<float>((size_t)B * (S->ncand + 1));
+    S->hist = c.take<unsigned int>((size_t)B * SEL_BINS);
+    S->cursor = c.take<unsigned int>((size_t)B * SEL_BINS);
+    S->offs = c.take<unsigned int>((size_t)B * (SEL_BINS + 1));
+    S->status = c.take<unsigned long long>((size_t)B * SEL_STATUS_WORDS);
+    S->plan = c.take<unsigned int>((size_t)B * SEL_PLAN_WORDS);
+    S->keys = c.take<unsigned long long>((size_t)B * S->key_stride);
+    S->keys2 = c.take<unsigned long long>((size_t)B * S->key_stride);
+    S->premap = (S->replace || masked) ? c.take<unsigned char>((size_t)B * S->map_stride) : nullptr;
+    S->grid_global = S->grid_in_smem ? nullptr : c.take<unsigned short>((size_t)B * S->grid_stride);
+    S->cellmin_global = S->grid_in_smem ? nullptr : c.take<unsigned int>((size_t)B * S->grid_stride);
+    S->free_slots = c.take<int>((size_t)B * S->n_features + 16);
+    c.take<char>(1024);              // slack behind the last buffer
+    return sat;
 }
 
 static size_t walk_smem(const SelDev *S) {
@@ -958,16 +939,14 @@ int klt_sel_launch_pick(klt_ctx *ctx, const SelDev *S, int B) {
 }
 
 int klt_launch_scan(klt_ctx *ctx, const float *gx, const float *gy, size_t pitch, int w, int h, int bx, int by, int hw,
-                    int hh, int skip, float *val_dev, int nx, int ny) {
+                    int hh, int skip, float *sat_dev, float *val_dev, int nx, int ny) {
     SelDev S;
     memset(&S, 0, sizeof S);
     S.W = w; S.H = h; S.bx = bx; S.by = by; S.hw = hw; S.hh = hh; S.step = skip + 1; S.nx = nx; S.ny = ny;
     S.ncand = (size_t)nx * ny; S.vmap = val_dev; S.min_val = 1.f;
-    const size_t plane = align_up((size_t)w * h * sizeof(float), 256);
-    int rc = klt_ws_reserve(ctx, 3 * plane);
-    if (rc) return rc;
+    int rc;
     if ((rc = klt_sel_prepare_kernels_scan(ctx, &S))) return rc;
-    return klt_sel_launch_eigen_strict(ctx, &S, 1, gx, gy, 0, pitch, (float *)ctx->ws);
+    return klt_sel_launch_eigen_strict(ctx, &S, 1, gx, gy, 0, pitch, sat_dev);
 }
 
 int klt_sel_prepare_kernels_scan(klt_ctx *ctx, const SelDev *S) {
@@ -984,42 +963,25 @@ int klt_select_batch(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr
     SelDev S;
     int rc = klt_sel_geometry(ctx, p, w, h, n_features, replace, &S);
     if (rc) return rc;
-    const bool host = !klt_is_device_ptr(x);
-    if (host != !klt_is_device_ptr(y) || host != !klt_is_device_ptr(val)) return klt_fail(ctx, KLT_ERR_INVALID, "x, y, val must all be host or all be device");
+    const size_t total = (size_t)B * n_features;
+    KltFeatures f;
+    if ((rc = klt_features(ctx, x, y, val, total, &f))) return rc;
     const bool masked = mask != nullptr;
     if (masked && mask_pitch < (size_t)w) return klt_fail(ctx, KLT_ERR_INVALID, "mask_pitch %zu smaller than width %d", mask_pitch, w);
-    // a host mask is uploaded behind the selection workspace
-    const bool mask_host = masked && !klt_is_device_ptr(mask);
-    const size_t mask_bytes = masked ? (size_t)(mask_stride ? B - 1 : 0) * mask_stride + (size_t)(h - 1) * mask_pitch + w : 0;
-    const size_t sel_b = klt_sel_workspace_bytes(&S, B, true, host, masked);
-    if ((rc = klt_ws_reserve(ctx, sel_b + (mask_host ? align_up(mask_bytes, 256) : 0)))) return rc;
+    KltArg<const uint8_t> dmask = klt_arg(mask, masked ? (size_t)(mask_stride ? B - 1 : 0) * mask_stride + (size_t)(h - 1) * mask_pitch + w : 0);
     float *sat;
-    klt_sel_carve(&S, B, true, host, (char *)ctx->ws, &sat, masked);
-    SelMask sm = {mask, mask_pitch, mask_stride, nullptr};
-    if (mask_host) {
-        unsigned char *d = (unsigned char *)ctx->ws + sel_b;
-        KLT_CUDA(ctx, cudaMemcpyAsync(d, mask, mask_bytes, cudaMemcpyHostToDevice, ctx->stream));
-        sm.mask = d;
-    }
-    const size_t total = (size_t)B * n_features;
-    if (host) {
-        if (replace) {
-            KLT_CUDA(ctx, cudaMemcpyAsync(S.fx, x, total * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-            KLT_CUDA(ctx, cudaMemcpyAsync(S.fy, y, total * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-            KLT_CUDA(ctx, cudaMemcpyAsync(S.fval, val, total * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-        }
-    } else { S.fx = x; S.fy = y; S.fval = val; }
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { sat = klt_sel_layout(c, &S, B, true, masked); f.place(c); dmask.place(c); }))) return rc;
+    S.fx = f.x.dev; S.fy = f.y.dev; S.fval = f.val.dev;
+    const SelMask sm = {dmask.dev, mask_pitch, mask_stride, nullptr};
+    if ((rc = klt_stage_in(ctx, dmask))) return rc;
+    if (replace && (rc = klt_stage_in(ctx, f))) return rc;
     if ((rc = klt_sel_prepare_kernels(ctx, &S))) return rc;
     if ((rc = klt_sel_launch_begin(ctx, &S, B, masked ? &sm : nullptr))) return rc;
     rc = pyr ? klt_sel_launch_eigen(ctx, &S, B, pyr, select_mode, sat) : klt_sel_launch_eigen_strict(ctx, &S, B, gx0, gy0, img_stride, pitch, sat);
     if (rc) return rc;
     if ((rc = klt_sel_launch_pick(ctx, &S, B))) return rc;
-    if (host) {
-        KLT_CUDA(ctx, cudaMemcpyAsync(x, S.fx, total * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(y, S.fy, total * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(val, S.fval, total * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-    }
-    if (host || n_consumed) {
+    if ((rc = klt_stage_out(ctx, f))) return rc;
+    if (f.x.host || n_consumed) {
         unsigned long long st[SEL_STATUS_WORDS] = {0, 0, 0, 0};
         KLT_CUDA(ctx, cudaMemcpyAsync(st, S.status, sizeof st, cudaMemcpyDeviceToHost, ctx->stream));
         KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1039,9 +1001,8 @@ int klt_eigen_maps(klt_ctx *ctx, const klt_params *p, int select_mode, klt_pyr *
     if (!val || !S.ncand) return KLT_OK;
     if (select_mode == KLT_SELECT_FAST && pyr->hx->taps_valid && !klt_sel_fast_covers(&S, &pyr->hx->taps.grad_gauss, &pyr->hx->taps.grad_deriv))
         return klt_fail(ctx, KLT_ERR_UNSUPPORTED, "the fused eigenvalue pass does not cover this window / gradient kernel");
-    if ((rc = klt_ws_reserve(ctx, klt_sel_workspace_bytes(&S, B, true, false)))) return rc;
     float *sat;
-    klt_sel_carve(&S, B, true, false, (char *)ctx->ws, &sat);
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { sat = klt_sel_layout(c, &S, B, true, false); }))) return rc;
     if ((rc = klt_sel_prepare_kernels(ctx, &S))) return rc;
     if ((rc = klt_sel_launch_begin(ctx, &S, B))) return rc;
     if ((rc = klt_sel_launch_eigen(ctx, &S, B, pyr, select_mode, sat))) return rc;
@@ -1061,23 +1022,19 @@ int klt_greedy_presorted(klt_ctx *ctx, const unsigned long long *keys_host, unsi
     int rc = klt_sel_geometry(ctx, &p, w, h, n_features, overwrite ? 0 : 1, &S);
     if (rc) return rc;
     S.ncand = nk; S.key_stride = align_up((size_t)nk + 1, 32);        // the key buffer holds the caller's list
-    if ((rc = klt_ws_reserve(ctx, klt_sel_workspace_bytes(&S, 1, false, true)))) return rc;
-    klt_sel_carve(&S, 1, false, true, (char *)ctx->ws, nullptr);
+    // the walk reads and writes the features in the workspace: the caller's arrays are copied in (replacement) and back
+    KltFeatures f{klt_arg_staged(x, n_features), klt_arg_staged(y, n_features), klt_arg_staged(val, n_features)};
+    if ((rc = klt_ws_layout(ctx, [&](KltCarver &c) { klt_sel_layout(c, &S, 1, false, false); f.place(c); }))) return rc;
+    S.fx = f.x.dev; S.fy = f.y.dev; S.fval = f.val.dev;
     unsigned int plan[SEL_PLAN_WORDS] = {0};
     plan[SEL_PLAN_RB_HI] = 0; plan[SEL_PLAN_NKEYS] = nk;
     KLT_CUDA(ctx, cudaMemcpyAsync(S.plan, plan, sizeof plan, cudaMemcpyHostToDevice, ctx->stream));
     if (nk) KLT_CUDA(ctx, cudaMemcpyAsync(S.keys, keys_host, (size_t)nk * sizeof(unsigned long long), cudaMemcpyHostToDevice, ctx->stream));
-    if (!overwrite) {
-        KLT_CUDA(ctx, cudaMemcpyAsync(S.fx, x, n_features * sizeof(double), cudaMemcpyDefault, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(S.fy, y, n_features * sizeof(double), cudaMemcpyDefault, ctx->stream));
-        KLT_CUDA(ctx, cudaMemcpyAsync(S.fval, val, n_features * sizeof(int), cudaMemcpyDefault, ctx->stream));
-    }
+    if (!overwrite && (rc = klt_stage_in(ctx, f))) return rc;
     if ((rc = klt_sel_prepare_kernels(ctx, &S))) return rc;
     if ((rc = klt_sel_launch_begin(ctx, &S, 1))) return rc;
     KLT_LAUNCH(ctx, "select_walk", 0.0, (select_walk_kernel<<<1, WALK_THREADS, walk_smem(&S), ctx->stream>>>(S, 1)));
-    KLT_CUDA(ctx, cudaMemcpyAsync(x, S.fx, n_features * sizeof(double), cudaMemcpyDefault, ctx->stream));
-    KLT_CUDA(ctx, cudaMemcpyAsync(y, S.fy, n_features * sizeof(double), cudaMemcpyDefault, ctx->stream));
-    KLT_CUDA(ctx, cudaMemcpyAsync(val, S.fval, n_features * sizeof(int), cudaMemcpyDefault, ctx->stream));
+    if ((rc = klt_stage_out(ctx, f))) return rc;
     KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return KLT_OK;
 }

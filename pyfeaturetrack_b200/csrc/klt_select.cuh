@@ -50,9 +50,10 @@ struct SelMask {
 };
 
 int klt_sel_geometry(klt_ctx *ctx, const klt_params *p, int w, int h, int n_features, int replace, SelDev *S);
-// masked: reserve / carve the pre-mark map also in SELECTING_ALL mode
-size_t klt_sel_workspace_bytes(const SelDev *S, int B, bool strict_sat, bool own_features, bool masked = false);
-void klt_sel_carve(SelDev *S, int B, bool strict_sat, bool own_features, char *base, float **sat, bool masked = false);
+// The selection buffers of B images, taken from `c` into S; returns the summed-area tables of the STRICT eigenvalue pass
+// (strict_sat, else null).  masked: the pre-mark map also in SELECTING_ALL mode.  The feature lists S->fx, fy, fval are the
+// caller's to place.
+float *klt_sel_layout(KltCarver &c, SelDev *S, int B, bool strict_sat, bool masked);
 int klt_sel_prepare_kernels(klt_ctx *ctx, const SelDev *S);          // cudaFuncSetAttribute calls: outside stream capture
 int klt_sel_prepare_kernels_scan(klt_ctx *ctx, const SelDev *S);
 int klt_sel_launch_begin(klt_ctx *ctx, const SelDev *S, int B, const SelMask *m = nullptr);

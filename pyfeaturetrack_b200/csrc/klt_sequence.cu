@@ -39,11 +39,10 @@ struct klt_sequence {
     SelDev S_all, S_rep;
     float *sat;
     bool fast_select_ok;
-    char *block;                     // selection workspace + feature lists + counters (one allocation)
+    void *block;                     // selection workspace + feature lists + status words (one allocation)
     double *fx, *fy;
     int *fval, *fval_tracked;
-    unsigned long long *iters;       // [0] Newton iterations since the last klt_sequence_sync
-    int *aflag;                      // sticky "a window left the image" flag (the reference's AssertionError case)
+    KltTrackStatus *status;          // since the last klt_sequence_sync
     uint8_t *stage[SEQ_ROT];         // device staging of the frames, one per rotation slot (the captured graphs carry the pointer)
     size_t stage_bytes, cap_pitch, cap_stride;
     cudaEvent_t stage_free[SEQ_ROT], stage_ready[SEQ_ROT];
@@ -61,7 +60,7 @@ struct klt_sequence {
     // forward-backward check (klt_sequence_set_fb_check): threshold (0 = off) and its arrays, allocated on first use
     float fb_max;
     bool fb_ran;                     // the last step ran the check (fb_err is current)
-    char *fb_block;
+    void *fb_block;
     FbArrays fb;
     float *fb_err;
     // selection mask (klt_sequence_set_mask): the pre-mark map it seeds, [B][map_stride], allocated on first use (its address
@@ -72,7 +71,6 @@ struct klt_sequence {
     size_t mask_up_bytes;
 };
 
-static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // selection on the level-0 planes of `p` (all images) into the sequence's feature lists, one stream
 // where the pre-mark map of a selection starts: the mask's map while a mask is set, else cleared
@@ -126,8 +124,9 @@ static int enqueue_back(klt_ctx *ctx, klt_sequence *q, int prev, int slot, int r
     // both pyramids stay alive until BACK ends (rotation of three), so the backward pass needs no further synchronisation
     if (q->fb_max > 0.f) {
         if ((rc = klt_launch_track_fb(ctx, &q->params, q->pyr[prev], q->pyr[slot], q->n, q->fb_max, q->fx, q->fy, q->fval, q->fb,
-                                      q->fb_err, q->iters, q->aflag))) return rc;
-    } else if ((rc = klt_launch_track(ctx, &q->params, q->pyr[prev], q->pyr[slot], q->n, q->fx, q->fy, q->fval, q->iters, q->aflag))) return rc;
+                                      q->fb_err, &q->status->iters, &q->status->asserted))) return rc;
+    } else if ((rc = klt_launch_track(ctx, &q->params, q->pyr[prev], q->pyr[slot], q->n, q->fx, q->fy, q->fval, &q->status->iters,
+                                      &q->status->asserted))) return rc;
     KLT_CUDA(ctx, cudaMemcpyAsync(q->fval_tracked, q->fval, (size_t)q->B * q->n * sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream));
     if (!replace) return KLT_OK;
     const SelDev S = sel_for_slot(q, slot);
@@ -252,21 +251,20 @@ int klt_sequence_create(klt_ctx *ctx, const klt_params *params, const klt_taps *
     q->fast_select_ok = select_mode == KLT_SELECT_FAST && klt_sel_fast_covers(&q->S_rep, &taps->grad_gauss, &taps->grad_deriv);
     const bool need_sat = !q->fast_select_ok;
     const size_t total = (size_t)q->B * q->n;
-    const size_t sel_b = klt_sel_workspace_bytes(&q->S_rep, q->B, need_sat, true);
-    const size_t extra = align_up(total * sizeof(int), 256) + 512;
-    cudaError_t e = cudaMalloc(&q->block, sel_b + extra);
-    if (e != cudaSuccess) { klt_sequence_destroy(ctx, q); return klt_fail(ctx, KLT_ERR_NOMEM, "cudaMalloc(%zu) for the sequence workspace failed: %s", sel_b + extra, cudaGetErrorString(e)); }
-    klt_sel_carve(&q->S_rep, q->B, need_sat, true, q->block, &q->sat);
+    if ((rc = klt_alloc_layout(ctx, &q->block, "the sequence workspace", [&](KltCarver &c) {
+            q->sat = klt_sel_layout(c, &q->S_rep, q->B, need_sat, false);
+            q->fx = c.take<double>(total); q->fy = c.take<double>(total); q->fval = c.take<int>(total);
+            q->fval_tracked = c.take<int>(total);
+            q->status = c.take<KltTrackStatus>(1);
+        }))) { klt_sequence_destroy(ctx, q); return rc; }
+    q->S_rep.fx = q->fx; q->S_rep.fy = q->fy; q->S_rep.fval = q->fval;
+    q->fb.scratch_assert = &q->status->scratch_assert;
     q->vmap[0] = q->S_rep.vmap;
     for (int i = 1; i < SEQ_ROT; i++) {
-        e = cudaMalloc(&q->vmap[i], (size_t)q->B * (q->S_rep.ncand + 1) * sizeof(float));
+        cudaError_t e = cudaMalloc(&q->vmap[i], (size_t)q->B * (q->S_rep.ncand + 1) * sizeof(float));
         if (e != cudaSuccess) { klt_sequence_destroy(ctx, q); return klt_fail(ctx, KLT_ERR_NOMEM, "cudaMalloc for an eigenvalue map failed: %s", cudaGetErrorString(e)); }
     }
-    q->fx = q->S_rep.fx; q->fy = q->S_rep.fy; q->fval = q->S_rep.fval;
-    q->fval_tracked = (int *)(q->block + sel_b);
-    q->iters = (unsigned long long *)(q->block + sel_b + align_up(total * sizeof(int), 256));
-    q->aflag = (int *)(q->iters + 4);
-    cudaMemsetAsync(q->block + sel_b, 0, extra, ctx->stream);
+    cudaMemsetAsync(q->fval_tracked, 0, (char *)(q->status + 1) - (char *)q->fval_tracked, ctx->stream);
     q->S_all = q->S_rep;                    // same buffers, SELECTING_ALL semantics
     q->S_all.replace = 0; q->S_all.premap = nullptr; q->S_all.target_mul = 32u; q->S_all.target_add = 8192u;
     if ((rc = klt_sel_prepare_kernels(ctx, &q->S_rep))) { klt_sequence_destroy(ctx, q); return rc; }
@@ -401,12 +399,12 @@ int klt_sequence_get_features(klt_ctx *ctx, klt_sequence *q, double *x, double *
 
 int klt_sequence_sync(klt_ctx *ctx, klt_sequence *q, int64_t *n_iterations) {
     if (!ctx || !q) return klt_fail(ctx, KLT_ERR_INVALID, "bad argument");
-    unsigned long long res[5] = {0, 0, 0, 0, 0};
-    KLT_CUDA(ctx, cudaMemcpyAsync(res, q->iters, sizeof res, cudaMemcpyDeviceToHost, ctx->stream));
-    KLT_CUDA(ctx, cudaMemsetAsync(q->iters, 0, sizeof res, ctx->stream));
+    KltTrackStatus res{};
+    KLT_CUDA(ctx, cudaMemcpyAsync(&res, q->status, sizeof res, cudaMemcpyDeviceToHost, ctx->stream));
+    KLT_CUDA(ctx, cudaMemsetAsync(q->status, 0, sizeof res, ctx->stream));
     KLT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (n_iterations) *n_iterations = (int64_t)res[0];
-    if ((int)(res[4] & 0xffffffffull))
+    if (n_iterations) *n_iterations = (int64_t)res.iters;
+    if (res.asserted)
         return klt_fail(ctx, KLT_ERR_ASSERT, "a feature window left the image at a pyramid level: the reference raises AssertionError (trackFeaturesUtils.pyx:35)");
     return KLT_OK;
 }
@@ -430,18 +428,13 @@ int klt_sequence_set_fb_check(klt_ctx *ctx, klt_sequence *q, float max_fb_error)
         return klt_fail(ctx, KLT_ERR_INVALID, "max_fb_error must be 0 (off) or finite and > 0 (got %g)", (double)max_fb_error);
     KLT_CUDA(ctx, cudaSetDevice(ctx->device));
     if (max_fb_error > 0.f && !q->fb_block) {
-        const size_t total = (size_t)q->B * q->n, db = align_up(total * sizeof(double), 256), ib = align_up(total * sizeof(int), 256);
-        const size_t bytes = 4 * db + 2 * ib + 256;
-        cudaError_t e = cudaMalloc(&q->fb_block, bytes);
-        if (e != cudaSuccess) { q->fb_block = nullptr; return klt_fail(ctx, KLT_ERR_NOMEM, "cudaMalloc(%zu) for the forward-backward arrays failed: %s", bytes, cudaGetErrorString(e)); }
-        char *b = q->fb_block;
-        q->fb.x0 = (double *)b; b += db;
-        q->fb.y0 = (double *)b; b += db;
-        q->fb.xb = (double *)b; b += db;
-        q->fb.yb = (double *)b; b += db;
-        q->fb.vb = (int32_t *)b; b += ib;
-        q->fb_err = (float *)b; b += ib;
-        q->fb.scratch_assert = (int *)b;
+        const size_t total = (size_t)q->B * q->n;
+        int rc = klt_alloc_layout(ctx, &q->fb_block, "the forward-backward arrays", [&](KltCarver &c) {
+            q->fb.x0 = c.take<double>(total); q->fb.y0 = c.take<double>(total); q->fb.xb = c.take<double>(total); q->fb.yb = c.take<double>(total);
+            q->fb.vb = c.take<int32_t>(total);
+            q->fb_err = c.take<float>(total);
+        });
+        if (rc) return rc;
     }
     if (max_fb_error != q->fb_max) drop_graphs(q);      // the captured BACK halves carry the check and its threshold
     q->fb_max = max_fb_error;
